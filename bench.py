@@ -18,6 +18,13 @@ measures; the one-batch-at-a-time figures are reported beside it (`single_batch`
   configs      : BASELINE.json configs[2..4] at their stated sizes
   cpu_baseline : the C port of the reference algorithm on the box's host cores, bounded sample
 
+Every leg above that is timed per batch runs K = --steps steps, one batch each (configs[2..3] too); configs[4] is one
+pass over its 2^24 inputs and `verify_one_us` the mean of 30 single-proof calls.
+
+--dump-outputs DIR : after the timed steps of `value`, what its last step computed goes to DIR/<name>.npy (float32 /
+                   float64; rank 0's batch): the verdict, the batch seed, and the challenges c_j and delinearization
+                   scalars z_j of a fixed sample of 2^16 proofs.  The inputs are fixed by the arguments, so two builds
+                   can be compared output for output.
 --impl reference : that CPU port timed alone on the same config (the reference is Rust on un-vendored crates and
                    cannot be built in this image; DESIGN.md section 2).
 --gpus N (torchrun): every rank serves whole batches on its own GPU (independent batches: no data-path
@@ -34,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -102,6 +110,29 @@ def workload_name(log2n):
     return "Bandersnatch thin-VRF batch verify, 2^%d synthetic proofs (M=1, 4096 signers), BASELINE.json configs[1]" % log2n
 
 
+DUMP_SAMPLE = 1 << 16
+
+
+def dump_outputs(out_dir, h, status):
+    """What the step `h` last ran computed, as DIR/<name>.npy: the verdict `BatchVerifier.verify` reports, the batch
+    seed, and for a fixed sample of proofs the challenges c_j and delinearization scalars z_j (the C and Z taps; one row
+    of bytes per proof).  Bytes are stored as float32, under 9 MB in all."""
+    from ark_vrf_b200 import Tap
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(h)
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    arrays = {
+        "verdict": np.array([status], dtype=np.float64),
+        "seed": h.tap(Tap.SEED).astype(np.float32),
+        "sample_index": idx.astype(np.float64),
+        "challenge_c": h.tap(Tap.C).reshape(n, 16)[idx].astype(np.float32),
+        "delinearization_z": h.tap(Tap.Z).reshape(n, -1)[idx].astype(np.float32),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] outputs of the last timed step -> {out_dir}: " + ", ".join(f"{k} {a.shape}" for k, a in arrays.items()))
+
+
 def cpu_reference_arm(args, rank):
     """--impl reference: the CPU port of thin::BatchVerifier (oracle/avrf_oracle.c) on all host threads, the SAME
     config as the GPU arm: every step prepares and verifies one whole 2^log2n-proof batch."""
@@ -154,7 +185,13 @@ def main():
     ap.add_argument("--hashers", type=int, default=-1,
                     help="shared multi-buffer SHA-512 threads per GPU for the e2e leg (0: one hashing core per worker; "
                          "-1: 0 when the rank has a core per worker, else up to 3 with 8 workers each)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -271,7 +308,7 @@ def main():
             sh_t.append(td)
         for _ in range(2):
             step_sharded()
-        k_sh = max(3, args.steps // 4)
+        k_sh = args.steps
         ms_sh, _ = timed(lambda: [step_sharded() for _ in range(k_sh)], k_sh, others=[shv])
         sharded = {"ms_per_batch": round(ms_sh, 3), "proofs_per_s": n / (ms_sh * 1e-3), "scaling": "strong",
                    "phases_ms": {k.replace("_s", ""): round(1e3 * float(np.mean([t[k] for t in sh_t[-k_sh:]])), 3)
@@ -291,7 +328,7 @@ def main():
         bv.clear()
         bv.push_many(*host)                  # H2D from pinned host memory
         assert bv.verify_status() == 0
-    k1 = max(3, min(args.steps, 8))
+    k1 = args.steps
     for _ in range(3):
         step_resident()
     ms_one, tms = timed(lambda: [step_resident() for _ in range(k1)], k1)
@@ -323,7 +360,7 @@ def main():
         pm, vm = ctypes.c_double(0), ctypes.c_double(0)
         for _ in range(2):
             assert pl.avrf_pushloop_step(hpl, 1, ctypes.byref(pm), ctypes.byref(vm)) == 0
-        kd = max(3, min(args.steps, 5))
+        kd = args.steps
         acc = []
 
         def step_drop():
@@ -361,7 +398,7 @@ def main():
             assert wv.verify_status() == 0
         for _ in range(2):
             step_wire()
-        kw = max(3, min(args.steps, 5))
+        kw = args.steps
         barrier()
         t0 = time.perf_counter()
         for _ in range(kw):
@@ -431,10 +468,12 @@ def main():
     stagger_s = (args.stagger_ms if args.stagger_ms >= 0 else (4.0 if (n_hash == 0 and T > 8) else 0.0)) * 1e-3
 
     def run_steps(k):
-        """k steps shared by the T handles: each host thread takes the next step until k are done."""
+        """k steps shared by the T handles: each host thread takes the next step until k are done.  Returns the handle
+        that ran the k-th step and its verdict."""
         lock = threading.Lock()
         left = [k]
         errs = []
+        last = [None, None]
         trace = [] if os.environ.get("AVRF_BENCH_TRACE") else None
         t_run0 = time.perf_counter()
 
@@ -447,10 +486,14 @@ def main():
                         if left[0] == 0:
                             return
                         left[0] -= 1
+                        is_last = left[0] == 0
                     t_a = time.perf_counter()
                     h.invalidate()
-                    if h.verify_status() != 0:
+                    st = h.verify_status()
+                    if st != 0:
                         errs.append("verdict")
+                    if is_last:
+                        last[:] = [h, st]
                     tm = h.timings()
                     with lock:
                         launches[0] += tm["kernel_launches"]
@@ -467,6 +510,7 @@ def main():
         assert not errs, errs
         if trace:
             log("[trace] (start_ms, end_ms, host_hash_ms, prepare_ms) per step:", sorted(trace))
+        return last
 
     t_e2e = T
 
@@ -479,9 +523,11 @@ def main():
         run_steps(max(args.warmup, T))             # warm-up: every handle has run at least once
         clk.rows.clear()
         launches[0] = 0
-        ms_step, _ = timed(lambda: run_steps(args.steps), args.steps, others=handles[1:])
+        ms_step, (h_last, st_last) = timed(lambda: run_steps(args.steps), args.steps, others=handles[1:])
         n_launch = launches[0]
         clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, h_last, st_last)
     for h in handles[1:]:
         h.close()
     bv.set_blocking(False)
@@ -565,8 +611,8 @@ def main():
             return {"proofs_per_s": (1 << lg) / (ms * 1e-3), "ms_per_batch": round(ms, 2), "batch": 1 << lg, "io_pairs": m,
                     "host_hash_ms": round(float(np.mean([t["host_hash_ms"] for t in tt[1:]])), 2), "accumulate_ms": round(a_ms, 3),
                     "roofline_frac": round(ent * CANON_MM_PER_ADD * MM_MACS / (a_ms * 1e-3) / peak_wide, 4), "reject_ok": True}
-        configs["C2_ed25519_2p20"] = run_cfg(1, 1, 20, 3)
-        configs["C3_babyjubjub_2p22_m4"] = run_cfg(2, 4, 22, 2)
+        configs["C2_ed25519_2p20"] = run_cfg(1, 1, 20, args.steps)
+        configs["C3_babyjubjub_2p22_m4"] = run_cfg(2, 4, 22, args.steps)
         # C4: bulk Elligator2 hash-to-curve + VRF output, 2^24 inputs over the ranks (no collective), host buffers
         n4 = (1 << 24) // world
         chunk = 1 << 21
