@@ -94,6 +94,10 @@ SIGNATURES = {
     "avrf_pedersen_batch_new": (C.c_void_p, [C.c_uint32, C.c_uint32]),
     "avrf_pedersen_batch_push_many": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
     "avrf_pedersen_batch_verify": (C.c_int, [C.c_void_p, i32p]),
+    "avrf_pedersen_batch_verify_each": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "avrf_pedersen_verify_one": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, i32p]),
+    "avrf_pedersen_prove_many": (C.c_int, [C.c_uint32, C.c_uint32, C.c_uint64] + [C.c_void_p] * 12),
     "avrf_hash_to_curve": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p,
                                      C.c_void_p, C.c_void_p]),
     "avrf_vrf_output": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]),

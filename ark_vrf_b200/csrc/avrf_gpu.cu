@@ -10,6 +10,8 @@
 //   Input::new         src/lib.rs:500-502       -> k_h2c
 //   Secret::output     src/lib.rs:391-393       -> k_scalar_mul
 //   Prover::prove      src/thin.rs:111-129      -> k_prove      (synthetic-input generator)
+//   pedersen::Prover::prove      src/pedersen.rs:136-186 -> k_prove_ped
+//   pedersen::Verifier::verify   src/pedersen.rs:188-253 -> k_verify_one_ped, k_verify_each_ped (per-proof verdicts)
 // There is no CPU fallback: without a CUDA device every compute entry point fails.
 #include <cstdlib>
 #include <map>
@@ -1303,22 +1305,30 @@ struct OneCtx {
   DevBuf dev;
 };
 
-int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios,
-                         const uint8_t* ad, uint32_t ad_len, const uint8_t r[64], const uint8_t s[32], int32_t* status) {
-  if (suite > 2 || fmt > 1) return fail(AVRF_ERR_ARG, "bad suite/fmt");
-  if (!pk || !r || !s || !status || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
-  if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
-  NEED_DEVICE();
+static int one_ctx(OneCtx** out) {
   static thread_local OneCtx ctx;
   int dev = g_device.load();
   if (ctx.device != dev) {
     if (!ctx.st) CK(cudaStreamCreateWithFlags(&ctx.st, cudaStreamNonBlocking));
     ctx.device = dev;
   }
+  *out = &ctx;
+  return 0;
+}
+
+int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios,
+                         const uint8_t* ad, uint32_t ad_len, const uint8_t r[64], const uint8_t s[32], int32_t* status) {
+  if (suite > 2 || fmt > 1) return fail(AVRF_ERR_ARG, "bad suite/fmt");
+  if (!pk || !r || !s || !status || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
+  if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
+  NEED_DEVICE();
+  OneCtx* cp;
+  int rc = one_ctx(&cp);
+  if (rc) return rc;
+  OneCtx& ctx = *cp;
   size_t in_bytes = 176 + 128 * (size_t)n_ios + ad_len;
   size_t z_off = (in_bytes + 255) & ~(size_t)255, st_off = z_off + 16 * (size_t)n_ios + 16;
   size_t total = st_off + 64;
-  int rc;
   if ((rc = ctx.pin.reserve(total)) || (rc = ctx.dev.reserve(total, 0, ctx.st))) return rc;
   uint8_t* h = ctx.pin.as<uint8_t>();
   memcpy(h, pk, 64);
@@ -1338,6 +1348,49 @@ int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], con
   a.canonical = fmt == AVRF_FMT_CANONICAL;
   DISPATCH(suite, (k_verify_one<S><<<1, 32, 0, ctx.st>>>(a)));
   LAUNCHED("k_verify_one");
+  CK(cudaMemcpyAsync(h + st_off, d + st_off, 8, cudaMemcpyDeviceToHost, ctx.st));
+  CK(cudaStreamSynchronize(ctx.st));
+  const int32_t* out = reinterpret_cast<const int32_t*>(h + st_off);
+  if (out[1] & 2) return fail(AVRF_ERR_ARG, "an input coordinate or scalar is not below its modulus (not a field element)");
+  *status = out[0];
+  return 0;
+}
+
+// ---- pedersen::Verifier::verify (src/pedersen.rs:188-253): both equations, exact, one thread -------------------
+int avrf_pedersen_verify_one(uint32_t suite, uint32_t fmt, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
+                             uint32_t ad_len, const uint8_t pk_com[64], const uint8_t r[64], const uint8_t ok[64],
+                             const uint8_t s[32], const uint8_t sb[32], int32_t* status) {
+  if (suite > 2 || fmt > 1) return fail(AVRF_ERR_ARG, "bad suite/fmt");
+  if (!pk_com || !r || !ok || !s || !sb || !status || (n_ios && !ios) || (ad_len && !ad))
+    return fail(AVRF_ERR_ARG, "null argument");
+  if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
+  NEED_DEVICE();
+  OneCtx* cp;
+  int rc = one_ctx(&cp);
+  if (rc) return rc;
+  OneCtx& ctx = *cp;
+  size_t in_bytes = 272 + 128 * (size_t)n_ios + ad_len;
+  size_t st_off = (in_bytes + 255) & ~(size_t)255, total = st_off + 64;
+  if ((rc = ctx.pin.reserve(total)) || (rc = ctx.dev.reserve(total, 0, ctx.st))) return rc;
+  uint8_t* h = ctx.pin.as<uint8_t>();
+  memcpy(h, pk_com, 64);
+  memcpy(h + 64, r, 64);
+  memcpy(h + 128, ok, 64);
+  memcpy(h + 192, s, 32);
+  memcpy(h + 224, sb, 32);
+  memcpy(h + 256, &n_ios, 4);
+  memcpy(h + 260, &ad_len, 4);
+  memset(h + 264, 0, 8);
+  if (n_ios) memcpy(h + 272, ios, 128 * (size_t)n_ios);
+  if (ad_len) memcpy(h + 272 + 128 * (size_t)n_ios, ad, ad_len);
+  uint8_t* d = ctx.dev.as<uint8_t>();
+  CK(cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx.st));
+  PedOneArgs a;
+  a.in = d;
+  a.status = reinterpret_cast<int32_t*>(d + st_off);
+  a.canonical = fmt == AVRF_FMT_CANONICAL;
+  DISPATCH(suite, (k_verify_one_ped<S><<<1, 32, 0, ctx.st>>>(a)));
+  LAUNCHED("k_verify_one_ped");
   CK(cudaMemcpyAsync(h + st_off, d + st_off, 8, cudaMemcpyDeviceToHost, ctx.st));
   CK(cudaStreamSynchronize(ctx.st));
   const int32_t* out = reinterpret_cast<const int32_t*>(h + st_off);
@@ -1415,6 +1468,26 @@ int avrf_thin_batch_verify_each(avrf_batch* b, int32_t* statuses) {
   a.io_off = b->io_off.as<uint32_t>(); a.status = dst.as<int32_t>(); a.n = (uint32_t)b->n;
   DISPATCH(b->suite, (k_verify_each<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
   LAUNCHED("k_verify_each");
+  CK(cudaMemcpyAsync(statuses, dst.p, 4 * b->n, cudaMemcpyDeviceToHost, b->st));
+  CK(hsync(b, b->st));
+  return 0;
+}
+
+int avrf_pedersen_batch_verify_each(avrf_batch* b, int32_t* statuses) {
+  if (!b || !statuses) return fail(AVRF_ERR_ARG, "null argument");
+  if (b->scheme != 1) return fail(AVRF_ERR_ARG, "not a Pedersen batch");
+  int32_t invalid = 0;                  // (per-proof verdicts below; this call only surfaces out-of-range inputs)
+  int rc = avrf_thin_batch_prepare(b, &invalid);
+  if (rc) return rc;
+  if (b->n == 0) return 0;
+  DevBuf dst;
+  if ((rc = dst.reserve(4 * b->n, 0, b->st))) return rc;
+  PedEachArgs a;
+  a.pkcom = b->pk.as<Affine>(); a.ios = b->ios.as<Affine>(); a.io_off = b->io_off.as<uint32_t>();
+  a.canonical = b->fmt == AVRF_FMT_CANONICAL;
+  a.pts = b->pts.as<BaseRec>(); a.cs = b->cs.as<uint32_t>(); a.status = dst.as<int32_t>(); a.n = (uint32_t)b->n;
+  DISPATCH(b->suite, (k_verify_each_ped<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
+  LAUNCHED("k_verify_each_ped");
   CK(cudaMemcpyAsync(statuses, dst.p, 4 * b->n, cudaMemcpyDeviceToHost, b->st));
   CK(hsync(b, b->st));
   return 0;

@@ -79,6 +79,52 @@ __global__ void __launch_bounds__(128) k_prove(ProveArgs a) {
   store_fe(a.s + j, s);
 }
 
+// pedersen::Prover::prove (src/pedersen.rs:136-186), one proof per thread: ped_prove_one_g (pedersen.cuh).
+struct PedProveArgs {
+  const Fe* sk;
+  const Affine* pk;
+  const Affine* ios;
+  const uint32_t* io_off;
+  const uint32_t* ad_off;
+  const uint8_t* ad;
+  Affine* pkcom;
+  Affine* r;
+  Affine* ok;
+  Fe* s;
+  Fe* sb;
+  Fe* blinding;             // may be null
+  uint32_t n;
+  int canonical;
+};
+
+template <int S>
+__global__ void __launch_bounds__(128) k_prove_ped(PedProveArgs a) {
+  constexpr int FR = SuiteT<S>::FR;
+  uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= a.n) return;
+  uint32_t io0 = a.io_off[j], m = a.io_off[j + 1] - io0;
+  Affine pk, PKC, R, OK;
+  load_affine_fmt<S>(pk, a.pk + j, a.canonical);
+  Fe sk, s, sb, bl;
+  load_fe(sk, a.sk + j);
+  if (!a.canonical) from_mont<FR>(sk, sk);
+  uint32_t ad0 = a.ad_off[j];
+  const Affine* base = a.ios + 2 * (size_t)io0;
+  int canonical = a.canonical;
+  ped_prove_one_g<S>(PKC, R, OK, s, sb, bl, sk, pk, [base, canonical](uint32_t k) {
+    Affine P;
+    load_affine_fmt<S>(P, base + k, canonical);
+    return P;
+  }, m, a.ad + ad0, a.ad_off[j + 1] - ad0);
+  store_affine_fmt<S>(a.pkcom + j, PKC, a.canonical);
+  store_affine_fmt<S>(a.r + j, R, a.canonical);
+  store_affine_fmt<S>(a.ok + j, OK, a.canonical);
+  if (!a.canonical) { to_mont<FR>(s, s); to_mont<FR>(sb, sb); to_mont<FR>(bl, bl); }
+  store_fe(a.s + j, s);
+  store_fe(a.sb + j, sb);
+  if (a.blinding) store_fe(a.blinding + j, bl);
+}
+
 template <int S>
 __global__ void __launch_bounds__(128) k_compress(const Affine* in, uint64_t n, uint32_t* out, int canonical, int hash) {
   uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -420,6 +466,57 @@ __global__ void __launch_bounds__(128) k_verify_each(EachArgs a) {
   ext_add_c<S>(q, q, e);                  // s I_m - c O_m - R
   (void)FQ;
   a.status[j] = bad ? AVRF_INVALID_DATA : (ext_is_identity<S>(q) ? AVRF_OK : AVRF_VERIFICATION_FAILURE);
+}
+
+// pedersen::Verifier::verify for every proof of a prepared Pedersen batch (src/pedersen.rs:188-253), one thread per
+// proof, reusing what k_prepare_ped left on the handle: c, s, sb (24 words per proof) and the bases O_m, Ok, I_m,
+// pk_com, R (an identity accumulator plus one mixed addition turns a base record back into the point, whatever the
+// suite's record layout).  The pushed pk_com and I/O points are read again only for the identity checks.
+struct PedEachArgs {
+  const Affine* pkcom;
+  const Affine* ios;
+  const uint32_t* io_off;
+  int canonical;
+  const BaseRec* pts;
+  const uint32_t* cs;
+  int32_t* status;
+  uint32_t n;
+};
+
+template <int S>
+__device__ __forceinline__ void base_to_ext(Ext& e, const BaseRec* b) {
+  Fe x, y, k;
+  load_fe(x, &b->x);
+  load_fe(y, &b->y);
+  load_fe(k, &b->k);
+  ext_identity<S>(e);
+  ext_madd<S>(e, x, y, k);
+}
+
+template <int S>
+__global__ void __launch_bounds__(128) k_verify_each_ped(PedEachArgs a) {
+  uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= a.n) return;
+  uint32_t io0 = a.io_off[j], m = a.io_off[j + 1] - io0;
+  Affine t;
+  load_affine_fmt<S>(t, a.pkcom + j, a.canonical);
+  bool bad = affine_is_identity<S>(t);
+  for (uint32_t i = 0; i < 2 * m; i++) {
+    load_affine_fmt<S>(t, a.ios + 2 * (size_t)io0 + i, a.canonical);
+    bad |= affine_is_identity<S>(t);
+  }
+  if (bad) { a.status[j] = AVRF_INVALID_DATA; return; }
+  const BaseRec* b = a.pts + 5 * (size_t)j;
+  const uint32_t* csj = a.cs + 24 * (size_t)j;
+  uint32_t c4[4] = {csj[0], csj[1], csj[2], csj[3]};
+  Fe s, sb;
+  for (int i = 0; i < 8; i++) { s.v[i] = csj[8 + i]; sb.v[i] = csj[16 + i]; }
+  // base records in the order O_m, Ok, I_m, pk_com, R (k_prepare_ped)
+  a.status[j] = ped_equations_hold<S>([b](int k) {
+    Ext e;
+    base_to_ext<S>(e, b + (k == PED_IM ? 2 : k == PED_OM ? 0 : k == PED_OK ? 1 : k));
+    return e;
+  }, c4, s, sb) ? AVRF_OK : AVRF_VERIFICATION_FAILURE;
 }
 
 }  // namespace avrf

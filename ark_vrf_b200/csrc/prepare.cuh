@@ -4,6 +4,7 @@
 //   k_tree_leaves  leaf digests of the opt-in tree seed (AVRF_WEIGHTS_TREE)
 #pragma once
 #include "msm.cuh"
+#include "pedersen.cuh"
 
 namespace avrf {
 // A field element of the ABI must be < p in either format (arkworks' types cannot hold anything else); anything
@@ -141,10 +142,9 @@ __global__ void __launch_bounds__(64) k_tree_leaves(const uint32_t* cs, uint32_t
   for (int i = 0; i < 8; i++) out[8 * (size_t)l + i] = bswap64(d[i]);     // digest bytes in memory order
 }
 
-// pedersen::BatchItem::new for one proof per thread (reference src/pedersen.rs:283-301): transcript
-// SUITE_ID || 0x02 || LE64(M) || pairs || LE64(|ad|) || ad (common.rs:159-173, no Schnorr pair), merged pair
-// (common.rs:181-202,389-419: (0,1),(0,1) for M = 0, the pair for M = 1, sum z_i (I_i, O_i) with z_0 = 1
-// otherwise, normalised), then || enc(Yb), c = challenge([R, Ok]).  Bases in the order of pedersen.rs:389-405.
+// pedersen::BatchItem::new for one proof per thread (reference src/pedersen.rs:283-301): the transcript and merged pair
+// of pedersen.cuh (the merged pair normalised here), then || enc(Yb), c = challenge([R, Ok]).  Bases in the order of
+// pedersen.rs:389-405.
 struct PedPrepArgs {
   const Affine* pkcom;
   const Affine* r;
@@ -173,47 +173,32 @@ __global__ void __launch_bounds__(128) k_prepare_ped(PedPrepArgs a) {
   bool bad = false;
   int oob = 0;                          // a coordinate or scalar >= its modulus: not a field element
   Sha512 t;
-  uint32_t enc[8];
+  uint32_t enc[8], enc2[8];
   Affine P, Im, Om;
   AffineK K;
-  sha512_init(t);
-  for (uint32_t i = 0; i < AVRF_CC(S).sid_len; i++) sha512_put_byte(t, AVRF_CC(S).suite_id[i]);
-  sha512_put_byte(t, 0x02);                            // DomSep::PedersenVrf
-  sha512_put_le64(t, m);
-  for (uint32_t i = 0; i < 2 * m; i++) {
-    load_affine_fmt<S>(P, a.ios + 2 * (size_t)io0 + i, a.canonical, &oob);
-    bad |= affine_is_identity<S>(P);
-    affine_compress<S>(enc, P);
-    sha512_put_words(t, enc);
-  }
+  const Affine* base = a.ios + 2 * (size_t)io0;
+  const int canonical = a.canonical;
   uint32_t ad0 = a.ad_off[j];
-  thin_transcript_ad(t, a.ad + ad0, a.ad_off[j + 1] - ad0);
+  ped_transcript<S>(t, m, [&](uint32_t k) {
+    Affine Q;
+    load_affine_fmt<S>(Q, base + k, canonical, &oob);
+    bad |= affine_is_identity<S>(Q);
+    return Q;
+  }, a.ad + ad0, a.ad_off[j + 1] - ad0);
+  auto get_io = [base, canonical](uint32_t k) {
+    Affine Q;
+    load_affine_fmt<S>(Q, base + k, canonical);
+    return Q;
+  };
   if (m == 0) {
     fe_zero(Im.x); fe_one<FQ>(Im.y);
     Om = Im;
   } else if (m == 1) {
-    load_affine_fmt<S>(Im, a.ios + 2 * (size_t)io0, a.canonical, &oob);
-    load_affine_fmt<S>(Om, a.ios + 2 * (size_t)io0 + 1, a.canonical, &oob);
+    Im = get_io(0);
+    Om = get_io(1);
   } else {
-    Ext im, om, e, q;
-    load_affine_fmt<S>(P, a.ios + 2 * (size_t)io0, a.canonical, &oob);
-    affine_to_ext<S>(im, P);
-    load_affine_fmt<S>(P, a.ios + 2 * (size_t)io0 + 1, a.canonical, &oob);
-    affine_to_ext<S>(om, P);
-    const Affine* base = a.ios + 2 * (size_t)io0;
-    int canonical = a.canonical;
-    thin_delinearize(t, m - 1, [&](uint32_t i, const uint32_t* z4) {      // z_1 .. z_{M-1}; z_0 = 1
-      uint32_t z8[8] = {z4[0], z4[1], z4[2], z4[3], 0, 0, 0, 0};
-      Affine Q;
-      load_affine_fmt<S>(Q, base + 2 * (i + 1), canonical);
-      affine_to_ext<S>(e, Q);
-      ext_scalar_mul<S>(q, e, z8, 128);
-      ext_add_c<S>(im, im, q);
-      load_affine_fmt<S>(Q, base + 2 * (i + 1) + 1, canonical);
-      affine_to_ext<S>(e, Q);
-      ext_scalar_mul<S>(q, e, z8, 128);
-      ext_add_c<S>(om, om, q);
-    });
+    Ext im, om;
+    ped_merge<S, true>(im, om, t, m, get_io);
     Fe zz, inv, zi, zo;                                 // normalize_batch: one inversion for both
     mont_mul_c<FQ>(zz, im.z, om.z);
     fe_inv<FQ>(inv, zz);
@@ -235,22 +220,16 @@ __global__ void __launch_bounds__(128) k_prepare_ped(PedPrepArgs a) {
   sha512_put_words(t, enc);
   affine_to_k<S>(K, P);
   store_affinek(out + 3, K);
-  sha512_put_byte(t, DOM_CHALLENGE);
   load_affine_fmt<S>(P, a.r + j, a.canonical, &oob);         // R
   affine_compress<S>(enc, P);
-  sha512_put_words(t, enc);
   affine_to_k<S>(K, P);
   store_affinek(out + 4, K);
   load_affine_fmt<S>(P, a.ok + j, a.canonical, &oob);        // Ok
-  affine_compress<S>(enc, P);
-  sha512_put_words(t, enc);
+  affine_compress<S>(enc2, P);
   affine_to_k<S>(K, P);
   store_affinek(out + 1, K);
-  uint64_t seed[8], blk[8];
-  sha512_final(t, seed);
-  sha512_xof_block(blk, seed, 0);
   uint32_t c4[4];
-  digest_le128(c4, blk, 0);
+  ped_challenge(t, enc, enc2, c4);
   Fe s, sb;
   load_fe(s, a.s + j);
   load_fe(sb, a.sb + j);

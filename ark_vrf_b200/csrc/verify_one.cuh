@@ -205,4 +205,49 @@ __global__ void __launch_bounds__(32) k_verify_one(OneArgs a) {
   }
 }
 
+// pedersen::Verifier::verify (src/pedersen.rs:188-253) for ONE proof: ped_verify_one_g (pedersen.cuh) on one thread.
+// Input: pk_com 64 | r 64 | ok 64 | s 32 | sb 32 | n_ios u32 | ad_len u32 | pad 8 | ios 128*M | ad.
+struct PedOneArgs {
+  const uint8_t* in;
+  int32_t* status;          // [0] verdict, [1] flags (2: a value is not a field element)
+  int canonical;
+};
+
+template <int S>
+__global__ void __launch_bounds__(32) k_verify_one_ped(PedOneArgs a) {
+  constexpr int FR = SuiteT<S>::FR;
+  if (threadIdx.x != 0) return;
+  const Affine* pts = reinterpret_cast<const Affine*>(a.in);
+  const Fe* sp = reinterpret_cast<const Fe*>(a.in + 192);
+  const uint32_t m = *reinterpret_cast<const uint32_t*>(a.in + 256);
+  const uint32_t ad_len = *reinterpret_cast<const uint32_t*>(a.in + 260);
+  const Affine* ios = reinterpret_cast<const Affine*>(a.in + 272);
+  const uint8_t* ad = a.in + 272 + 128 * (size_t)m;
+  const int canonical = a.canonical;
+  int oob = 0;
+  Affine PKC, R, OK;
+  load_affine_fmt<S>(PKC, pts + 0, canonical, &oob);
+  load_affine_fmt<S>(R, pts + 1, canonical, &oob);
+  load_affine_fmt<S>(OK, pts + 2, canonical, &oob);
+  for (uint32_t i = 0; i < 2 * m; i++) {
+    Affine P;
+    load_affine_fmt<S>(P, ios + i, canonical, &oob);
+  }
+  Fe s, sb;
+  load_fe(s, sp);
+  load_fe(sb, sp + 1);
+  oob |= !(fe_in_range<FR>(s) && fe_in_range<FR>(sb));
+  if (oob) {
+    a.status[1] = 2;
+    return;
+  }
+  if (!canonical) { from_mont<FR>(s, s); from_mont<FR>(sb, sb); }
+  a.status[0] = ped_verify_one_g<S>([ios, canonical](uint32_t k) {
+    Affine P;
+    load_affine_fmt<S>(P, ios + k, canonical);
+    return P;
+  }, m, ad, ad_len, PKC, R, OK, s, sb);
+  a.status[1] = 0;
+}
+
 }  // namespace avrf

@@ -6,6 +6,7 @@
     secret.output(input)        src/lib.rs:391-393    vrf_output(suite, sk, inputs)
     Secret::from_scalar().public src/lib.rs:331-334   public_keys(suite, sk)
     secret.prove(ios, ad)       src/thin.rs:111-129   thin_prove_many(...)
+    pedersen Prover::prove      src/pedersen.rs:136-186  pedersen_prove_many(...)
     point.serialize_compressed  ark-serialize         point_compress(suite, points)
     output.hash::<32>()         common.rs:290-305     point_to_hash(suite, points)
 
@@ -98,6 +99,19 @@ def thin_prove_many(suite, sk, pk, ios, io_offsets, ad_blob, ad_offsets, fmt=For
     _lib.check(lib.avrf_thin_prove_many(int(suite), int(fmt), n, ptr(sk), ptr(pk), ptr(ios), ptr(io_offsets),
                                         ptr(ad_blob), ptr(ad_offsets), ptr(r), ptr(s)))
     return r, s
+
+
+def pedersen_prove_many(suite, sk, pk, ios, io_offsets, ad_blob, ad_offsets, fmt=Format.CANONICAL):
+    """pedersen::Prover::prove for n proofs (arrays as for thin_prove_many).  Returns (pk_com, r, ok, s, sb, blinding):
+    (n,64) points and (n,32) scalars in `fmt`; `blinding` is the factor the reference returns beside each proof."""
+    lib = _lib.load()
+    n = len(io_offsets) - 1
+    pk_com, r, ok = (np.zeros((n, 64), dtype=np.uint8) for _ in range(3))
+    s, sb, blinding = (np.zeros((n, 32), dtype=np.uint8) for _ in range(3))
+    _lib.check(lib.avrf_pedersen_prove_many(int(suite), int(fmt), n, ptr(sk), ptr(pk), ptr(ios), ptr(io_offsets),
+                                            ptr(ad_blob), ptr(ad_offsets), ptr(pk_com), ptr(r), ptr(ok), ptr(s), ptr(sb),
+                                            ptr(blinding)))
+    return pk_com, r, ok, s, sb, blinding
 
 
 def point_compress(suite, points: np.ndarray, fmt=Format.CANONICAL) -> np.ndarray:

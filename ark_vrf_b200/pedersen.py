@@ -1,8 +1,11 @@
-"""Pedersen VRF batch verification on the same GPU engine (SURVEY.md 8f-3).
+"""Pedersen VRF on the GPU (SURVEY.md 8f-3): proving, single and batch verification.
 
-Mirror of `ark_vrf::pedersen::BatchVerifier` (reference src/pedersen.rs:322-427):
-`new()`, `push(ios, ad, proof)`, `push_prepared(item)`, `verify()`.  A proof is
-`(pk_com, r, ok, s, sb)` (pedersen.rs:43-50); the MSM has 5N+2 points."""
+Mirror of `ark_vrf::pedersen` (reference src/pedersen.rs):
+    Prover::prove                    prove_many(...)             (pedersen.rs:136-186, n proofs per call)
+    Verifier::verify                 verify(suite, ios, ad, proof)  (pedersen.rs:188-253, exact)
+    BatchVerifier::{new, push, push_prepared, verify}   BatchVerifier  (pedersen.rs:322-427; the MSM has 5N+2 points)
+    (per-proof verdicts)             BatchVerifier.verify_each() / find_invalid()
+A proof is `(pk_com, r, ok, s, sb)` (pedersen.rs:43-50)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -12,6 +15,7 @@ from typing import Union
 import numpy as np
 
 from . import _lib
+from .ops import pedersen_prove_many as prove_many          # noqa: F401  (re-exported: pedersen.prove_many)
 from .thin import Format, Suite, Tap, _bytes_of, _ios_bytes, _raise_for_status, ptr
 
 
@@ -77,6 +81,16 @@ class BatchVerifier:
     def verify(self) -> None:
         _raise_for_status(self.verify_status())
 
+    def verify_each(self) -> np.ndarray:
+        """Per-proof status codes (0 Ok, 1 VerificationFailure, 2 InvalidData) under `pedersen::Verifier::verify`."""
+        out = np.full(max(self._n, 1), -1, dtype=np.int32)
+        _lib.check(self._lib.avrf_pedersen_batch_verify_each(self._h, ptr(out)))
+        return out[:self._n]
+
+    def find_invalid(self) -> np.ndarray:
+        """Indices of the proofs a failed batch owes its verdict to; empty when every proof verifies."""
+        return np.nonzero(self.verify_each() != 0)[0]
+
     def tap(self, what: Tap) -> np.ndarray:
         n = self._n
         size = {Tap.C: 16 * n, Tap.W: 32 * n, Tap.SEED: 64, Tap.SCALARS: 32 * (5 * n + 2)}[Tap(what)]
@@ -97,3 +111,16 @@ class BatchVerifier:
             self.close()
         except Exception:
             pass
+
+
+def verify(suite: Union[Suite, int], ios, ad, proof: Proof, fmt: Union[Format, int] = Format.CANONICAL) -> None:
+    """`pedersen::Verifier::verify` (src/pedersen.rs:188-253) for one proof: returns None, or raises VerificationFailure
+    / InvalidData like `thin.Public.verify`."""
+    lib = _lib.load()
+    iob, k = _ios_bytes(ios)
+    st = C.c_int32(-1)
+    _lib.check(lib.avrf_pedersen_verify_one(int(Suite(suite)), int(Format(fmt)), iob if k else None, k,
+                                            bytes(ad) if ad else None, len(ad), _bytes_of(proof.pk_com, 64),
+                                            _bytes_of(proof.r, 64), _bytes_of(proof.ok, 64), _bytes_of(proof.s, 32),
+                                            _bytes_of(proof.sb, 32), C.byref(st)))
+    _raise_for_status(st.value)

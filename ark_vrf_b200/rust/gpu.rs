@@ -1,4 +1,5 @@
-//! `ark_vrf::gpu` - B200 batch verification of the Thin VRF behind the reference's own API.
+//! `ark_vrf::gpu` - B200 batch verification of the Thin VRF (and the Pedersen VRF, `gpu::pedersen`) behind the
+//! reference's own API.
 //!
 //! Drop this file in as `src/gpu.rs` of davxy/ark-vrf 0.5.3, add `pub mod gpu;` to `src/lib.rs`
 //! behind a `gpu` cargo feature, and link `libavrf_gpu.so` (see INTEGRATION.md).  It keeps the
@@ -65,6 +66,18 @@ extern "C" {
         ad_blob: *const u8, ad_offsets: *const u32, r: *const u8, s: *const u8,
     ) -> i32;
     fn avrf_thin_sharded_verify(sh: *mut AvrfSharded, status: *mut i32) -> i32;
+    fn avrf_thin_batch_len(b: *const AvrfBatch) -> i64;
+    fn avrf_pedersen_batch_new(suite: u32, fmt: u32) -> *mut AvrfBatch;
+    fn avrf_pedersen_batch_push_many(
+        b: *mut AvrfBatch, n: u64, ios: *const u8, io_offsets: *const u32, ad_blob: *const u8,
+        ad_offsets: *const u32, pk_com: *const u8, r: *const u8, ok: *const u8, s: *const u8, sb: *const u8,
+    ) -> i32;
+    fn avrf_pedersen_batch_verify(b: *mut AvrfBatch, status: *mut i32) -> i32;
+    fn avrf_pedersen_batch_verify_each(b: *mut AvrfBatch, statuses: *mut i32) -> i32;
+    fn avrf_pedersen_verify_one(
+        suite: u32, fmt: u32, ios: *const u8, n_ios: u32, ad: *const u8, ad_len: u32, pk_com: *const u8,
+        r: *const u8, ok: *const u8, s: *const u8, sb: *const u8, status: *mut i32,
+    ) -> i32;
 }
 
 #[repr(C)]
@@ -404,3 +417,88 @@ impl<S: GpuSuite> Drop for ShardedBatchVerifier<S> {
     }
 }
 unsafe impl<S: GpuSuite> Send for ShardedBatchVerifier<S> {}
+
+/// `pedersen::Verifier` and `pedersen::BatchVerifier` (src/pedersen.rs:188-253, 322-427) on the GPU, with per-proof
+/// verdicts after a failed batch.  The proof's five fields are passed one by one (each an arkworks memory image, as
+/// checked by `layout_self_check`), so `pedersen::Proof`'s own layout does not matter.
+pub mod pedersen {
+    use super::*;
+    use crate::pedersen::{PedersenSuite, Proof};
+
+    /// `pedersen::Verifier::verify` for one proof: exact, both equations (`avrf_pedersen_verify_one`).
+    pub fn verify<S: GpuSuite + PedersenSuite>(
+        ios: impl AsRef<[VrfIo<S>]>, ad: impl AsRef<[u8]>, proof: &Proof<S>,
+    ) -> Result<(), Error> {
+        let (ios, ad) = (ios.as_ref(), ad.as_ref());
+        let mut status = -1i32;
+        let rc = unsafe {
+            avrf_pedersen_verify_one(
+                S::AVRF_SUITE, AVRF_FMT_MONTGOMERY, ios.as_ptr() as *const u8, ios.len() as u32, ad.as_ptr(),
+                ad.len() as u32, point_bytes::<S>(&proof.pk_com), point_bytes::<S>(&proof.r),
+                point_bytes::<S>(&proof.ok), scalar_bytes::<S>(&proof.s), scalar_bytes::<S>(&proof.sb), &mut status,
+            )
+        };
+        status_to_result(rc, status)
+    }
+
+    /// `pedersen::BatchVerifier` on one B200.
+    pub struct BatchVerifier<S: GpuSuite + PedersenSuite> {
+        h: *mut AvrfBatch,
+        _s: PhantomData<S>,
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Default for BatchVerifier<S> {
+        fn default() -> Self {
+            Self::new()
+        }
+    }
+
+    impl<S: GpuSuite + PedersenSuite> BatchVerifier<S> {
+        pub fn new() -> Self {
+            let h = unsafe {
+                avrf_init(0);
+                avrf_pedersen_batch_new(S::AVRF_SUITE, AVRF_FMT_MONTGOMERY)
+            };
+            assert!(!h.is_null(), "avrf_pedersen_batch_new failed (no CUDA device?)");
+            static CHECKED: std::sync::Once = std::sync::Once::new();
+            CHECKED.call_once(layout_self_check::<S>);
+            Self { h, _s: PhantomData }
+        }
+
+        pub fn push(&mut self, ios: impl AsRef<[VrfIo<S>]>, ad: impl AsRef<[u8]>, proof: &Proof<S>) {
+            let (ios, ad) = (ios.as_ref(), ad.as_ref());
+            let io_off = [0u32, ios.len() as u32];
+            let ad_off = [0u32, ad.len() as u32];
+            let rc = unsafe {
+                avrf_pedersen_batch_push_many(
+                    self.h, 1, ios.as_ptr() as *const u8, io_off.as_ptr(), ad.as_ptr(), ad_off.as_ptr(),
+                    point_bytes::<S>(&proof.pk_com), point_bytes::<S>(&proof.r), point_bytes::<S>(&proof.ok),
+                    scalar_bytes::<S>(&proof.s), scalar_bytes::<S>(&proof.sb),
+                )
+            };
+            assert!(rc == 0, "libavrf_gpu system error {rc}");
+        }
+
+        /// Same contract as `pedersen::BatchVerifier::verify` (src/pedersen.rs:341-426).
+        pub fn verify(&self) -> Result<(), Error> {
+            let mut status = -1i32;
+            let rc = unsafe { avrf_pedersen_batch_verify(self.h, &mut status) };
+            status_to_result(rc, status)
+        }
+
+        /// `pedersen::Verifier::verify` of every pushed proof, in push order: names the offenders of a failed batch.
+        pub fn verify_each(&self) -> Vec<Result<(), Error>> {
+            let n = unsafe { avrf_thin_batch_len(self.h) } as usize;
+            let mut st = vec![-1i32; n];
+            let rc = unsafe { avrf_pedersen_batch_verify_each(self.h, st.as_mut_ptr()) };
+            st.into_iter().map(|s| status_to_result(rc, s)).collect()
+        }
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Drop for BatchVerifier<S> {
+        fn drop(&mut self) {
+            unsafe { avrf_thin_batch_free(self.h) }
+        }
+    }
+    unsafe impl<S: GpuSuite + PedersenSuite> Send for BatchVerifier<S> {}
+}

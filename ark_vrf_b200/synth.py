@@ -1,9 +1,9 @@
-"""Synthetic Thin-VRF workloads (SURVEY.md section 8d), generated on the GPU.
+"""Synthetic Thin- and Pedersen-VRF workloads (SURVEY.md section 8d), generated on the GPU.
 
 Signer k has sk_k = Secret::from_seed(LE64(k) || 0^24) (reference src/lib.rs:346-369);
 proof j is signed by k = j mod K; inputs I_{j,i} = data_to_point(LE64(j) || LE32(i));
 O = sk * I; ad_j = b"ad-{j}" (reference benches/thin.rs:55); proofs by the reference's
-deterministic prove (src/thin.rs:111-129).  Only `secret_from_seed` (two SHA-512 calls per
+deterministic prove (src/thin.rs:111-129; make_pedersen_batch: src/pedersen.rs:136-186).  Only `secret_from_seed` (two SHA-512 calls per
 signer) runs on the host; everything else uses the library's feeder kernels.
 """
 from __future__ import annotations
@@ -92,10 +92,8 @@ def _mont_scalars(suite: Suite, sk_ints) -> np.ndarray:
     return np.frombuffer(b"".join(((k << 256) % r).to_bytes(32, "little") for k in sk_ints), dtype=np.uint8).reshape(-1, 32).copy()
 
 
-def make_batch(suite, n: int, m: int = 1, signers: int = 4096, fmt: Format = Format.MONTGOMERY,
-               first: int = 0) -> Batch:
-    """Proofs first .. first+n-1 of the synthetic set, as host arrays in `fmt`."""
-    suite = Suite(suite)
+def _inputs(suite: Suite, n: int, m: int, signers: int, fmt: Format, first: int):
+    """Signer keys, I/O pairs and ad of proofs first .. first+n-1 (shared by the Thin and Pedersen generators)."""
     K = max(1, min(signers, 4096))
     sk_int = [secret_from_seed(suite, k.to_bytes(8, "little") + bytes(24)) for k in range(K)]
     sk_can = np.frombuffer(b"".join(k.to_bytes(32, "little") for k in sk_int), dtype=np.uint8).reshape(K, 32)
@@ -123,8 +121,47 @@ def make_batch(suite, n: int, m: int = 1, signers: int = 4096, fmt: Format = For
     ad_offsets = np.zeros(n + 1, dtype=np.uint32)
     ad_offsets[1:] = np.cumsum([len(a) for a in ads], dtype=np.uint64).astype(np.uint32)
     ad_blob = np.frombuffer(b"".join(ads) + bytes(16), dtype=np.uint8).copy()
+    return sk, pk, ios, io_offsets, ad_blob, ad_offsets
+
+
+def make_batch(suite, n: int, m: int = 1, signers: int = 4096, fmt: Format = Format.MONTGOMERY,
+               first: int = 0) -> Batch:
+    """Proofs first .. first+n-1 of the synthetic set, as host arrays in `fmt`."""
+    suite = Suite(suite)
+    sk, pk, ios, io_offsets, ad_blob, ad_offsets = _inputs(suite, n, m, signers, fmt, first)
     r, s = ops.thin_prove_many(suite, sk, pk, ios, io_offsets, ad_blob, ad_offsets, fmt)
     return Batch(suite, Format(fmt), n, m, pk, ios, io_offsets, ad_blob, ad_offsets, r, s, sk)
+
+
+@dataclass
+class PedersenBatch:
+    suite: Suite
+    fmt: Format
+    n: int
+    m: int
+    ios: np.ndarray         # (n*m, 128)  input || output
+    io_offsets: np.ndarray  # (n+1,) uint32
+    ad_blob: np.ndarray     # uint8
+    ad_offsets: np.ndarray  # (n+1,) uint32
+    pk_com: np.ndarray      # (n, 64)
+    r: np.ndarray           # (n, 64)
+    ok: np.ndarray          # (n, 64)
+    s: np.ndarray           # (n, 32)
+    sb: np.ndarray          # (n, 32)
+    blinding: np.ndarray    # (n, 32) the blinding factor of each proof
+    sk: np.ndarray          # (n, 32) per proof, in `fmt`
+    pk: np.ndarray          # (n, 64) sk * G
+
+
+def make_pedersen_batch(suite, n: int, m: int = 1, signers: int = 4096, fmt: Format = Format.MONTGOMERY,
+                        first: int = 0) -> PedersenBatch:
+    """The Pedersen twin of `make_batch`: the same signers, messages and ad, proofs by the GPU's
+    pedersen::Prover::prove (src/pedersen.rs:136-186)."""
+    suite = Suite(suite)
+    sk, pk, ios, io_offsets, ad_blob, ad_offsets = _inputs(suite, n, m, signers, fmt, first)
+    pk_com, r, ok, s, sb, blinding = ops.pedersen_prove_many(suite, sk, pk, ios, io_offsets, ad_blob, ad_offsets, fmt)
+    return PedersenBatch(suite, Format(fmt), n, m, ios, io_offsets, ad_blob, ad_offsets, pk_com, r, ok, s, sb, blinding,
+                         sk, pk)
 
 
 def splitmix64(x: int) -> int:

@@ -250,6 +250,21 @@ int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios,
                                   const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);
 int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status);
 
+/* pedersen::Verifier::verify (src/pedersen.rs:188-253) for every proof pushed to a Pedersen handle: statuses[j] in
+ * {AVRF_OK, AVRF_VERIFICATION_FAILURE, AVRF_INVALID_DATA}, each proof judged on its own as avrf_pedersen_verify_one
+ * would.  Use after a failed batch to name the offenders.  Runs on the handle's stream; a Thin handle is an argument
+ * error (and avrf_thin_batch_verify_each refuses Pedersen handles). */
+int avrf_pedersen_batch_verify_each(avrf_batch* b, int32_t* statuses);
+
+/* pedersen::Verifier::verify (src/pedersen.rs:188-253) for ONE proof, exact: InvalidData when pk_com or an I/O point
+ * is the identity (before any equation), otherwise Ok when BOTH s*I_m - c*O_m == Ok and s*G + sb*B - c*pk_com == R
+ * hold, each tested with integer scalars and no batch weight (exact on every curve point, in the prime-order subgroup
+ * or not).  A coordinate >= p or s / sb >= r is AVRF_ERR_ARG (status untouched).  Uses a per-thread context, as
+ * avrf_thin_verify_one does; latency-bound (use a batch for throughput). */
+int avrf_pedersen_verify_one(uint32_t suite, uint32_t fmt, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
+                             uint32_t ad_len, const uint8_t pk_com[64], const uint8_t r[64], const uint8_t ok[64],
+                             const uint8_t s[32], const uint8_t sb[32], int32_t* status);
+
 /* ---- Feeder operations (inputs of the hot path; also the synthetic-data generator) ------ */
 
 /* Input::new -> Suite::data_to_point (src/lib.rs:500-502; Elligator2-XMD for Bandersnatch,
@@ -279,6 +294,14 @@ int avrf_public_keys(uint32_t suite, uint32_t fmt, const uint8_t* sk, uint64_t n
 int avrf_thin_prove_many(uint32_t suite, uint32_t fmt, uint64_t n, const uint8_t* sk, const uint8_t* pk,
                          const uint8_t* ios, const uint32_t* io_offsets, const uint8_t* ad_blob,
                          const uint32_t* ad_offsets, uint8_t* r, uint8_t* s);
+
+/* pedersen::Prover::prove (src/pedersen.rs:136-186) for n proofs; layout as avrf_thin_prove_many (pk = sk*G).
+ * Outputs in `fmt`: pk_com, r, ok (64 B each), s, sb (32 B each); blinding (32 B each, may be NULL) = the blinding
+ * factor the reference returns beside the proof. */
+int avrf_pedersen_prove_many(uint32_t suite, uint32_t fmt, uint64_t n, const uint8_t* sk, const uint8_t* pk,
+                             const uint8_t* ios, const uint32_t* io_offsets, const uint8_t* ad_blob,
+                             const uint32_t* ad_offsets, uint8_t* pk_com, uint8_t* r, uint8_t* ok, uint8_t* s,
+                             uint8_t* sb, uint8_t* blinding);
 
 /* CanonicalSerialize of affine points (ark-serialize compressed; src/utils/transcript.rs:48-50). */
 int avrf_point_compress(uint32_t suite, uint32_t fmt, const uint8_t* points, uint64_t n, uint8_t* out32);

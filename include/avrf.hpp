@@ -7,6 +7,10 @@
 //   Public<S>::verify  (thin::Verifier)           src/thin.rs:95-109,131-165
 //   thin::BatchServer<S>::{submit, wait}          (new: worker pool over avrf_server_*, throughput mode)
 //   thin::ShardedBatchVerifier<S>                 (new: one batch over several GPUs of this process, avrf_thin_sharded_*)
+//   pedersen::Proof{pk_com, r, ok, s, sb}         src/pedersen.rs:43-50
+//   pedersen::verify (pedersen::Verifier)         src/pedersen.rs:188-253
+//   pedersen::BatchVerifier<S>::{push, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
+//   pedersen::prove_many (Prover::prove, n proofs) src/pedersen.rs:136-186
 //   Error::{VerificationFailure, InvalidData}     src/lib.rs:136-147
 //
 // The host toolchain of the reference (Rust) is absent from the build image, so this header is the
@@ -181,6 +185,88 @@ class BatchServer {
 };
 
 }  // namespace thin
+
+namespace pedersen {
+
+struct Proof { AffinePoint pk_com, r, ok; ScalarField s, sb; };   // src/pedersen.rs:43-50
+static_assert(sizeof(Proof) == 256, "pedersen::Proof must be five contiguous fields");
+
+// pedersen::Verifier::verify (src/pedersen.rs:188-253) for one proof: exact, both equations (avrf_pedersen_verify_one).
+template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
+Result verify(const std::vector<VrfIo>& ios, const std::vector<uint8_t>& ad, const Proof& proof) {
+  int32_t st = -1;
+  check(avrf_pedersen_verify_one(S::ID, FMT, ios.empty() ? nullptr : ios[0].input.data(), (uint32_t)ios.size(),
+                                 ad.empty() ? nullptr : ad.data(), (uint32_t)ad.size(), proof.pk_com.data(), proof.r.data(),
+                                 proof.ok.data(), proof.s.data(), proof.sb.data(), &st));
+  return Result{st};
+}
+
+// pedersen::BatchVerifier (src/pedersen.rs:322-427), plus per-proof verdicts after a failed batch.
+template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
+class BatchVerifier {
+ public:
+  BatchVerifier() : h_(avrf_pedersen_batch_new(S::ID, FMT)) { if (!h_) throw std::runtime_error(avrf_last_error()); }
+  ~BatchVerifier() { avrf_thin_batch_free(h_); }
+  BatchVerifier(const BatchVerifier&) = delete;
+  BatchVerifier& operator=(const BatchVerifier&) = delete;
+  int64_t len() const { return avrf_thin_batch_len(h_); }
+  void clear() { check(avrf_thin_batch_clear(h_)); }
+  void push(const std::vector<VrfIo>& ios, const std::vector<uint8_t>& ad, const Proof& proof) {
+    uint32_t io_off[2] = {0, (uint32_t)ios.size()}, ad_off[2] = {0, (uint32_t)ad.size()};
+    check(avrf_pedersen_batch_push_many(h_, 1, ios.empty() ? nullptr : ios[0].input.data(), io_off,
+                                        ad.empty() ? nullptr : ad.data(), ad_off, proof.pk_com.data(), proof.r.data(),
+                                        proof.ok.data(), proof.s.data(), proof.sb.data()));
+  }
+  Result verify() const {
+    int32_t st = -1;
+    check(avrf_pedersen_batch_verify(h_, &st));
+    return Result{st};
+  }
+  // statuses[j] = pedersen::Verifier::verify of proof j (AVRF_OK / AVRF_VERIFICATION_FAILURE / AVRF_INVALID_DATA)
+  std::vector<int32_t> verify_each() const {
+    std::vector<int32_t> st((size_t)len(), -1);
+    check(avrf_pedersen_batch_verify_each(h_, st.empty() ? nullptr : st.data()));
+    return st;
+  }
+  std::vector<size_t> find_invalid() const {
+    std::vector<size_t> bad;
+    std::vector<int32_t> st = verify_each();
+    for (size_t j = 0; j < st.size(); j++)
+      if (st[j] != AVRF_OK) bad.push_back(j);
+    return bad;
+  }
+  avrf_batch* handle() const { return h_; }
+
+ private:
+  avrf_batch* h_;
+};
+
+struct Proven { std::vector<Proof> proofs; std::vector<ScalarField> blinding; };
+
+// pedersen::Prover::prove (src/pedersen.rs:136-186) for n = sk.size() proofs (avrf_pedersen_prove_many): proof j signs
+// pairs ios[io_offsets[j] ..] and ad[ad_offsets[j] ..] with sk[j]; pk[j] = sk[j] * G.
+template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
+Proven prove_many(const std::vector<ScalarField>& sk, const std::vector<AffinePoint>& pk, const std::vector<VrfIo>& ios,
+                  const std::vector<uint32_t>& io_offsets, const std::vector<uint8_t>& ad,
+                  const std::vector<uint32_t>& ad_offsets) {
+  const size_t n = sk.size();
+  if (pk.size() != n || io_offsets.size() != n + 1 || ad_offsets.size() != n + 1)
+    throw std::invalid_argument("prove_many: sk, pk and the offsets must describe the same proofs");
+  std::vector<AffinePoint> pkc(n), r(n), ok(n);
+  std::vector<ScalarField> s(n), sb(n);
+  Proven out;
+  out.blinding.resize(n);
+  check(avrf_pedersen_prove_many(S::ID, FMT, n, n ? sk[0].data() : nullptr, n ? pk[0].data() : nullptr,
+                                 ios.empty() ? nullptr : ios[0].input.data(), io_offsets.data(),
+                                 ad.empty() ? nullptr : ad.data(), ad_offsets.data(), n ? pkc[0].data() : nullptr,
+                                 n ? r[0].data() : nullptr, n ? ok[0].data() : nullptr, n ? s[0].data() : nullptr,
+                                 n ? sb[0].data() : nullptr, n ? out.blinding[0].data() : nullptr));
+  out.proofs.resize(n);
+  for (size_t j = 0; j < n; j++) out.proofs[j] = Proof{pkc[j], r[j], ok[j], s[j], sb[j]};
+  return out;
+}
+
+}  // namespace pedersen
 
 template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
 struct Public {                      // Public<S> with thin::Verifier::verify
