@@ -93,6 +93,7 @@ SIGNATURES = {
     "avrf_thin_sharded_shard": (C.c_void_p, [C.c_void_p, C.c_int]),
     "avrf_pedersen_batch_new": (C.c_void_p, [C.c_uint32, C.c_uint32]),
     "avrf_pedersen_batch_push_many": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
+    "avrf_pedersen_batch_push_compressed": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 7),
     "avrf_pedersen_batch_verify": (C.c_int, [C.c_void_p, i32p]),
     "avrf_pedersen_batch_verify_each": (C.c_int, [C.c_void_p, C.c_void_p]),
     "avrf_pedersen_verify_one": (C.c_int, [C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32,

@@ -12,6 +12,7 @@
 //   Prover::prove      src/thin.rs:111-129      -> k_prove      (synthetic-input generator)
 //   pedersen::Prover::prove      src/pedersen.rs:136-186 -> k_prove_ped
 //   pedersen::Verifier::verify   src/pedersen.rs:188-253 -> k_verify_one_ped, k_verify_each_ped (per-proof verdicts)
+//   pedersen Proof::deserialize_compressed (wire push) -> k_ped_wire_unpack, k_dec_prep/k_dec_finish, k_ped_proof_ok
 // There is no CPU fallback: without a CUDA device every compute entry point fails.
 #include <cstdlib>
 #include <map>
@@ -543,8 +544,8 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
     CK(cudaMemcpyAsync(b->r.as<uint8_t>() + 64 * n0, r, 64 * n, cudaMemcpyDefault, b->st));
     CK(cudaMemcpyAsync(b->s.as<uint8_t>() + 32 * n0, s, 32 * n, cudaMemcpyDefault, b->st));
     if (ped) {
-      CK(cudaMemcpyAsync(b->ok.as<uint8_t>() + 64 * n0, ok, 64 * n, cudaMemcpyHostToDevice, b->st));
-      CK(cudaMemcpyAsync(b->sb.as<uint8_t>() + 32 * n0, sb, 32 * n, cudaMemcpyHostToDevice, b->st));
+      CK(cudaMemcpyAsync(b->ok.as<uint8_t>() + 64 * n0, ok, 64 * n, cudaMemcpyDefault, b->st));
+      CK(cudaMemcpyAsync(b->sb.as<uint8_t>() + 32 * n0, sb, 32 * n, cudaMemcpyDefault, b->st));
     }
     if (add_ios) CK(cudaMemcpyAsync(b->ios.as<uint8_t>() + 128 * i0, ios, 128 * add_ios, cudaMemcpyDefault, b->st));
     if (add_ad) CK(cudaMemcpyAsync(b->ad.as<uint8_t>() + a0, ad_blob, add_ad, cudaMemcpyDefault, b->st));

@@ -407,6 +407,40 @@ __global__ void __launch_bounds__(256) k_proof_ok(const uint8_t* ok_r, const uin
   if (!g) atomicAdd(n_bad, 1ull);
 }
 
+// Wire-format Pedersen proofs (pedersen::Proof::serialize_compressed, src/pedersen.rs:43-50): n records of 160 bytes,
+// pk_com | r | ok | s | sb.  The three point encodings go to enc as pk_com (n) | R (n) | Ok (n), ahead of the I/O
+// encodings the caller copies behind them, and the two scalars to sc as s (n) | sb (n).  One thread per 16-byte word:
+// the loads are coalesced across the records.
+__global__ void __launch_bounds__(256) k_ped_wire_unpack(const uint4* rec, uint64_t n, uint4* enc, uint4* sc) {
+  uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= 10 * n) return;
+  uint64_t j = t / 10;
+  uint32_t w = (uint32_t)(t - 10 * j), field = w >> 1, half = w & 1;
+  uint4 v = rec[t];
+  if (field < 3) enc[2 * (field * n + j) + half] = v;
+  else sc[2 * ((field - 3) * n + j) + half] = v;
+}
+
+// Per-proof decode verdict of a wire-format Pedersen push: proof j is good when pk_com, R and Ok decoded
+// (ok_pts: pk_com (n) | R (n) | Ok (n)), every point of its I/O pairs decoded, and s, sb are canonical scalars (< r),
+// which `Fr::deserialize_compressed` demands.
+template <int S>
+__global__ void __launch_bounds__(256) k_ped_proof_ok(const uint8_t* ok_pts, const uint8_t* ok_ios, const uint32_t* io_off,
+                                                      uint32_t io_base, const Fe* sc, uint64_t n, uint8_t* ok,
+                                                      unsigned long long* n_bad) {
+  constexpr int FR = SuiteT<S>::FR;
+  uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  uint8_t g = ok_pts[j] & ok_pts[n + j] & ok_pts[2 * n + j];
+  for (uint32_t i = 2 * (io_off[j] - io_base); i < 2 * (io_off[j + 1] - io_base); i++) g &= ok_ios[i];
+  Fe s, sb;
+  load_fe(s, sc + j);
+  load_fe(sb, sc + n + j);
+  if (!(fe_in_range<FR>(s) && fe_in_range<FR>(sb))) g = 0;
+  ok[j] = g;
+  if (!g) atomicAdd(n_bad, 1ull);
+}
+
 // thin::Verifier::verify for every proof of a prepared batch (src/thin.rs:131-165), one thread per
 // proof, reusing c_j and z_ij of k_prepare: status 0 Ok / 1 VerificationFailure / 2 InvalidData.
 struct EachArgs {

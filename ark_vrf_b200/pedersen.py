@@ -4,6 +4,7 @@ Mirror of `ark_vrf::pedersen` (reference src/pedersen.rs):
     Prover::prove                    prove_many(...)             (pedersen.rs:136-186, n proofs per call)
     Verifier::verify                 verify(suite, ios, ad, proof)  (pedersen.rs:188-253, exact)
     BatchVerifier::{new, push, push_prepared, verify}   BatchVerifier  (pedersen.rs:322-427; the MSM has 5N+2 points)
+    (wire-format proofs)             BatchVerifier.push_compressed(), serialize_proofs()  (Proof::{de,}serialize_compressed)
     (per-proof verdicts)             BatchVerifier.verify_each() / find_invalid()
 A proof is `(pk_com, r, ok, s, sb)` (pedersen.rs:43-50)."""
 from __future__ import annotations
@@ -16,6 +17,8 @@ import numpy as np
 
 from . import _lib
 from .ops import pedersen_prove_many as prove_many          # noqa: F401  (re-exported: pedersen.prove_many)
+from .ops import point_compress
+from .synth import ORDER
 from .thin import Format, Suite, Tap, _bytes_of, _ios_bytes, _raise_for_status, ptr
 
 
@@ -67,6 +70,21 @@ class BatchVerifier:
         _lib.check(self._lib.avrf_pedersen_batch_push_many(self._h, n, ptr(ios), ptr(io_offsets), ptr(ad_blob),
                                                            ptr(ad_offsets), ptr(pk_com), ptr(r), ptr(ok), ptr(s), ptr(sb)))
         self._n += n
+
+    def push_compressed(self, ios32, io_offsets, ad_blob, ad_offsets, proofs) -> np.ndarray:
+        """`avrf_pedersen_batch_push_compressed`: proofs in wire format, (n, 160) records of
+        `Proof::serialize_compressed` (see `serialize_proofs`), and 64 bytes of compressed (input, output) per pair;
+        decoded and validated on the device.  Returns the per-proof decode flags; when any is 0 nothing was pushed -
+        those proofs are the ones `Proof::deserialize_compressed` / `Input` / `Output` deserialisation would refuse."""
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        ok = np.zeros(max(n, 1), dtype=np.uint8)
+        bad = C.c_uint64(0)
+        _lib.check(self._lib.avrf_pedersen_batch_push_compressed(self._h, n, ptr(ios32), ptr(io_offsets), ptr(ad_blob),
+                                                                 ptr(ad_offsets), ptr(proofs), ptr(ok), C.byref(bad)))
+        if bad.value == 0:
+            self._n += n
+        return ok[:n]
 
     def clear(self) -> None:
         """Forget all pushed proofs, keep allocations."""
@@ -124,3 +142,26 @@ def verify(suite: Union[Suite, int], ios, ad, proof: Proof, fmt: Union[Format, i
                                             _bytes_of(proof.r, 64), _bytes_of(proof.ok, 64), _bytes_of(proof.s, 32),
                                             _bytes_of(proof.sb, 32), C.byref(st)))
     _raise_for_status(st.value)
+
+
+def serialize_proofs(suite: Union[Suite, int], pk_com, r, ok, s, sb, fmt: Union[Format, int] = Format.CANONICAL) -> np.ndarray:
+    """`pedersen::Proof::serialize_compressed` for n proofs: (n, 64) points and (n, 32) scalars in `fmt` (the arrays
+    `prove_many` returns) -> (n, 160) uint8 records pk_com | r | ok | s | sb, as `BatchVerifier.push_compressed` takes
+    them.  The points are compressed on the device; Montgomery scalars are converted to canonical on the host."""
+    suite, fmt = Suite(suite), Format(fmt)
+    pts = np.ascontiguousarray(np.stack([np.asarray(x, dtype=np.uint8).reshape(-1, 64) for x in (pk_com, r, ok)], axis=1))
+    n = pts.shape[0]
+    out = np.empty((n, 160), dtype=np.uint8)
+    out[:, :96] = point_compress(suite, pts.reshape(-1, 64), fmt).reshape(n, 96)
+    for k, x in enumerate((s, sb)):
+        x = np.ascontiguousarray(x, dtype=np.uint8).reshape(n, 32)
+        out[:, 96 + 32 * k:128 + 32 * k] = x if fmt == Format.CANONICAL else _from_mont_scalars(suite, x)
+    return out
+
+
+def _from_mont_scalars(suite: Suite, x: np.ndarray) -> np.ndarray:
+    """(n, 32) Montgomery-form scalars (a * 2^256 mod r) -> canonical little-endian."""
+    mod = ORDER[suite]
+    rinv = pow(1 << 256, -1, mod)
+    return np.frombuffer(b"".join((int.from_bytes(bytes(v), "little") * rinv % mod).to_bytes(32, "little") for v in x),
+                         dtype=np.uint8).reshape(-1, 32).copy()

@@ -72,6 +72,10 @@ extern "C" {
         b: *mut AvrfBatch, n: u64, ios: *const u8, io_offsets: *const u32, ad_blob: *const u8,
         ad_offsets: *const u32, pk_com: *const u8, r: *const u8, ok: *const u8, s: *const u8, sb: *const u8,
     ) -> i32;
+    fn avrf_pedersen_batch_push_compressed(
+        b: *mut AvrfBatch, n: u64, ios32: *const u8, io_offsets: *const u32, ad_blob: *const u8,
+        ad_offsets: *const u32, proofs: *const u8, ok: *mut u8, n_bad: *mut u64,
+    ) -> i32;
     fn avrf_pedersen_batch_verify(b: *mut AvrfBatch, status: *mut i32) -> i32;
     fn avrf_pedersen_batch_verify_each(b: *mut AvrfBatch, statuses: *mut i32) -> i32;
     fn avrf_pedersen_verify_one(
@@ -477,6 +481,28 @@ pub mod pedersen {
                 )
             };
             assert!(rc == 0, "libavrf_gpu system error {rc}");
+        }
+
+        /// Proofs in wire format: `Proof::serialize_compressed` records (pk_com | r | ok | s | sb, 160 bytes) and
+        /// compressed (input, output) pairs, decoded and validated on the GPU as `Proof::deserialize_compressed` and the
+        /// `Input` / `Output` deserialisers would on the CPU.  Returns the number of proofs that do not deserialize;
+        /// when it is not zero NOTHING was pushed and `ok[j] == 0` names them.
+        pub fn push_compressed(
+            &mut self, ios32: &[[u8; 64]], io_offsets: &[u32], ad_blob: &[u8], ad_offsets: &[u32],
+            proofs: &[[u8; 160]], ok: Option<&mut [u8]>,
+        ) -> u64 {
+            let n = proofs.len();
+            assert!(io_offsets.len() == n + 1 && ad_offsets.len() == n + 1);
+            let mut bad = 0u64;
+            let okp = match ok { Some(v) => { assert!(v.len() >= n); v.as_mut_ptr() } None => core::ptr::null_mut() };
+            let rc = unsafe {
+                avrf_pedersen_batch_push_compressed(
+                    self.h, n as u64, ios32.as_ptr() as *const u8, io_offsets.as_ptr(), ad_blob.as_ptr(),
+                    ad_offsets.as_ptr(), proofs.as_ptr() as *const u8, okp, &mut bad,
+                )
+            };
+            assert!(rc == 0, "libavrf_gpu system error {rc}");
+            bad
         }
 
         /// Same contract as `pedersen::BatchVerifier::verify` (src/pedersen.rs:341-426).

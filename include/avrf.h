@@ -250,6 +250,19 @@ int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios,
                                   const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);
 int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status);
 
+/* The same push for proofs in WIRE format: `proofs` is n records of 160 bytes, each exactly
+ * pedersen::Proof::serialize_compressed (pk_com 32 | r 32 | ok 32 | s 32 | sb 32, src/pedersen.rs:43-50: compressed
+ * points, canonical little-endian scalars), and ios32 is 64 bytes per pair (input, output) as in
+ * avrf_thin_batch_push_compressed.  Decoded and validated on the device: pk_com, R and Ok are bare points (on the curve,
+ * prime-order subgroup, identity allowed: an identity pk_com decodes and verify then reports InvalidData); I and O are
+ * Input / Output (identity refused); s >= r or sb >= r fails the proof's deserialisation.  224 instead of 384 bytes per
+ * proof cross PCIe at M = 1.  All or nothing: when any proof does not decode, *n_bad is their number, ok[j] (optional,
+ * n bytes) is 0 for them, and NOTHING is pushed - a handle that held proofs keeps exactly those, and their seed.
+ * A Thin handle is an argument error.  Works with handles of either format. */
+int avrf_pedersen_batch_push_compressed(avrf_batch* b, uint64_t n, const uint8_t* ios32, const uint32_t* io_offsets,
+                                        const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* proofs,
+                                        uint8_t* ok, uint64_t* n_bad);
+
 /* pedersen::Verifier::verify (src/pedersen.rs:188-253) for every proof pushed to a Pedersen handle: statuses[j] in
  * {AVRF_OK, AVRF_VERIFICATION_FAILURE, AVRF_INVALID_DATA}, each proof judged on its own as avrf_pedersen_verify_one
  * would.  Use after a failed batch to name the offenders.  Runs on the handle's stream; a Thin handle is an argument

@@ -9,7 +9,7 @@
 //   thin::ShardedBatchVerifier<S>                 (new: one batch over several GPUs of this process, avrf_thin_sharded_*)
 //   pedersen::Proof{pk_com, r, ok, s, sb}         src/pedersen.rs:43-50
 //   pedersen::verify (pedersen::Verifier)         src/pedersen.rs:188-253
-//   pedersen::BatchVerifier<S>::{push, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
+//   pedersen::BatchVerifier<S>::{push, push_compressed, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
 //   pedersen::prove_many (Prover::prove, n proofs) src/pedersen.rs:136-186
 //   Error::{VerificationFailure, InvalidData}     src/lib.rs:136-147
 //
@@ -216,6 +216,17 @@ class BatchVerifier {
     check(avrf_pedersen_batch_push_many(h_, 1, ios.empty() ? nullptr : ios[0].input.data(), io_off,
                                         ad.empty() ? nullptr : ad.data(), ad_off, proof.pk_com.data(), proof.r.data(),
                                         proof.ok.data(), proof.s.data(), proof.sb.data()));
+  }
+  // Proofs in wire format: n records of Proof::serialize_compressed (pk_com | r | ok | s | sb, 160 bytes) and 64 bytes
+  // of compressed (input, output) per pair, decoded and validated on the device.  Returns the number of proofs that
+  // do not decode; when it is not zero nothing was pushed and ok[j] == 0 names them.
+  uint64_t push_compressed(uint64_t n, const uint8_t* ios32, const uint32_t* io_offsets, const uint8_t* ad_blob,
+                           const uint32_t* ad_offsets, const uint8_t* proofs, std::vector<uint8_t>* ok = nullptr) {
+    uint64_t bad = 0;
+    if (ok) ok->assign(n, 0);
+    check(avrf_pedersen_batch_push_compressed(h_, n, ios32, io_offsets, ad_blob, ad_offsets, proofs,
+                                              ok && n ? ok->data() : nullptr, &bad));
+    return bad;
   }
   Result verify() const {
     int32_t st = -1;

@@ -3,6 +3,9 @@ each, 4096 signers; every proof distinct).  Prints one JSON line with the device
 run.  Legs (best of --reps after a warm-up, except the latency leg):
   prove_many        avrf_pedersen_prove_many, proofs/s
   batch             push of the 2^20 proofs from pinned memory + verify, wall time, with avrf_thin_batch_timings
+  wire              the same batch serialised once (pedersen.serialize_proofs: 160-byte records, compressed I/O pairs),
+                    pushed from pinned memory through push_compressed (decoded and validated on the GPU) + verify, wall
+                    time; then one more push + verify under torch.profiler for the device time of the decode kernels
   verify_each       avrf_pedersen_batch_verify_each over the batch, proofs/s
   verify_one        median latency of 200 avrf_pedersen_verify_one calls
   thin_prove_many / thin_verify_each   the same two legs of the Thin VRF on its batch of the same size
@@ -36,6 +39,28 @@ def best(fn, reps):
         fn()
         ts.append(time.perf_counter() - t0)
     return min(ts)
+
+
+DECODE_KERNELS = ("k_ped_wire_unpack", "k_dec_prep", "k_batch_inv", "k_dec_finish", "k_ped_proof_ok", "k_scalars_to_mont")
+
+
+def decode_kernel_ms(fn):
+    """Device time (ms) of the wire decode kernels during one call of fn, from torch.profiler's CUDA activity records,
+    per kernel and in total."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    per = {}
+    for ev in prof.events():
+        if ev.device_type == torch.autograd.DeviceType.CUDA:
+            k = next((k for k in DECODE_KERNELS if k in ev.name), None)
+            if k:
+                per[k] = per.get(k, 0.0) + ev.device_time_total / 1e3
+    out = {k: round(v, 3) for k, v in per.items()}
+    out["total"] = round(sum(per.values()), 3)
+    return out
 
 
 def main():
@@ -79,6 +104,26 @@ def main():
     res["batch_push_verify_ms"] = round(1e3 * t, 2)
     res["batch_proofs_per_s"] = round(n / t)
     res["batch_timings"] = {k: (round(v, 3) if isinstance(v, float) else v) for k, v in tm.as_dict().items()}
+
+    # wire format: what callers hold before Proof::deserialize_compressed
+    nio = int(b.io_offsets[n])
+    ios32 = np.concatenate([ops.point_compress(sid, b.ios[:nio].reshape(-1, 64), F).reshape(-1), np.zeros(64, np.uint8)])
+    recs = ped.serialize_proofs(sid, b.pk_com, b.r, b.ok, b.s, b.sb, F)
+    warrs = [pin(x) for x in (ios32, b.io_offsets, b.ad_blob, b.ad_offsets, recs)]
+    wv = ped.BatchVerifier(sid, F)
+    wstatus = []
+
+    def wire():
+        wv.clear()
+        assert wv.push_compressed(*warrs).all()
+        wstatus.append(wv.verify_status())
+    t = best(wire, a.reps)
+    assert set(wstatus) == {0}, wstatus
+    res["wire_push_verify_ms"] = round(1e3 * t, 2)
+    res["wire_proofs_per_s"] = round(n / t)
+    res["wire_bytes_per_proof"] = int((recs.nbytes + 64 * nio) // n)
+    res["wire_decode_kernels_ms"] = decode_kernel_ms(wire)
+
     each = []
     t = best(lambda: each.append(bv.verify_each()), a.reps)
     assert all((e == 0).all() for e in each)
