@@ -14,7 +14,9 @@
 //   pedersen::Verifier::verify   src/pedersen.rs:188-253 -> k_verify_one_ped, k_verify_each_ped (per-proof verdicts)
 //   pedersen Proof::deserialize_compressed (wire push) -> k_ped_wire_unpack, k_dec_prep/k_dec_finish, k_ped_proof_ok
 // There is no CPU fallback: without a CUDA device every compute entry point fails.
+#include <array>
 #include <cstdlib>
+#include <functional>
 #include <map>
 #include <memory>
 #include <new>
@@ -109,8 +111,32 @@ static cudaError_t hsync(avrf_batch* b, cudaStream_t st) {
   return cudaEventSynchronize(b->sync_ev);
 }
 
-static size_t npoints_of(const avrf_batch* b) { return b->scheme ? 5 * b->n + 2 : 2 * b->n + 2 * b->n_ios + 1; }
-static size_t cs_stride(const avrf_batch* b) { return b->scheme ? 96 : 64; }
+// What a proof scheme stores in a batch handle, indexed by avrf_batch::scheme.
+struct Column {
+  DevBuf avrf_batch::*buf;
+  size_t bytes;                         // per proof
+};
+struct Scheme {
+  uint32_t ncol;
+  Column col[5];                        // the per-proof device inputs, in the order push_many_impl takes them
+  size_t cs_stride;                     // bytes per proof of the (c,s) stream that the batch seed hashes
+  size_t w_tap;                         // bytes per proof of AVRF_TAP_W
+  size_t pts_proof, pts_pair, pts_fixed;  // MSM terms: per proof, per I/O pair, and the fixed bases added at MSM time
+  uint32_t scal_per_thread;             // proofs per k_scalars / k_scalars_ped thread
+  const char* prepare;                  // k_prepare<S> / k_prepare_ped<S>
+  size_t proof_points(uint64_t n, uint64_t n_ios) const { return pts_proof * n + pts_pair * n_ios; }
+  size_t points(uint64_t n, uint64_t n_ios) const { return proof_points(n, n_ios) + pts_fixed; }
+};
+static constexpr Scheme SCHEMES[2] = {
+    // Thin VRF (src/thin.rs): pk | r | s; bases R, pk, (O_i, I_i) per proof and the generator
+    {3, {{&avrf_batch::pk, 64}, {&avrf_batch::r, 64}, {&avrf_batch::s, 32}}, 64, 16, 2, 2, 1, SCAL_PER_THREAD, "k_prepare"},
+    // Pedersen VRF (src/pedersen.rs): pk holds the key commitments; five bases per proof, then G and B
+    {5, {{&avrf_batch::pk, 64}, {&avrf_batch::r, 64}, {&avrf_batch::s, 32}, {&avrf_batch::ok, 64}, {&avrf_batch::sb, 32}},
+     96, 32, 5, 0, 2, 1, "k_prepare_ped"},
+};
+static const Scheme& scheme_of(const avrf_batch* b) { return SCHEMES[b->scheme]; }
+using Columns = std::array<const uint8_t*, 5>;     // one array per input column of a push, in table order
+
 static uint64_t pending_of(const avrf_batch* b) { return b->stage[0].n + b->stage[1].n + (b->h_io_off.size() - 1); }
 
 #define DISPATCH(suite, STMT)                      \
@@ -128,9 +154,22 @@ static int launch_check(const char* name) {
 }
 #define LAUNCHED(name) do { int rc__ = launch_check(name); if (rc__) return rc__; } while (0)
 
-static const unsigned char* suite_id_of(uint32_t suite, size_t* len) {
-  *len = CC_HOST[suite].sid_len;
-  return CC_HOST[suite].suite_id;
+// SUITE_ID || 0x50: the start of every batch-seed hash (src/thin.rs:273-279).  Returns its length.
+static size_t batch_prefix(uint32_t suite, unsigned char buf[40]) {
+  size_t sl = CC_HOST[suite].sid_len;
+  memcpy(buf, CC_HOST[suite].suite_id, sl);
+  buf[sl] = DOM_BATCH;
+  return sl + 1;
+}
+
+// Orders `waiter` after the work enqueued so far on `st`.
+static int stream_after(cudaStream_t waiter, cudaStream_t st) {
+  cudaEvent_t e;
+  CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  cudaEventRecord(e, st);
+  cudaStreamWaitEvent(waiter, e, 0);
+  cudaEventDestroy(e);
+  return 0;
 }
 
 static int finish_inflight(avrf_batch* b);
@@ -154,6 +193,30 @@ static int grow(avrf_batch* b, DevBuf& buf, size_t bytes, size_t keep) {
   if (bytes <= buf.cap) return 0;
   int rc = quiesce(b);
   return rc ? rc : buf.reserve(bytes, keep, b->st);
+}
+// Room for n proofs with n_ios pairs and ad_bytes of additional data in the input buffers, keeping the handle's proofs.
+static int grow_inputs(avrf_batch* b, uint64_t n, uint64_t n_ios, uint64_t ad_bytes) {
+  const Scheme& sc = scheme_of(b);
+  int rc;
+  for (uint32_t k = 0; k < sc.ncol; k++)
+    if ((rc = grow(b, b->*sc.col[k].buf, sc.col[k].bytes * n, sc.col[k].bytes * b->n))) return rc;
+  if ((rc = grow(b, b->ios, 128 * n_ios + 128, 128 * b->n_ios)) || (rc = grow(b, b->ad, ad_bytes + 16, b->ad_bytes)) ||
+      (rc = grow(b, b->io_off, 4 * (n + 1), 4 * (b->n + 1))) || (rc = grow(b, b->ad_off, 4 * (n + 1), 4 * (b->n + 1))))
+    return rc;
+  return 0;
+}
+// ... and in the buffers k_prepare fills, keeping what it derived for the handle's proofs when they are prepared
+static int grow_derived(avrf_batch* b, uint64_t n, uint64_t n_ios) {
+  const Scheme& sc = scheme_of(b);
+  const bool keep = b->prepared;
+  size_t np = sc.points(n, n_ios), np_old = b->n ? sc.proof_points(b->n, b->n_ios) : 0;
+  int rc;
+  if ((rc = grow(b, b->pts, sizeof(BaseRec) * np, keep ? sizeof(BaseRec) * np_old : 0)) ||
+      (rc = grow(b, b->cs, sc.cs_stride * n + 64, keep ? sc.cs_stride * b->n : 0)) ||
+      (rc = grow(b, b->z, 16 * n_ios + 16, keep ? 16 * b->n_ios : 0)) ||
+      (rc = grow(b, b->renc, 32 * n + 32, keep ? 32 * b->n : 0)))
+    return rc;
+  return 0;
 }
 
 static Hasher* hasher_of(avrf_batch* b) {
@@ -333,7 +396,9 @@ void avrf_thin_batch_free(avrf_batch* b) {
     cudaEventDestroy(b->h2d_gate_ev);
   }
   for (cudaStream_t q : {b->st, b->st_copy, b->st_h2d, b->st_prep}) if (q) cudaStreamSynchronize(q);
-  DevBuf* bufs[] = {&b->ok, &b->sb, &b->pk, &b->r, &b->s, &b->ios, &b->io_off, &b->ad_off, &b->ad, &b->pts, &b->cs, &b->z, &b->renc,
+  const Scheme& sc = scheme_of(b);
+  for (uint32_t k = 0; k < sc.ncol; k++) (b->*sc.col[k].buf).release();
+  DevBuf* bufs[] = {&b->ios, &b->io_off, &b->ad_off, &b->ad, &b->pts, &b->cs, &b->z, &b->renc,
                     &b->dig_w, &b->rank_w, &b->digits, &b->hist, &b->cursor, &b->offs, &b->toff, &b->btot, &b->totals, &b->entries, &b->tasks,
                     &b->task_out, &b->chunk_out, &b->wsum, &b->partial, &b->gpart, &b->flags, &b->w_tap, &b->scalars_tap,
                     &b->segs_dev};
@@ -447,21 +512,8 @@ int avrf_thin_batch_set_weights_mode(avrf_batch* b, uint32_t mode) {
 int avrf_thin_batch_reserve(avrf_batch* b, uint64_t n, uint64_t n_ios, uint64_t ad_bytes) {
   ENTER(b);
   if (n >= (1ull << 30) || n_ios >= (1ull << 30) || ad_bytes >= (1ull << 32)) return fail(AVRF_ERR_ARG, "batch too large");
-  const bool ped = b->scheme == 1;
-  int rc;
-  if ((rc = grow(b, b->pk, 64 * n, 64 * b->n)) || (rc = grow(b, b->r, 64 * n, 64 * b->n)) ||
-      (rc = grow(b, b->s, 32 * n, 32 * b->n)) || (rc = grow(b, b->ios, 128 * n_ios + 128, 128 * b->n_ios)) ||
-      (rc = grow(b, b->ad, ad_bytes + 16, b->ad_bytes)) || (rc = grow(b, b->io_off, 4 * (n + 1), 4 * (b->n + 1))) ||
-      (rc = grow(b, b->ad_off, 4 * (n + 1), 4 * (b->n + 1))))
-    return rc;
-  if (ped && ((rc = grow(b, b->ok, 64 * n, 64 * b->n)) || (rc = grow(b, b->sb, 32 * n, 32 * b->n)))) return rc;
-  size_t np = ped ? 5 * n + 2 : 2 * n + 2 * n_ios + 1, np_old = b->n ? (ped ? 5 * b->n : 2 * b->n + 2 * b->n_ios) : 0;
-  if ((rc = grow(b, b->pts, sizeof(BaseRec) * np, b->prepared ? sizeof(BaseRec) * np_old : 0)) ||
-      (rc = grow(b, b->cs, cs_stride(b) * n + 64, b->prepared ? cs_stride(b) * b->n : 0)) ||
-      (rc = grow(b, b->z, 16 * n_ios + 16, b->prepared ? 16 * b->n_ios : 0)) ||
-      (rc = grow(b, b->renc, 32 * n + 32, b->prepared ? 32 * b->n : 0)))
-    return rc;
-  return 0;
+  int rc = grow_inputs(b, n, n_ios, ad_bytes);
+  return rc ? rc : grow_derived(b, n, n_ios);
 }
 
 // Leaf digests (64 B each) of this handle's (c,s) stream; first_index = global index of its first proof
@@ -486,36 +538,56 @@ int avrf_thin_batch_tree_leaves(avrf_batch* b, uint64_t first_index, uint8_t* ou
 // seed = SHA512(SUITE_ID || 0x50 || 0x01 || LE64(n_total) || leaf_0 || leaf_1 || ...)
 int avrf_thin_seed_tree(uint32_t suite, uint64_t n_total, const uint8_t* leaves, uint64_t n_leaves, uint8_t seed[64]) {
   if (suite > 2 || !seed || (n_leaves && !leaves)) return fail(AVRF_ERR_ARG, "bad argument");
-  size_t sl;
-  const unsigned char* sid = suite_id_of(suite, &sl);
-  EVP_MD_CTX* ctx = EVP_MD_CTX_new();
-  if (!ctx) return fail(AVRF_ERR_NOMEM, "EVP_MD_CTX_new");
-  unsigned char tag[2] = {DOM_BATCH, 0x01}, le[8];
-  for (int i = 0; i < 8; i++) le[i] = (unsigned char)(n_total >> (8 * i));
-  unsigned int outl = 64;
-  EVP_DigestInit_ex(ctx, EVP_sha512(), nullptr);
-  EVP_DigestUpdate(ctx, sid, sl);
-  EVP_DigestUpdate(ctx, tag, 2);
-  EVP_DigestUpdate(ctx, le, 8);
-  if (n_leaves) EVP_DigestUpdate(ctx, leaves, 64 * n_leaves);
-  EVP_DigestFinal_ex(ctx, seed, &outl);
-  EVP_MD_CTX_free(ctx);
-  return 0;
+  unsigned char head[49];
+  size_t hl = batch_prefix(suite, head);
+  head[hl++] = 0x01;
+  for (int i = 0; i < 8; i++) head[hl++] = (unsigned char)(n_total >> (8 * i));
+  return sha512({{head, hl}, {leaves, 64 * n_leaves}}, seed);
 }
 
 // =========================================================================================
 // Push
 // =========================================================================================
-// n proofs from host arrays into the handle.  With the eager pipeline the (c,s) chunks are handed to the
-// hasher thread and the call returns without waiting for the hash; `consumed` (optional) is recorded once the
-// device no longer reads the host arrays.
-static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const uint8_t* ios, const uint32_t* io_offsets,
-                          const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* r, const uint8_t* s,
-                          const uint8_t* ok = nullptr, const uint8_t* sb = nullptr, cudaEvent_t consumed = nullptr,
+// The offsets of a push of n proofs start at 0, and a blob that the offsets say is not empty is present.
+static int check_offsets(uint64_t n, const uint32_t* io_offsets, const uint32_t* ad_offsets, const uint8_t* ios,
+                         const uint8_t* ad_blob) {
+  if (io_offsets[0] != 0 || ad_offsets[0] != 0) return fail(AVRF_ERR_ARG, "offsets must start at 0");
+  if ((io_offsets[n] && !ios) || (ad_offsets[n] && !ad_blob)) return fail(AVRF_ERR_ARG, "null argument");
+  return 0;
+}
+
+// k_prepare<S> (Thin) / k_prepare_ped<S> (Pedersen) over the resident proofs [first, last) of the handle, on `st`.
+static int launch_prepare(avrf_batch* b, size_t first, size_t last, cudaStream_t st) {
+  const uint32_t grid = cdiv(last - first, 128);
+  if (b->scheme == 1) {
+    PedPrepArgs a;
+    a.pkcom = b->pk.as<Affine>(); a.r = b->r.as<Affine>(); a.ok = b->ok.as<Affine>(); a.s = b->s.as<Fe>();
+    a.sb = b->sb.as<Fe>(); a.ios = b->ios.as<Affine>(); a.io_off = b->io_off.as<uint32_t>();
+    a.ad_off = b->ad_off.as<uint32_t>(); a.ad = b->ad.as<uint8_t>(); a.pts = b->pts.as<BaseRec>();
+    a.cs = b->cs.as<uint32_t>(); a.flags = b->flags.as<int>();
+    a.first = (uint32_t)first; a.n = (uint32_t)last; a.canonical = b->fmt == AVRF_FMT_CANONICAL;
+    DISPATCH(b->suite, (k_prepare_ped<S><<<grid, 128, 0, st>>>(a)));
+  } else {
+    PrepArgs a;
+    a.pk = b->pk.as<Affine>(); a.r = b->r.as<Affine>(); a.s = b->s.as<Fe>(); a.ios = b->ios.as<Affine>();
+    a.io_off = b->io_off.as<uint32_t>(); a.ad_off = b->ad_off.as<uint32_t>(); a.ad = b->ad.as<uint8_t>();
+    a.pts = b->pts.as<BaseRec>(); a.cs = b->cs.as<uint32_t>(); a.z = b->z.as<uint32_t>();
+    a.renc = b->renc.as<uint32_t>(); a.flags = b->flags.as<int>();
+    a.first = (uint32_t)first; a.n = (uint32_t)last; a.canonical = b->fmt == AVRF_FMT_CANONICAL;
+    DISPATCH(b->suite, (k_prepare<S><<<grid, 128, 0, st>>>(a)));
+  }
+  LAUNCHED(scheme_of(b).prepare);
+  return 0;
+}
+
+// n proofs from host arrays into the handle: `cols` holds one array per input column of the handle's scheme, in table
+// order.  With the eager pipeline the (c,s) chunks are handed to the hasher thread and the call returns without waiting
+// for the hash; `consumed` (optional) is recorded once the device no longer reads the host arrays.
+static int push_many_impl(avrf_batch* b, uint64_t n, const Columns& cols, const uint8_t* ios, const uint32_t* io_offsets,
+                          const uint8_t* ad_blob, const uint32_t* ad_offsets, cudaEvent_t consumed = nullptr,
                           size_t stage_chunks = 0) {
-  // thin: pk = public keys.  Pedersen (b->scheme == 1): pk = key commitments, plus ok (64 B) and sb (32 B) per proof.
-  const bool ped = b->scheme == 1;
-  const size_t stride = cs_stride(b);
+  const Scheme& sc = scheme_of(b);
+  const size_t stride = sc.cs_stride;
   if (n == 0) return 0;
   // offsets may start anywhere (a slice of a larger push): `ios` / `ad_blob` point at the slice's first pair / byte
   const uint32_t iob = io_offsets[0], adb = ad_offsets[0];
@@ -525,14 +597,7 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
     return fail(AVRF_ERR_ARG, "batch too large");
   int rc;
   bool pipeline = b->eager && (b->prepared || n0 == 0) && b->hashed == n0;
-  if ((rc = grow(b, b->pk, 64 * (n0 + n), 64 * n0))) return rc;
-  if ((rc = grow(b, b->r, 64 * (n0 + n), 64 * n0))) return rc;
-  if ((rc = grow(b, b->s, 32 * (n0 + n), 32 * n0))) return rc;
-  if (ped && ((rc = grow(b, b->ok, 64 * (n0 + n), 64 * n0)) || (rc = grow(b, b->sb, 32 * (n0 + n), 32 * n0)))) return rc;
-  if ((rc = grow(b, b->ios, 128 * (i0 + add_ios) + 128, 128 * i0))) return rc;
-  if ((rc = grow(b, b->ad, a0 + add_ad + 16, a0))) return rc;
-  if ((rc = grow(b, b->io_off, 4 * (n0 + n + 1), 4 * (n0 + 1)))) return rc;
-  if ((rc = grow(b, b->ad_off, 4 * (n0 + n + 1), 4 * (n0 + 1)))) return rc;
+  if ((rc = grow_inputs(b, n0 + n, i0 + add_ios, a0 + add_ad))) return rc;
   // offsets first (small), rebased on the device
   cudaStream_t ost = pipeline ? b->st_prep : b->st;
   CK(cudaMemcpyAsync(b->io_off.as<uint32_t>() + n0, io_offsets, 4 * (n + 1), cudaMemcpyHostToDevice, ost));
@@ -540,12 +605,9 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
   if (i0 != iob) { k_rebase<<<cdiv(n + 1, 256), 256, 0, ost>>>(b->io_off.as<uint32_t>() + n0, n + 1, (uint32_t)i0 - iob); LAUNCHED("k_rebase"); }
   if (a0 != adb) { k_rebase<<<cdiv(n + 1, 256), 256, 0, ost>>>(b->ad_off.as<uint32_t>() + n0, n + 1, (uint32_t)a0 - adb); LAUNCHED("k_rebase"); }
   if (!pipeline) {
-    CK(cudaMemcpyAsync(b->pk.as<uint8_t>() + 64 * n0, pk, 64 * n, cudaMemcpyDefault, b->st));
-    CK(cudaMemcpyAsync(b->r.as<uint8_t>() + 64 * n0, r, 64 * n, cudaMemcpyDefault, b->st));
-    CK(cudaMemcpyAsync(b->s.as<uint8_t>() + 32 * n0, s, 32 * n, cudaMemcpyDefault, b->st));
-    if (ped) {
-      CK(cudaMemcpyAsync(b->ok.as<uint8_t>() + 64 * n0, ok, 64 * n, cudaMemcpyDefault, b->st));
-      CK(cudaMemcpyAsync(b->sb.as<uint8_t>() + 32 * n0, sb, 32 * n, cudaMemcpyDefault, b->st));
+    for (uint32_t k = 0; k < sc.ncol; k++) {
+      const Column& c = sc.col[k];
+      CK(cudaMemcpyAsync((b->*c.buf).as<uint8_t>() + c.bytes * n0, cols[k], c.bytes * n, cudaMemcpyDefault, b->st));
     }
     if (add_ios) CK(cudaMemcpyAsync(b->ios.as<uint8_t>() + 128 * i0, ios, 128 * add_ios, cudaMemcpyDefault, b->st));
     if (add_ad) CK(cudaMemcpyAsync(b->ad.as<uint8_t>() + a0, ad_blob, add_ad, cudaMemcpyDefault, b->st));
@@ -561,22 +623,13 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
   // ---- eager pipeline: per chunk  H2D (st_h2d) -> k_prepare (st_prep) -> D2H of (c,s) (st_copy) -> hasher thread ----
   Hasher* hs = hasher_of(b);
   if (!hs) return fail(AVRF_ERR_NOMEM, "hasher");
-  size_t np_new = ped ? 5 * (n0 + n) + 2 : 2 * (n0 + n) + 2 * (i0 + add_ios) + 1;
-  size_t np_old = n0 ? (ped ? 5 * n0 : 2 * n0 + 2 * i0) : 0;
   if ((rc = b->flags.reserve(64))) return rc;
   if ((rc = b->h_small.reserve(4096))) return rc;
-  if ((rc = grow(b, b->pts, sizeof(BaseRec) * np_new, sizeof(BaseRec) * np_old))) return rc;
-  if ((rc = grow(b, b->cs, stride * (n0 + n) + 64, stride * n0))) return rc;
-  if ((rc = grow(b, b->z, 16 * (i0 + add_ios) + 16, 16 * i0))) return rc;
-  if ((rc = grow(b, b->renc, 32 * (n0 + n) + 32, 32 * n0))) return rc;
+  if ((rc = grow_derived(b, n0 + n, i0 + add_ios))) return rc;       // (the pipeline runs on prepared or empty handles)
   if (n0 == 0) {
     if (!b->ext_hasher) {                 // a shard's parent starts the stream of the whole batch itself
-      size_t sl;
-      const unsigned char* sid = suite_id_of(b->suite, &sl);
       unsigned char prefix[40];
-      memcpy(prefix, sid, sl);
-      prefix[sl] = DOM_BATCH;
-      if ((rc = hs->begin(prefix, sl + 1))) return rc;
+      if ((rc = hs->begin(prefix, batch_prefix(b->suite, prefix)))) return rc;
     }
     CK(cudaMemsetAsync(b->flags.p, 0, 64, b->st_prep));
   }
@@ -589,21 +642,6 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
   if (!off_ev) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
   CK(cudaEventRecord(off_ev, b->st_prep));
   CK(cudaStreamWaitEvent(b->st_h2d, off_ev, 0));         // also orders after any device-side realloc copies
-  PrepArgs a;
-  PedPrepArgs pa;
-  if (ped) {
-    pa.pkcom = b->pk.as<Affine>(); pa.r = b->r.as<Affine>(); pa.ok = b->ok.as<Affine>(); pa.s = b->s.as<Fe>();
-    pa.sb = b->sb.as<Fe>(); pa.ios = b->ios.as<Affine>(); pa.io_off = b->io_off.as<uint32_t>();
-    pa.ad_off = b->ad_off.as<uint32_t>(); pa.ad = b->ad.as<uint8_t>(); pa.pts = b->pts.as<BaseRec>();
-    pa.cs = b->cs.as<uint32_t>(); pa.flags = b->flags.as<int>();
-    pa.canonical = b->fmt == AVRF_FMT_CANONICAL;
-  } else {
-    a.pk = b->pk.as<Affine>(); a.r = b->r.as<Affine>(); a.s = b->s.as<Fe>(); a.ios = b->ios.as<Affine>();
-    a.io_off = b->io_off.as<uint32_t>(); a.ad_off = b->ad_off.as<uint32_t>(); a.ad = b->ad.as<uint8_t>();
-    a.pts = b->pts.as<BaseRec>(); a.cs = b->cs.as<uint32_t>(); a.z = b->z.as<uint32_t>();
-    a.renc = b->renc.as<uint32_t>(); a.flags = b->flags.as<int>();
-    a.canonical = b->fmt == AVRF_FMT_CANONICAL;
-  }
   if (!b->h2d_gate_ev) CK(cudaEventCreateWithFlags(&b->h2d_gate_ev, cudaEventDisableTiming));
   MsmGate& hgate = g_h2d_gate[b->device];
   std::unique_lock<std::mutex> hgate_lock(hgate.mu);
@@ -614,27 +652,16 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const uint8_t* pk, const ui
     cudaEvent_t h2d_ev = evs.make(), prep_ev = evs.make();
     cudaEvent_t d2h_ev = nullptr;                          // owned by the hasher once queued
     if (!h2d_ev || !prep_ev) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
-    CK(cudaMemcpyAsync(b->pk.as<uint8_t>() + 64 * (n0 + c0), pk + 64 * c0, 64 * cnt, cudaMemcpyDefault, b->st_h2d));
-    CK(cudaMemcpyAsync(b->r.as<uint8_t>() + 64 * (n0 + c0), r + 64 * c0, 64 * cnt, cudaMemcpyDefault, b->st_h2d));
-    CK(cudaMemcpyAsync(b->s.as<uint8_t>() + 32 * (n0 + c0), s + 32 * c0, 32 * cnt, cudaMemcpyDefault, b->st_h2d));
-    if (ped) {
-      CK(cudaMemcpyAsync(b->ok.as<uint8_t>() + 64 * (n0 + c0), ok + 64 * c0, 64 * cnt, cudaMemcpyDefault, b->st_h2d));
-      CK(cudaMemcpyAsync(b->sb.as<uint8_t>() + 32 * (n0 + c0), sb + 32 * c0, 32 * cnt, cudaMemcpyDefault, b->st_h2d));
+    for (uint32_t k = 0; k < sc.ncol; k++) {
+      const Column& col = sc.col[k];
+      CK(cudaMemcpyAsync((b->*col.buf).as<uint8_t>() + col.bytes * (n0 + c0), cols[k] + col.bytes * c0, col.bytes * cnt,
+                         cudaMemcpyDefault, b->st_h2d));
     }
     if (q1 > q0) CK(cudaMemcpyAsync(b->ios.as<uint8_t>() + 128 * (i0 + q0), ios + 128 * q0, 128 * (q1 - q0), cudaMemcpyDefault, b->st_h2d));
     if (d1 > d0) CK(cudaMemcpyAsync(b->ad.as<uint8_t>() + a0 + d0, ad_blob + d0, d1 - d0, cudaMemcpyDefault, b->st_h2d));
     CK(cudaEventRecord(h2d_ev, b->st_h2d));
     CK(cudaStreamWaitEvent(b->st_prep, h2d_ev, 0));
-    if (ped) {
-      pa.first = (uint32_t)(n0 + c0);
-      pa.n = (uint32_t)(n0 + c1);
-      DISPATCH(b->suite, (k_prepare_ped<S><<<cdiv(cnt, 128), 128, 0, b->st_prep>>>(pa)));
-    } else {
-      a.first = (uint32_t)(n0 + c0);
-      a.n = (uint32_t)(n0 + c1);
-      DISPATCH(b->suite, (k_prepare<S><<<cdiv(cnt, 128), 128, 0, b->st_prep>>>(a)));
-    }
-    LAUNCHED("k_prepare");
+    if ((rc = launch_prepare(b, n0 + c0, n0 + c1, b->st_prep))) return rc;
     CK(cudaEventRecord(prep_ev, b->st_prep));
     CK(cudaStreamWaitEvent(b->st_copy, prep_ev, 0));
     uint8_t* dst = hs->stage(stride * cnt);
@@ -677,9 +704,8 @@ static int flush_stage(avrf_batch* b) {
   if (sg.n == 0) return 0;
   { int rc0 = bind_device(b->device); if (rc0) return rc0; }
   stage_fence();
-  int rc = push_many_impl(b, sg.n, sg.pk.as<uint8_t>(), sg.ios.as<uint8_t>(), sg.io_off.as<uint32_t>(), sg.ad.as<uint8_t>(),
-                          sg.ad_off.as<uint32_t>(), sg.r.as<uint8_t>(), sg.s.as<uint8_t>(), nullptr, nullptr, sg.free_ev,
-                          sg.n == STAGE_CHUNK ? 4 : 0);
+  int rc = push_many_impl(b, sg.n, {sg.pk.as<uint8_t>(), sg.r.as<uint8_t>(), sg.s.as<uint8_t>()}, sg.ios.as<uint8_t>(), sg.io_off.as<uint32_t>(), sg.ad.as<uint8_t>(),
+                          sg.ad_off.as<uint32_t>(), sg.free_ev, sg.n == STAGE_CHUNK ? 4 : 0);
   if (rc) return rc;
   sg.n = sg.nio = sg.nad = 0;
   sg.inflight = true;
@@ -694,8 +720,7 @@ static int flush_pending(avrf_batch* b) {
   if (rc) return rc;
   uint64_t pend = b->h_io_off.size() - 1;
   if (!pend) return 0;
-  rc = push_many_impl(b, pend, b->h_pk.data(), b->h_ios.data(), b->h_io_off.data(), b->h_ad.data(),
-                      b->h_ad_off.data(), b->h_r.data(), b->h_s.data());
+  rc = push_many_impl(b, pend, {b->h_pk.data(), b->h_r.data(), b->h_s.data()}, b->h_ios.data(), b->h_io_off.data(), b->h_ad.data(), b->h_ad_off.data());
   if (rc) return rc;
   if ((rc = quiesce(b))) return rc;        // host vectors are about to be cleared
   b->h_pk.clear(); b->h_r.clear(); b->h_s.clear(); b->h_ios.clear(); b->h_ad.clear();
@@ -746,6 +771,20 @@ int avrf_thin_batch_push(avrf_batch* b, const uint8_t pk[64], const uint8_t* ios
   return 0;
 }
 
+// push_many of arrays that the caller only lends for the duration of the call (thin.rs:218-225): returns once the
+// device has consumed them - not the hash, which proceeds on the hasher thread.
+static int push_borrowed(avrf_batch* b, uint64_t n, const Columns& cols, const uint8_t* ios, const uint32_t* io_offsets,
+                         const uint8_t* ad_blob, const uint32_t* ad_offsets) {
+  int rc = check_offsets(n, io_offsets, ad_offsets, ios, ad_blob);
+  if (rc) return rc;
+  ENTER(b);
+  if ((rc = flush_pending(b))) return rc;          // (single pushes are Thin only: a no-op on a Pedersen handle)
+  if ((rc = push_many_impl(b, n, cols, ios, io_offsets, ad_blob, ad_offsets))) return rc;
+  CK(hsync(b, b->st_h2d));
+  CK(hsync(b, b->prepared ? b->st_prep : b->st));
+  return 0;
+}
+
 int avrf_thin_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* pk, const uint8_t* ios,
                               const uint32_t* io_offsets, const uint8_t* ad_blob, const uint32_t* ad_offsets,
                               const uint8_t* r, const uint8_t* s) {
@@ -753,18 +792,7 @@ int avrf_thin_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* pk, cons
   if (b->scheme != 0) return fail(AVRF_ERR_ARG, "not a Thin-VRF batch");
   if (n == 0) return 0;
   if (!pk || !io_offsets || !ad_offsets || !r || !s) return fail(AVRF_ERR_ARG, "null argument");
-  if (io_offsets[0] != 0 || ad_offsets[0] != 0) return fail(AVRF_ERR_ARG, "offsets must start at 0");
-  if ((io_offsets[n] && !ios) || (ad_offsets[n] && !ad_blob)) return fail(AVRF_ERR_ARG, "null argument");
-  ENTER(b);
-  int rc = flush_pending(b);
-  if (rc) return rc;
-  rc = push_many_impl(b, n, pk, ios, io_offsets, ad_blob, ad_offsets, r, s);
-  if (rc) return rc;
-  // the caller's buffers are only borrowed for the duration of the call (thin.rs:218-225): wait until the device
-  // has consumed them - not for the hash, which proceeds on the hasher thread
-  CK(hsync(b, b->st_h2d));
-  CK(hsync(b, b->prepared ? b->st_prep : b->st));
-  return 0;
+  return push_borrowed(b, n, {pk, r, s}, ios, io_offsets, ad_blob, ad_offsets);
 }
 
 // =========================================================================================
@@ -777,11 +805,7 @@ int avrf_thin_batch_prepare(avrf_batch* b, int32_t* invalid) {
   if ((rc = b->flags.reserve(64))) return rc;
   if ((rc = b->h_small.reserve(4096))) return rc;
   if (!b->prepared) {
-    size_t np = npoints_of(b);
-    if ((rc = grow(b, b->pts, sizeof(BaseRec) * np, 0))) return rc;
-    if ((rc = grow(b, b->cs, cs_stride(b) * b->n + 64, 0))) return rc;
-    if ((rc = grow(b, b->z, 16 * b->n_ios + 16, 0))) return rc;
-    if ((rc = grow(b, b->renc, 32 * b->n + 32, 0))) return rc;
+    if ((rc = grow_derived(b, b->n, b->n_ios))) return rc;
     CK(cudaMemsetAsync(b->flags.p, 0, 64, b->st));
     size_t nch = (b->n + PREP_CHUNK - 1) / PREP_CHUNK;
     while (b->prep_ev.size() < nch) {
@@ -789,43 +813,14 @@ int avrf_thin_batch_prepare(avrf_batch* b, int32_t* invalid) {
       CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
       b->prep_ev.push_back(e);
     }
-    PedPrepArgs pa;
-    PrepArgs ta;
-    if (b->scheme == 1) {
-      pa.pkcom = b->pk.as<Affine>(); pa.r = b->r.as<Affine>(); pa.ok = b->ok.as<Affine>(); pa.s = b->s.as<Fe>();
-      pa.sb = b->sb.as<Fe>(); pa.ios = b->ios.as<Affine>(); pa.io_off = b->io_off.as<uint32_t>();
-      pa.ad_off = b->ad_off.as<uint32_t>(); pa.ad = b->ad.as<uint8_t>(); pa.pts = b->pts.as<BaseRec>();
-      pa.cs = b->cs.as<uint32_t>(); pa.flags = b->flags.as<int>(); pa.n = (uint32_t)b->n;
-      pa.canonical = b->fmt == AVRF_FMT_CANONICAL;
-    } else {
-      ta.pk = b->pk.as<Affine>(); ta.r = b->r.as<Affine>(); ta.s = b->s.as<Fe>(); ta.ios = b->ios.as<Affine>();
-      ta.io_off = b->io_off.as<uint32_t>(); ta.ad_off = b->ad_off.as<uint32_t>(); ta.ad = b->ad.as<uint8_t>();
-      ta.pts = b->pts.as<BaseRec>(); ta.cs = b->cs.as<uint32_t>(); ta.z = b->z.as<uint32_t>();
-      ta.renc = b->renc.as<uint32_t>(); ta.flags = b->flags.as<int>(); ta.n = (uint32_t)b->n;
-      ta.canonical = b->fmt == AVRF_FMT_CANONICAL;
-    }
     // one launch per chunk, an event after each: the D2H + host hash of chunk i start while chunk i+1 runs.  The
     // launches go to the handle's high-priority stream: with several handles sharing the GPU the transcripts of this
     // batch (2 ms, and the 82 ms host hash that waits for them) must not queue behind another batch's 8 ms MSM.
     cudaStream_t ps = b->st_prep;
-    {
-      cudaEvent_t e;
-      CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      cudaEventRecord(e, b->st);                       // inputs and the flag reset are ordered on the compute stream
-      cudaStreamWaitEvent(ps, e, 0);
-      cudaEventDestroy(e);
-    }
+    if ((rc = stream_after(ps, b->st))) return rc;     // inputs and the flag reset are ordered on the compute stream
     if (nch) cudaEventRecord(b->ev[0], ps);
     for (size_t c = 0; c < nch; c++) {
-      size_t cnt = std::min((size_t)PREP_CHUNK, (size_t)b->n - c * PREP_CHUNK);
-      if (b->scheme == 1) {
-        pa.first = (uint32_t)(c * PREP_CHUNK);
-        DISPATCH(b->suite, (k_prepare_ped<S><<<cdiv(cnt, 128), 128, 0, ps>>>(pa)));
-      } else {
-        ta.first = (uint32_t)(c * PREP_CHUNK);
-        DISPATCH(b->suite, (k_prepare<S><<<cdiv(cnt, 128), 128, 0, ps>>>(ta)));
-      }
-      LAUNCHED(b->scheme == 1 ? "k_prepare_ped" : "k_prepare");
+      if ((rc = launch_prepare(b, c * PREP_CHUNK, std::min<size_t>(b->n, (c + 1) * PREP_CHUNK), ps))) return rc;
       CK(cudaEventRecord(b->prep_ev[c], ps));
     }
     if (nch) {
@@ -838,11 +833,7 @@ int avrf_thin_batch_prepare(avrf_batch* b, int32_t* invalid) {
     b->have_seed = false;
   } else {
     // prepared by the push pipeline on st_prep: order the compute stream after it
-    cudaEvent_t e;
-    CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    cudaEventRecord(e, b->st_prep);
-    cudaStreamWaitEvent(b->st, e, 0);
-    cudaEventDestroy(e);
+    if ((rc = stream_after(b->st, b->st_prep))) return rc;
   }
   if (invalid) {
     CK(cudaMemcpyAsync(b->h_small.p, b->flags.p, 8, cudaMemcpyDeviceToHost, b->st));
@@ -858,7 +849,7 @@ int avrf_thin_batch_cs_stream(avrf_batch* b, uint8_t* out) {
   if (!b || !out) return fail(AVRF_ERR_ARG, "null argument");
   int rc = avrf_thin_batch_prepare(b, nullptr);
   if (rc) return rc;
-  if (b->n) CK(cudaMemcpyAsync(out, b->cs.p, cs_stride(b) * b->n, cudaMemcpyDeviceToHost, b->st));
+  if (b->n) CK(cudaMemcpyAsync(out, b->cs.p, scheme_of(b).cs_stride * b->n, cudaMemcpyDeviceToHost, b->st));
   CK(hsync(b, b->st));
   return 0;
 }
@@ -872,19 +863,8 @@ void* avrf_thin_batch_cs_dev(avrf_batch* b) {
 
 int avrf_thin_seed(uint32_t suite, const uint8_t* cs_stream, uint64_t n_items, uint8_t seed[64]) {
   if (suite > 2 || !seed || (n_items && !cs_stream)) return fail(AVRF_ERR_ARG, "bad argument");
-  size_t sl;
-  const unsigned char* sid = suite_id_of(suite, &sl);
-  EVP_MD_CTX* ctx = EVP_MD_CTX_new();
-  if (!ctx) return fail(AVRF_ERR_NOMEM, "EVP_MD_CTX_new");
-  unsigned char tag = DOM_BATCH;
-  unsigned int outl = 64;
-  EVP_DigestInit_ex(ctx, EVP_sha512(), nullptr);
-  EVP_DigestUpdate(ctx, sid, sl);
-  EVP_DigestUpdate(ctx, &tag, 1);
-  if (n_items) EVP_DigestUpdate(ctx, cs_stream, 64 * n_items);
-  EVP_DigestFinal_ex(ctx, seed, &outl);
-  EVP_MD_CTX_free(ctx);
-  return 0;
+  unsigned char prefix[40];
+  return sha512({{prefix, batch_prefix(suite, prefix)}, {cs_stream, 64 * n_items}}, seed);
 }
 
 }  // extern "C"
@@ -917,23 +897,16 @@ static int seed_of_device_stream(cudaStream_t st, cudaStream_t st_copy, uint32_t
     CK(cudaEventRecord(evs[i], st_copy));
   }
   auto t0 = std::chrono::steady_clock::now();
-  size_t sl;
-  const unsigned char* sid = suite_id_of(suite, &sl);
-  EVP_MD_CTX* ctx = EVP_MD_CTX_new();
-  if (!ctx) return fail(AVRF_ERR_NOMEM, "EVP_MD_CTX_new");
-  unsigned char tag = DOM_BATCH;
-  unsigned int outl = 64;
-  EVP_DigestInit_ex(ctx, EVP_sha512(), nullptr);
-  EVP_DigestUpdate(ctx, sid, sl);
-  EVP_DigestUpdate(ctx, &tag, 1);
+  unsigned char prefix[40];
+  EVP_MD_CTX* ctx = sha512_begin({{prefix, batch_prefix(suite, prefix)}});
+  if (!ctx) return AVRF_ERR_NOMEM;
   cudaError_t ce = cudaSuccess;
   for (size_t i = 0; i < nch && ce == cudaSuccess; i++) {
     size_t off = i * CH, len = std::min(CH, total - off);
     ce = cudaEventSynchronize(evs[i]);
     EVP_DigestUpdate(ctx, (uint8_t*)pin.p + off, len);
   }
-  EVP_DigestFinal_ex(ctx, seed, &outl);
-  EVP_MD_CTX_free(ctx);
+  sha512_end(ctx, seed);
   if (ce != cudaSuccess) return fail(AVRF_ERR_CUDA, "cudaEventSynchronize", cudaGetErrorString(ce));
   if (hash_ms) *hash_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return 0;
@@ -947,23 +920,13 @@ static int seed_from_device(avrf_batch* b) {
   Hasher* hs = hasher_of(b);
   if (!hs || b->ext_hasher) return fail(AVRF_ERR_STATE, "no hasher for this handle");
   int rc;
-  size_t sl;
-  const unsigned char* sid = suite_id_of(b->suite, &sl);
   unsigned char prefix[40];
-  memcpy(prefix, sid, sl);
-  prefix[sl] = DOM_BATCH;
-  if ((rc = hs->begin(prefix, sl + 1))) return rc;
-  const size_t stride = cs_stride(b), total = stride * b->n, CH = stride * PREP_CHUNK;
+  if ((rc = hs->begin(prefix, batch_prefix(b->suite, prefix)))) return rc;
+  const size_t stride = scheme_of(b).cs_stride, total = stride * b->n, CH = stride * PREP_CHUNK;
   const size_t nch = (total + CH - 1) / CH;
   if ((rc = hs->reserve_stage(std::min(total, 16 * CH) + 64 * (nch + 1)))) return rc;
   const bool per_chunk = b->prep_ev_chunks >= nch && b->prep_ev.size() >= nch;      // this batch's own chunk events
-  if (!per_chunk) {
-    cudaEvent_t ready;
-    CK(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-    cudaEventRecord(ready, b->st);
-    cudaStreamWaitEvent(b->st_copy, ready, 0);
-    cudaEventDestroy(ready);
-  }
+  if (!per_chunk && (rc = stream_after(b->st_copy, b->st))) return rc;
   auto t0 = std::chrono::steady_clock::now();
   for (size_t i = 0; i < nch; i++) {
     size_t off = i * CH, len = std::min(CH, total - off);
@@ -1000,10 +963,11 @@ static void seed_to_words(Seed64& sd, const uint8_t seed[64]) {
 // b->partial and flags[1] (and in b->remote_slot for the shards of a multi-GPU batch).
 static int run_msm(avrf_batch* b, const uint8_t seed[64], uint64_t first_index) {
   int rc;
-  size_t np = npoints_of(b);
+  const Scheme& sc = scheme_of(b);
+  size_t np = sc.points(b->n, b->n_ios);
   if (np >= (1ull << 28)) return fail(AVRF_ERR_ARG, "batch too large for one handle (2^28 MSM terms): shard it");
   size_t max_entries = np * MSM_NWIN;
-  uint32_t nblk = cdiv(b->n, 128 * (b->scheme ? 1 : SCAL_PER_THREAD));
+  uint32_t nblk = cdiv(b->n, 128 * sc.scal_per_thread);
   // accumulation grid: four waves of resident blocks (lazy-reduction additions: 120-126 registers, 4 blocks of 128 threads
   // per SM; Ed25519 5), every thread an equal share of the sorted entries
   // (measured at 2^20 proofs: 1 wave 7.38 ms - the slowest SM sets the time -, 2 waves 7.14, 4 waves 6.99, 8 waves 6.92 with
@@ -1280,16 +1244,8 @@ int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios,
   if (!b || b->scheme != 1) return fail(AVRF_ERR_ARG, "not a Pedersen batch");
   if (n == 0) return 0;
   if (!io_offsets || !ad_offsets || !pk_com || !r || !ok || !s || !sb) return fail(AVRF_ERR_ARG, "null argument");
-  if (io_offsets[0] != 0 || ad_offsets[0] != 0) return fail(AVRF_ERR_ARG, "offsets must start at 0");
-  uint64_t add_ios = io_offsets[n], add_ad = ad_offsets[n];
-  if ((add_ios && !ios) || (add_ad && !ad_blob)) return fail(AVRF_ERR_ARG, "null argument");
-  ENTER(b);
   // same pipeline as the thin verifier: chunked H2D -> k_prepare_ped -> D2H of (c, s, sb) -> incremental SHA-512
-  int rc = push_many_impl(b, n, pk_com, ios, io_offsets, ad_blob, ad_offsets, r, s, ok, sb);
-  if (rc) return rc;
-  CK(hsync(b, b->st_h2d));     // the caller's buffers are only borrowed for the duration of the call
-  CK(hsync(b, b->prepared ? b->st_prep : b->st));
-  return 0;
+  return push_borrowed(b, n, {pk_com, r, s, ok, sb}, ios, io_offsets, ad_blob, ad_offsets);
 }
 
 int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status) {
@@ -1297,7 +1253,7 @@ int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status) {
   return avrf_thin_batch_verify(b, status);
 }
 
-// ---- thin::Verifier::verify (src/thin.rs:131-165): the exact single-proof equation ---------------
+// ---- the exact single-proof verifiers ---------------------------------------------------------------------------
 // One small context per host thread and device: a pinned + a device buffer and a stream, reused across calls.
 struct OneCtx {
   int device = -1;
@@ -1306,49 +1262,34 @@ struct OneCtx {
   DevBuf dev;
 };
 
-static int one_ctx(OneCtx** out) {
+// One proof through a single-proof verifier kernel.  Its input on the device: the proof's fixed-size fields (`proof`),
+// n_ios (u32), ad_len (u32), 8 zero bytes, the I/O pairs and ad; then `scratch` bytes at the next 256-byte boundary, and
+// the two status words after them.  `launch` starts the kernel on the given stream with (input, scratch, status).
+using OneLaunch = std::function<int(cudaStream_t, const uint8_t*, uint8_t*, int32_t*)>;
+static int run_one(std::initializer_list<ByteRange> proof, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
+                   uint32_t ad_len, size_t scratch, const OneLaunch& launch, int32_t* status) {
   static thread_local OneCtx ctx;
-  int dev = g_device.load();
+  int rc, dev = g_device.load();
   if (ctx.device != dev) {
     if (!ctx.st) CK(cudaStreamCreateWithFlags(&ctx.st, cudaStreamNonBlocking));
     ctx.device = dev;
   }
-  *out = &ctx;
-  return 0;
-}
-
-int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios,
-                         const uint8_t* ad, uint32_t ad_len, const uint8_t r[64], const uint8_t s[32], int32_t* status) {
-  if (suite > 2 || fmt > 1) return fail(AVRF_ERR_ARG, "bad suite/fmt");
-  if (!pk || !r || !s || !status || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
-  if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
-  NEED_DEVICE();
-  OneCtx* cp;
-  int rc = one_ctx(&cp);
-  if (rc) return rc;
-  OneCtx& ctx = *cp;
-  size_t in_bytes = 176 + 128 * (size_t)n_ios + ad_len;
-  size_t z_off = (in_bytes + 255) & ~(size_t)255, st_off = z_off + 16 * (size_t)n_ios + 16;
-  size_t total = st_off + 64;
+  size_t head = 16;
+  for (const ByteRange& f : proof) head += f.n;
+  size_t in_bytes = head + 128 * (size_t)n_ios + ad_len;
+  size_t scr_off = (in_bytes + 255) & ~(size_t)255, st_off = scr_off + scratch, total = st_off + 64;
   if ((rc = ctx.pin.reserve(total)) || (rc = ctx.dev.reserve(total, 0, ctx.st))) return rc;
   uint8_t* h = ctx.pin.as<uint8_t>();
-  memcpy(h, pk, 64);
-  memcpy(h + 64, r, 64);
-  memcpy(h + 128, s, 32);
-  memcpy(h + 160, &n_ios, 4);
-  memcpy(h + 164, &ad_len, 4);
-  memset(h + 168, 0, 8);
-  if (n_ios) memcpy(h + 176, ios, 128 * (size_t)n_ios);
-  if (ad_len) memcpy(h + 176 + 128 * (size_t)n_ios, ad, ad_len);
+  for (const ByteRange& f : proof) { memcpy(h, f.p, f.n); h += f.n; }
+  memcpy(h, &n_ios, 4);
+  memcpy(h + 4, &ad_len, 4);
+  memset(h + 8, 0, 8);
+  if (n_ios) memcpy(h + 16, ios, 128 * (size_t)n_ios);
+  if (ad_len) memcpy(h + 16 + 128 * (size_t)n_ios, ad, ad_len);
+  h = ctx.pin.as<uint8_t>();
   uint8_t* d = ctx.dev.as<uint8_t>();
   CK(cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx.st));
-  OneArgs a;
-  a.in = d;
-  a.z = reinterpret_cast<uint32_t*>(d + z_off);
-  a.status = reinterpret_cast<int32_t*>(d + st_off);
-  a.canonical = fmt == AVRF_FMT_CANONICAL;
-  DISPATCH(suite, (k_verify_one<S><<<1, 32, 0, ctx.st>>>(a)));
-  LAUNCHED("k_verify_one");
+  if ((rc = launch(ctx.st, d, d + scr_off, reinterpret_cast<int32_t*>(d + st_off)))) return rc;
   CK(cudaMemcpyAsync(h + st_off, d + st_off, 8, cudaMemcpyDeviceToHost, ctx.st));
   CK(cudaStreamSynchronize(ctx.st));
   const int32_t* out = reinterpret_cast<const int32_t*>(h + st_off);
@@ -1357,7 +1298,27 @@ int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], con
   return 0;
 }
 
-// ---- pedersen::Verifier::verify (src/pedersen.rs:188-253): both equations, exact, one thread -------------------
+// thin::Verifier::verify (src/thin.rs:131-165): the exact single-proof equation; 16 bytes of z scratch per pair
+int avrf_thin_verify_one(uint32_t suite, uint32_t fmt, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios,
+                         const uint8_t* ad, uint32_t ad_len, const uint8_t r[64], const uint8_t s[32], int32_t* status) {
+  if (suite > 2 || fmt > 1) return fail(AVRF_ERR_ARG, "bad suite/fmt");
+  if (!pk || !r || !s || !status || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
+  if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
+  NEED_DEVICE();
+  return run_one({{pk, 64}, {r, 64}, {s, 32}}, ios, n_ios, ad, ad_len, 16 * (size_t)n_ios + 16,
+                 [&](cudaStream_t st, const uint8_t* in, uint8_t* z, int32_t* out) {
+                   OneArgs a;
+                   a.in = in;
+                   a.z = reinterpret_cast<uint32_t*>(z);
+                   a.status = out;
+                   a.canonical = fmt == AVRF_FMT_CANONICAL;
+                   DISPATCH(suite, (k_verify_one<S><<<1, 32, 0, st>>>(a)));
+                   LAUNCHED("k_verify_one");
+                   return 0;
+                 }, status);
+}
+
+// pedersen::Verifier::verify (src/pedersen.rs:188-253): both equations, exact, one thread
 int avrf_pedersen_verify_one(uint32_t suite, uint32_t fmt, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
                              uint32_t ad_len, const uint8_t pk_com[64], const uint8_t r[64], const uint8_t ok[64],
                              const uint8_t s[32], const uint8_t sb[32], int32_t* status) {
@@ -1366,38 +1327,16 @@ int avrf_pedersen_verify_one(uint32_t suite, uint32_t fmt, const uint8_t* ios, u
     return fail(AVRF_ERR_ARG, "null argument");
   if (n_ios >= (1u << 20)) return fail(AVRF_ERR_ARG, "too many I/O pairs");
   NEED_DEVICE();
-  OneCtx* cp;
-  int rc = one_ctx(&cp);
-  if (rc) return rc;
-  OneCtx& ctx = *cp;
-  size_t in_bytes = 272 + 128 * (size_t)n_ios + ad_len;
-  size_t st_off = (in_bytes + 255) & ~(size_t)255, total = st_off + 64;
-  if ((rc = ctx.pin.reserve(total)) || (rc = ctx.dev.reserve(total, 0, ctx.st))) return rc;
-  uint8_t* h = ctx.pin.as<uint8_t>();
-  memcpy(h, pk_com, 64);
-  memcpy(h + 64, r, 64);
-  memcpy(h + 128, ok, 64);
-  memcpy(h + 192, s, 32);
-  memcpy(h + 224, sb, 32);
-  memcpy(h + 256, &n_ios, 4);
-  memcpy(h + 260, &ad_len, 4);
-  memset(h + 264, 0, 8);
-  if (n_ios) memcpy(h + 272, ios, 128 * (size_t)n_ios);
-  if (ad_len) memcpy(h + 272 + 128 * (size_t)n_ios, ad, ad_len);
-  uint8_t* d = ctx.dev.as<uint8_t>();
-  CK(cudaMemcpyAsync(d, h, in_bytes, cudaMemcpyHostToDevice, ctx.st));
-  PedOneArgs a;
-  a.in = d;
-  a.status = reinterpret_cast<int32_t*>(d + st_off);
-  a.canonical = fmt == AVRF_FMT_CANONICAL;
-  DISPATCH(suite, (k_verify_one_ped<S><<<1, 32, 0, ctx.st>>>(a)));
-  LAUNCHED("k_verify_one_ped");
-  CK(cudaMemcpyAsync(h + st_off, d + st_off, 8, cudaMemcpyDeviceToHost, ctx.st));
-  CK(cudaStreamSynchronize(ctx.st));
-  const int32_t* out = reinterpret_cast<const int32_t*>(h + st_off);
-  if (out[1] & 2) return fail(AVRF_ERR_ARG, "an input coordinate or scalar is not below its modulus (not a field element)");
-  *status = out[0];
-  return 0;
+  return run_one({{pk_com, 64}, {r, 64}, {ok, 64}, {s, 32}, {sb, 32}}, ios, n_ios, ad, ad_len, 0,
+                 [&](cudaStream_t st, const uint8_t* in, uint8_t*, int32_t* out) {
+                   PedOneArgs a;
+                   a.in = in;
+                   a.status = out;
+                   a.canonical = fmt == AVRF_FMT_CANONICAL;
+                   DISPATCH(suite, (k_verify_one_ped<S><<<1, 32, 0, st>>>(a)));
+                   LAUNCHED("k_verify_one_ped");
+                   return 0;
+                 }, status);
 }
 
 int avrf_thin_batch_timings(const avrf_batch* b, avrf_timings* out) {
@@ -1420,7 +1359,7 @@ int avrf_thin_batch_tap(avrf_batch* b, uint32_t what, void* out, size_t out_byte
     case AVRF_TAP_C: {
       if ((rc = avrf_thin_batch_prepare(b, nullptr))) return rc;
       if (out_bytes < 16 * b->n) return fail(AVRF_ERR_ARG, "tap buffer too small");
-      if (b->n) CK(cudaMemcpy2DAsync(out, 16, b->cs.p, cs_stride(b), 16, b->n, cudaMemcpyDeviceToHost, b->st));
+      if (b->n) CK(cudaMemcpy2DAsync(out, 16, b->cs.p, scheme_of(b).cs_stride, 16, b->n, cudaMemcpyDeviceToHost, b->st));
       CK(hsync(b, b->st));
       return 0;
     }
@@ -1444,7 +1383,8 @@ int avrf_thin_batch_tap(avrf_batch* b, uint32_t what, void* out, size_t out_byte
       rc = run_msm(b, b->seed, b->first_index);
       b->want_taps = false;
       if (rc) return rc;
-      return what == AVRF_TAP_W ? d2h(b->w_tap.p, (b->scheme ? 32 : 16) * b->n) : d2h(b->scalars_tap.p, 32 * npoints_of(b));
+      const Scheme& sc = scheme_of(b);
+      return what == AVRF_TAP_W ? d2h(b->w_tap.p, sc.w_tap * b->n) : d2h(b->scalars_tap.p, 32 * sc.points(b->n, b->n_ios));
     }
     case AVRF_TAP_PARTIAL:
       if (!b->have_seed || !b->partial.p) return fail(AVRF_ERR_STATE, "no partial yet");
@@ -1454,24 +1394,33 @@ int avrf_thin_batch_tap(avrf_batch* b, uint32_t what, void* out, size_t out_byte
   }
 }
 
+// Per-proof verdicts of a prepared batch: `launch` writes one status word per proof on b->st, copied back to `statuses`.
+static int verdicts(avrf_batch* b, int32_t* statuses, const std::function<int(int32_t*)>& launch) {
+  if (b->n == 0) return 0;
+  DevBuf dst;
+  int rc;
+  if ((rc = dst.reserve(4 * b->n, 0, b->st))) return rc;
+  if ((rc = launch(dst.as<int32_t>()))) return rc;
+  CK(cudaMemcpyAsync(statuses, dst.p, 4 * b->n, cudaMemcpyDeviceToHost, b->st));
+  CK(hsync(b, b->st));
+  return 0;
+}
+
 int avrf_thin_batch_verify_each(avrf_batch* b, int32_t* statuses) {
   if (!b || !statuses) return fail(AVRF_ERR_ARG, "null argument");
   if (b->scheme != 0) return fail(AVRF_ERR_ARG, "not a Thin-VRF batch");
   int rc = avrf_thin_batch_prepare(b, nullptr);
   if (rc) return rc;
-  if (b->n == 0) return 0;
-  DevBuf dst;
-  if ((rc = dst.reserve(4 * b->n, 0, b->st))) return rc;
-  EachArgs a;
-  a.pk = b->pk.as<Affine>(); a.r = b->r.as<Affine>(); a.ios = b->ios.as<Affine>();
-  a.canonical = b->fmt == AVRF_FMT_CANONICAL;
-  a.cs = b->cs.as<uint32_t>(); a.z = b->z.as<uint32_t>();
-  a.io_off = b->io_off.as<uint32_t>(); a.status = dst.as<int32_t>(); a.n = (uint32_t)b->n;
-  DISPATCH(b->suite, (k_verify_each<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
-  LAUNCHED("k_verify_each");
-  CK(cudaMemcpyAsync(statuses, dst.p, 4 * b->n, cudaMemcpyDeviceToHost, b->st));
-  CK(hsync(b, b->st));
-  return 0;
+  return verdicts(b, statuses, [&](int32_t* out) {
+    EachArgs a;
+    a.pk = b->pk.as<Affine>(); a.r = b->r.as<Affine>(); a.ios = b->ios.as<Affine>();
+    a.canonical = b->fmt == AVRF_FMT_CANONICAL;
+    a.cs = b->cs.as<uint32_t>(); a.z = b->z.as<uint32_t>();
+    a.io_off = b->io_off.as<uint32_t>(); a.status = out; a.n = (uint32_t)b->n;
+    DISPATCH(b->suite, (k_verify_each<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
+    LAUNCHED("k_verify_each");
+    return 0;
+  });
 }
 
 int avrf_pedersen_batch_verify_each(avrf_batch* b, int32_t* statuses) {
@@ -1480,18 +1429,15 @@ int avrf_pedersen_batch_verify_each(avrf_batch* b, int32_t* statuses) {
   int32_t invalid = 0;                  // (per-proof verdicts below; this call only surfaces out-of-range inputs)
   int rc = avrf_thin_batch_prepare(b, &invalid);
   if (rc) return rc;
-  if (b->n == 0) return 0;
-  DevBuf dst;
-  if ((rc = dst.reserve(4 * b->n, 0, b->st))) return rc;
-  PedEachArgs a;
-  a.pkcom = b->pk.as<Affine>(); a.ios = b->ios.as<Affine>(); a.io_off = b->io_off.as<uint32_t>();
-  a.canonical = b->fmt == AVRF_FMT_CANONICAL;
-  a.pts = b->pts.as<BaseRec>(); a.cs = b->cs.as<uint32_t>(); a.status = dst.as<int32_t>(); a.n = (uint32_t)b->n;
-  DISPATCH(b->suite, (k_verify_each_ped<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
-  LAUNCHED("k_verify_each_ped");
-  CK(cudaMemcpyAsync(statuses, dst.p, 4 * b->n, cudaMemcpyDeviceToHost, b->st));
-  CK(hsync(b, b->st));
-  return 0;
+  return verdicts(b, statuses, [&](int32_t* out) {
+    PedEachArgs a;
+    a.pkcom = b->pk.as<Affine>(); a.ios = b->ios.as<Affine>(); a.io_off = b->io_off.as<uint32_t>();
+    a.canonical = b->fmt == AVRF_FMT_CANONICAL;
+    a.pts = b->pts.as<BaseRec>(); a.cs = b->cs.as<uint32_t>(); a.status = out; a.n = (uint32_t)b->n;
+    DISPATCH(b->suite, (k_verify_each_ped<S><<<cdiv(b->n, 128), 128, 0, b->st>>>(a)));
+    LAUNCHED("k_verify_each_ped");
+    return 0;
+  });
 }
 
 #include "feed_api.inl"     // hash-to-curve, outputs, proving, ingest, compression, microbenchmarks

@@ -11,6 +11,7 @@
 #include <cstdio>
 #include <cstring>
 #include <deque>
+#include <initializer_list>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -167,6 +168,31 @@ struct EventPool {
 };
 
 static inline uint32_t cdiv(size_t a, size_t b) { return (uint32_t)((a + b - 1) / b); }
+
+// ---- SHA-512 on the calling thread --------------------------------------------------------
+struct ByteRange {
+  const void* p;
+  size_t n;
+};
+// A SHA-512 context that has absorbed `parts`; nullptr (with the error set) when it cannot be allocated.
+static EVP_MD_CTX* sha512_begin(std::initializer_list<ByteRange> parts) {
+  EVP_MD_CTX* ctx = EVP_MD_CTX_new();
+  if (!ctx) { fail(AVRF_ERR_NOMEM, "EVP_MD_CTX_new"); return nullptr; }
+  EVP_DigestInit_ex(ctx, EVP_sha512(), nullptr);
+  for (const ByteRange& r : parts) if (r.n) EVP_DigestUpdate(ctx, r.p, r.n);
+  return ctx;
+}
+static void sha512_end(EVP_MD_CTX* ctx, uint8_t out[64]) {
+  unsigned int outl = 64;
+  EVP_DigestFinal_ex(ctx, out, &outl);
+  EVP_MD_CTX_free(ctx);
+}
+static int sha512(std::initializer_list<ByteRange> parts, uint8_t out[64]) {
+  EVP_MD_CTX* ctx = sha512_begin(parts);
+  if (!ctx) return AVRF_ERR_NOMEM;
+  sha512_end(ctx, out);
+  return 0;
+}
 
 // ---- hasher -------------------------------------------------------------------------------
 // The batch seed is ONE serial SHA-512 over SUITE_ID || 0x50 || (c_j, s_j)... (src/thin.rs:273-279).  A Hasher

@@ -269,6 +269,44 @@ def test_full_size(av):
     assert list(bv.find_invalid()) == bad
 
 
+def test_reserve_slices_and_invalidate(av):
+    """A Pedersen handle through avrf_thin_batch_reserve (smaller than the batch), two uneven push_many slices (the
+    second one longer than a k_prepare chunk of 75 776 proofs) and, after avrf_thin_batch_invalidate, the prepare of
+    the resident inputs: seed, C, W and SCALARS taps bit-identical to one push_many of the whole batch, and one
+    corrupted sb named by find_invalid."""
+    from ark_vrf_b200 import pedersen as ped, synth
+    n, k, bad = 100_000, 20_000, 77_777
+    b = synth.make_pedersen_batch(0, n, 1)
+    taps = (av.Tap.SEED, av.Tap.C, av.Tap.W, av.Tap.SCALARS)
+    ref = ped.BatchVerifier(0, b.fmt)
+    ref.push_many(b.ios, b.io_offsets, b.ad_blob, b.ad_offsets, b.pk_com, b.r, b.ok, b.s, b.sb)
+    assert ref.verify_status() == 0
+    want = [bytes(ref.tap(t)) for t in taps]
+    lib = av.load()
+
+    def push_two(bv, sb):
+        h, ao = b.io_offsets, b.ad_offsets
+        bv.push_many(b.ios, h[:k + 1], b.ad_blob, ao[:k + 1], b.pk_com[:k], b.r[:k], b.ok[:k], b.s[:k], sb[:k])
+        q, a = int(h[k]), int(ao[k])
+        bv.push_many(b.ios[q:], (h[k:] - q).astype(np.uint32), b.ad_blob[a:], (ao[k:] - a).astype(np.uint32),
+                     b.pk_com[k:], b.r[k:], b.ok[k:], b.s[k:], sb[k:])
+
+    bv = ped.BatchVerifier(0, b.fmt)
+    assert lib.avrf_thin_batch_reserve(bv._h, n // 2, n // 2, len(b.ad_blob) // 2) == 0
+    push_two(bv, b.sb)
+    assert bv.verify_status() == 0
+    assert [bytes(bv.tap(t)) for t in taps] == want
+    assert lib.avrf_thin_batch_invalidate(bv._h) == 0
+    assert bv.verify_status() == 0
+    assert [bytes(bv.tap(t)) for t in taps] == want
+    sb2 = b.sb.copy()
+    sb2[bad, 0] ^= 1
+    bv.clear()
+    push_two(bv, sb2)
+    assert bv.verify_status() == 1
+    assert list(bv.find_invalid()) == [bad]
+
+
 def test_cpp_pedersen_driver(av):
     """include/avrf.hpp's ark_vrf::pedersen through a compiled driver: prove, verify, batch verify, verify_each."""
     import struct
