@@ -245,6 +245,49 @@ static void feed_pool_release(int dev) {
   fp.w.u01.release(); fp.w.den.release(); fp.w.scr.release();
 }
 
+// One call over a device's feed pool: holds the pool for the duration of the call, hands out its buffers in order and
+// stages the call's copies on `st`.  The first error is kept in `rc` and turns every later buffer or copy into a no-op,
+// so a caller checks `rc` once before it launches.
+struct FeedFrame {
+  FeedPool& fp;
+  std::lock_guard<std::mutex> lock;
+  cudaStream_t st;
+  int rc = 0;
+  FeedFrame(int device, cudaStream_t s) : fp(g_feed[device]), lock(fp.mu), st(s) {}
+  H2cScratch& scratch() { return fp.w; }
+  // the next pool buffer, grown to at least `bytes` (an empty buffer once an error is kept)
+  DevBuf& take(size_t bytes) {
+    if (!rc && used == std::size(fp.b)) rc = fail(AVRF_ERR_STATE, "feed pool exhausted");
+    if (rc) return none;
+    DevBuf& d = fp.b[used++];
+    rc = d.reserve(bytes);
+    return d;
+  }
+  // the next pool buffer, grown to `bytes + slack`, with `bytes` of host memory copied in
+  DevBuf& in(const void* h, size_t bytes, size_t slack = 0) {
+    DevBuf& d = take(bytes + slack);
+    if (!rc && bytes) rc = copy(d.p, h, bytes, cudaMemcpyHostToDevice);
+    return d;
+  }
+  // `bytes` of device memory back to `h`; nothing when `h` is null (an output the caller did not ask for).  Returns
+  // the kept error, for a caller that launches more work after the copy.
+  int out(void* h, const void* d, size_t bytes) {
+    if (!rc && h) rc = copy(h, d, bytes, cudaMemcpyDeviceToHost);
+    return rc;
+  }
+  // the end of the call: waits for the stream, so that every output has landed
+  int sync() {
+    if (!rc) rc = wait();
+    return rc;
+  }
+
+ private:
+  size_t used = 0;
+  DevBuf none;
+  int copy(void* dst, const void* src, size_t bytes, cudaMemcpyKind kind) { CK(cudaMemcpyAsync(dst, src, bytes, kind, st)); return 0; }
+  int wait() { CK(cudaStreamSynchronize(st)); return 0; }
+};
+
 // MSM gate: the heavy part of the MSMs of different handles on one device (scalars, sort, bucket accumulation) runs
 // one batch after the other, in submission order.  Left to themselves the streams of T handles interleave kernel by
 // kernel, all T MSMs finish together after T x 10 ms, and no handle can start hashing its next batch before that;
@@ -870,33 +913,25 @@ int avrf_thin_seed(uint32_t suite, const uint8_t* cs_stream, uint64_t n_items, u
 }  // extern "C"
 
 // Device->host copy of a (c,s) stream in chunks on the copy stream, each chunk hashed on the host
-// as soon as it lands: the serial SHA-512 of thin.rs:273-279 (SURVEY.md H1).  `chunk_ready` (optional): one event
-// per chunk, recorded when the kernel that produces that chunk has finished.
+// as soon as it lands: the serial SHA-512 of thin.rs:273-279 (SURVEY.md H1).
 static int seed_of_device_stream(cudaStream_t st, cudaStream_t st_copy, uint32_t suite, const uint8_t* cs_dev,
-                                 size_t total, PinBuf& pin, uint8_t seed[64], float* hash_ms,
-                                 const std::vector<cudaEvent_t>* chunk_ready = nullptr, size_t n_ready = 0, size_t stride = 64,
-                                 bool blocking = false) {
+                                 size_t total, PinBuf& pin, uint8_t seed[64]) {
   int rc;
   if ((rc = pin.reserve(total + 64))) return rc;
-  const size_t CH = stride * PREP_CHUNK;  // one k_prepare chunk: 4.6 MiB (thin) / 6.9 MiB (pedersen)
+  const size_t CH = 64 * PREP_CHUNK;      // one k_prepare chunk: 4.6 MiB
   size_t nch = (total + CH - 1) / CH;
-  if (chunk_ready && (n_ready < nch || chunk_ready->size() < nch)) chunk_ready = nullptr;   // not this batch's events
   EventPool pool;
   std::vector<cudaEvent_t> evs(nch);
-  if (!chunk_ready) {
-    cudaEvent_t ready = pool.make();
-    if (!ready) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
-    CK(cudaEventRecord(ready, st));
-    CK(cudaStreamWaitEvent(st_copy, ready, 0));
-  }
+  cudaEvent_t ready = pool.make();
+  if (!ready) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
+  CK(cudaEventRecord(ready, st));
+  CK(cudaStreamWaitEvent(st_copy, ready, 0));
   for (size_t i = 0; i < nch; i++) {
     size_t off = i * CH, len = std::min(CH, total - off);
-    if (chunk_ready) CK(cudaStreamWaitEvent(st_copy, (*chunk_ready)[i], 0));
     CK(cudaMemcpyAsync((uint8_t*)pin.p + off, cs_dev + off, len, cudaMemcpyDeviceToHost, st_copy));
-    if (!(evs[i] = pool.make(cudaEventDisableTiming | (blocking ? cudaEventBlockingSync : 0)))) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
+    if (!(evs[i] = pool.make())) return fail(AVRF_ERR_CUDA, "cudaEventCreate");
     CK(cudaEventRecord(evs[i], st_copy));
   }
-  auto t0 = std::chrono::steady_clock::now();
   unsigned char prefix[40];
   EVP_MD_CTX* ctx = sha512_begin({{prefix, batch_prefix(suite, prefix)}});
   if (!ctx) return AVRF_ERR_NOMEM;
@@ -908,7 +943,6 @@ static int seed_of_device_stream(cudaStream_t st, cudaStream_t st_copy, uint32_t
   }
   sha512_end(ctx, seed);
   if (ce != cudaSuccess) return fail(AVRF_ERR_CUDA, "cudaEventSynchronize", cudaGetErrorString(ce));
-  if (hash_ms) *hash_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return 0;
 }
 
@@ -1118,7 +1152,7 @@ int avrf_thin_seed_dev(uint32_t suite, const void* cs_stream_dev, uint64_t n_ite
   if (suite > 2 || !seed || (n_items && !cs_stream_dev)) return fail(AVRF_ERR_ARG, "bad argument");
   NEED_DEVICE();
   std::lock_guard<std::mutex> lock(g_pin_mu);
-  return seed_of_device_stream(gs(), gc(), suite, (const uint8_t*)cs_stream_dev, 64 * n_items, g_pin_stream[g_device.load()], seed, nullptr);
+  return seed_of_device_stream(gs(), gc(), suite, (const uint8_t*)cs_stream_dev, 64 * n_items, g_pin_stream[g_device.load()], seed);
 }
 
 int avrf_thin_batch_partial(avrf_batch* b, const uint8_t seed[64], uint64_t first_index, uint8_t partial[128]) {
@@ -1141,15 +1175,17 @@ int avrf_thin_batch_partial(avrf_batch* b, const uint8_t seed[64], uint64_t firs
 int avrf_thin_combine_partials(uint32_t suite, const uint8_t* partials, uint32_t n, int32_t* status) {
   if (suite > 2 || !partials || !status || n == 0) return fail(AVRF_ERR_ARG, "bad argument");
   NEED_DEVICE();
-  DevBuf in, out, flags;
-  int rc;
-  if ((rc = in.reserve(128 * (size_t)n)) || (rc = out.reserve(128)) || (rc = flags.reserve(64))) return rc;
-  CK(cudaMemcpyAsync(in.p, partials, 128 * (size_t)n, cudaMemcpyHostToDevice, gs()));
-  DISPATCH(suite, (k_combine_partials<S><<<1, 32, 0, gs()>>>(in.as<Ext>(), n, out.as<Ext>(), flags.as<int>())));
+  FeedFrame f(g_device.load(), gs());
+  DevBuf& in = f.in(partials, 128 * (size_t)n);
+  DevBuf& out = f.take(128);
+  DevBuf& flags = f.take(64);
+  if (f.rc) return f.rc;
+  DISPATCH(suite, (k_combine_partials<S><<<1, 32, 0, f.st>>>(in.as<Ext>(), n, out.as<Ext>(), flags.as<int>())));
   LAUNCHED("k_combine_partials");
   int h[2] = {0, 0};
-  CK(cudaMemcpyAsync(h, flags.p, 8, cudaMemcpyDeviceToHost, gs()));
-  CK(cudaStreamSynchronize(gs()));
+  f.out(h, flags.p, 8);
+  int rc = f.sync();
+  if (rc) return rc;
   *status = h[1] ? AVRF_OK : AVRF_VERIFICATION_FAILURE;
   return 0;
 }

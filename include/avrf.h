@@ -340,9 +340,15 @@ typedef struct avrf_timings {
 } avrf_timings;
 int avrf_thin_batch_timings(const avrf_batch* b, avrf_timings* out);
 
-/* Integer-multiply roofline probe: runs dependency-free IMAD.WIDE.U32 streams on every SM and
- * returns wide MACs per second (kind 0), Montgomery multiplications per second (kind 1), or
- * mixed point additions per second (kind 2). */
+/* Integer-multiply roofline probe: runs dependency-free multiply streams on every SM and returns
+ * operations per second:
+ *   kind 0: wide MACs (IMAD.WIDE.U32);
+ *   kind 1: Montgomery multiplications;
+ *   kind 2: mixed point additions;
+ *   kind 3: wide MACs in the carry-chained rows of the field multiplication (IMAD.WIDE.U32.X);
+ *   kind 4: 32-bit MACs (IMAD);
+ *   kind 6, 7: wide MACs with the carry out only / the carry in only.
+ * Any other kind is AVRF_ERR_ARG. */
 int avrf_microbench(uint32_t kind, uint32_t iters, double* per_second, float* ms);
 
 /* ---- Batch server: the throughput mode -----------------------------------------------------
