@@ -111,7 +111,7 @@ class BatchVerifier:
 
     def tap(self, what: Tap) -> np.ndarray:
         n = self._n
-        size = {Tap.C: 16 * n, Tap.W: 32 * n, Tap.SEED: 64, Tap.SCALARS: 32 * (5 * n + 2)}[Tap(what)]
+        size = {Tap.C: 16 * n, Tap.W: 32 * n, Tap.SEED: 64, Tap.SCALARS: 32 * (5 * n + 2), Tap.PARTIAL: 128}[Tap(what)]
         buf = np.zeros(max(size, 1), dtype=np.uint8)
         _lib.check(self._lib.avrf_thin_batch_tap(self._h, int(what), ptr(buf), buf.nbytes))
         return buf

@@ -243,7 +243,8 @@ avrf_batch* avrf_thin_sharded_shard(avrf_sharded* sh, int index);
 
 /* ---- Pedersen VRF batch verifier (SURVEY 8f-3; reference src/pedersen.rs:255-427) on the same MSM engine ---
  * pedersen::BatchVerifier::new / push (x n) / verify.  The handle is an avrf_batch: _free, _clear, _len,
- * _tap (C, SEED, W = t_i||u_i, SCALARS) apply; proofs are (pk_com 64, r 64, ok 64, s 32, sb 32). */
+ * _tap (C, SEED, W = t_i||u_i, SCALARS, PARTIAL = the 5N+2-point MSM sum) apply; proofs are (pk_com 64, r 64,
+ * ok 64, s 32, sb 32). */
 avrf_batch* avrf_pedersen_batch_new(uint32_t suite, uint32_t fmt);
 int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
                                   const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,

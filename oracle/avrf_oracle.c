@@ -444,9 +444,11 @@ static void* window_worker(void* arg) {
   }
   free(buckets); return NULL;
 }
-static void msm(const sctx* S, ext* out, const aff* bases, const fe* scalars, size_t n, int nthreads) {
+/* `bits`: scalar width the windows must cover (ark-ec: the scalar field's MODULUS_BIT_SIZE); the last window's
+ * signed digit absorbs the final carry as long as every scalar is below 2^bits. */
+static void msm(const sctx* S, ext* out, const aff* bases, const fe* scalars, size_t n, int bits, int nthreads) {
   int c = n < 32 ? 3 : (int)(log((double)n)) + 2;                         /* ark-ec ln_without_floats(n) + 2 */
-  int bits = S->Fr.bits, nwin = (bits + c - 1) / c + 1;
+  int nwin = (bits + c - 1) / c + 1;
   int32_t* digits = (int32_t*)malloc(n * (size_t)nwin * sizeof(int32_t));
   for (size_t i = 0; i < n; i++) {                                        /* make_digits: signed radix 2^c */
     u64 carry = 0; const u64* k = scalars[i].v;
@@ -515,13 +517,31 @@ int orc_thin_batch_verify(int s, size_t n, const uint8_t* pk, const uint8_t* ios
     }
     bases[np - 1] = S->G; scalars[np - 1] = g;                                                 /* thin.rs:315-317 */
     if (scalars32) memcpy(scalars32, scalars, 32 * np);
-    ext res; msm(S, &res, bases, scalars, np, nthreads);                                       /* thin.rs:319 */
+    ext res; msm(S, &res, bases, scalars, np, S->Fr.bits, nthreads);                           /* thin.rs:319 */
     status = ext_is_id(&res) ? ORC_OK : ORC_VERIFICATION_FAILURE;                              /* thin.rs:320-324 */
   }
 done:
   if (times) { times[0] = t1 - t0; times[1] = now_s() - t1; }
   free(bases); free(scalars); free(c); free(z);
   return status;
+}
+
+/* sum_i k_i * P_i by the same msm() the batch verifier runs, for checking another MSM against it.  bases64: n canonical
+ * affine points (any curve point: nothing is reduced into the subgroup); scalars32: n canonical little-endian integers,
+ * any value below 2^256, used as they are (not reduced mod r, so a small-order component of a base keeps the exact
+ * residue of its scalar).  out64: the canonical affine sum.  Returns 1 if the sum is the identity, 0 if not, -1 on a
+ * bad suite. */
+int orc_msm(int s, size_t n, const uint8_t* bases64, const uint8_t* scalars32, int nthreads, uint8_t out64[64]) {
+  const sctx* S = suite(s); if (!S) return -1;
+  ext res; ext_id(S, &res);
+  if (n) {
+    aff* bases = (aff*)malloc(n * sizeof(aff)); fe* scalars = (fe*)malloc(n * sizeof(fe));
+    for (size_t i = 0; i < n; i++) { aff_load(S, &bases[i], bases64 + 64 * i); memcpy(scalars[i].v, scalars32 + 32 * i, 32); }
+    msm(S, &res, bases, scalars, n, 256, nthreads < 1 ? 1 : nthreads);
+    free(bases); free(scalars);
+  }
+  aff P; ext_to_aff(S, &P, &res); aff_store(S, out64, &P);
+  return ext_is_id(&res);
 }
 
 /* ---- synthetic workload of SURVEY.md section 8(d), generated with the restated prover ----

@@ -30,6 +30,8 @@ def lib():
         L.orc_thin_verify.argtypes = [C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_char_p, C.c_size_t, C.c_void_p, C.c_void_p]
         L.orc_thin_batch_verify.restype = C.c_int
         L.orc_thin_batch_verify.argtypes = [C.c_int, C.c_size_t] + [C.c_void_p] * 7 + [C.c_int, C.c_void_p] + [C.c_void_p] * 5
+        L.orc_msm.restype = C.c_int
+        L.orc_msm.argtypes = [C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
         L.orc_synth_batch.restype = C.c_int
         L.orc_synth_batch.argtypes = [C.c_int, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int] + [C.c_void_p] * 4
         _LIB = L
@@ -97,6 +99,19 @@ def thin_batch_verify(sid: int, pk, ios, io_off, ad, ad_off, r, s, nthreads=1, t
     if taps:
         t["z"] = t["z"][:nio]
     return st, (float(times[0]), float(times[1])), t
+
+
+def msm(sid: int, bases, scalars, nthreads: int = 1):
+    """sum_i k_i * P_i by the oracle's MSM (the one its batch verifier runs).  bases: (n, 64) canonical affine points,
+    scalars: (n, 32) canonical little-endian integers below 2^256, not reduced mod r.  Returns (sum as 64 canonical
+    bytes, is_identity)."""
+    b = np.ascontiguousarray(np.asarray(bases, dtype=np.uint8).reshape(-1, 64))
+    k = np.ascontiguousarray(np.asarray(scalars, dtype=np.uint8).reshape(-1, 32))
+    assert b.shape[0] == k.shape[0]
+    out = np.zeros(64, np.uint8)
+    rc = lib().orc_msm(sid, b.shape[0], _p(b), _p(k), nthreads, _p(out))
+    assert rc in (0, 1)
+    return out.tobytes(), bool(rc)
 
 
 def synth_batch(sid: int, n: int, m: int = 1, signers: int = 4096, first: int = 0, nthreads: int = 1):

@@ -54,6 +54,45 @@ def oracle_items(pr: "o.Proofs"):
     return [o.batch_prepare(pr.suite, pr.pk[j], pr.ios[j], pr.ad[j], pr.r[j], pr.s[j]) for j in range(len(pr.pk))]
 
 
+def point_order_2k(S, T) -> int:
+    """Order of a point of the 2-power torsion (1, 2, 4, 8 or 16)."""
+    k = 1
+    while T != o.IDENTITY:
+        assert k < 16, "not a small-order point"
+        T, k = o.pt_add(S, T, T), 2 * k
+    return k
+
+
+def torsion_points(S) -> dict:
+    """{order: point} for the affine points of order 2, 4 and 8 the suite has: a curve point outside the prime-order
+    subgroup (x solved from the curve equation at some y) multiplied by r, doubled down to each order.  With `a` a
+    non-square (Bandersnatch) the other points of order 2 lie at infinity and nothing halves (0, -1): only T2 exists."""
+    out = {2: (0, S.p - 1)}
+    if pow(S.a, (S.p - 1) // 2, S.p) != 1:
+        return out
+    want = {d for d in (2, 4, 8) if S.cofactor % d == 0}
+    for y in range(2, 200):
+        P = o.x_from_y(S, y, False)
+        if P is None:
+            continue
+        T = o.pt_mul_raw(S, P, S.r)
+        k = point_order_2k(S, T)
+        while k >= 2:
+            out.setdefault(k, T)
+            T, k = o.pt_add(S, T, T), k // 2
+        if want <= set(out):
+            break
+    return out
+
+
+def msm_py(S, bases, scalars):
+    """sum k_i * P_i by scalar multiplication without any reduction of k_i (pyref.pt_mul_raw)."""
+    acc = o.IDENTITY
+    for P, k in zip(bases, scalars):
+        acc = o.pt_add(S, acc, o.pt_mul_raw(S, P, k))
+    return acc
+
+
 def golden_proofs(S, vectors) -> "o.Proofs":
     pr = o.Proofs(S)
     for v in vectors:

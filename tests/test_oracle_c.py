@@ -4,7 +4,8 @@ import numpy as np
 import pytest
 
 from oracle import corc, pyref as o
-from helpers import GOLDEN_SEEDS, arrays_from_proofs, golden_proofs, oracle_items, pt_bytes, sc_bytes
+from helpers import (GOLDEN_SEEDS, arrays_from_proofs, golden_proofs, msm_py, oracle_items, point_order_2k, pt_bytes,
+                     pt_from_bytes, sc_bytes, torsion_points)
 
 
 @pytest.mark.parametrize("sid", [0, 1, 2])
@@ -67,6 +68,47 @@ def test_c_random_batches(sid, m, n):
     assert corc.thin_verify(sid, pt_bytes(pr.pk[1]), iob, pr.ad[1], r, s) == 0
     pr.ad[n - 1] += b"?"
     assert corc.thin_batch_verify(sid, *arrays_from_proofs(pr), nthreads=2)[0] == 1
+
+
+@pytest.mark.parametrize("sid", [0, 1, 2])
+def test_c_msm_vs_python(sid):
+    """orc_msm (the oracle's signed-digit Pippenger, exported) against sum k_i * P_i by plain double-and-add, before any
+    GPU MSM is compared with it: repeated bases, P with -P, the identity, small-order bases and their sums with
+    subgroup points, scalars 0, r - 1, r, 2^256 - 1 and every 16-bit chunk 0x8000 / 0x7fff (the signed-digit carry edge),
+    none of them reduced mod r."""
+    import random
+    S = o.SUITES[sid]
+    rnd = random.Random(0x5EED + sid)
+    tors = torsion_points(S)
+    assert set(tors) == ({2} if sid == 0 else {2, 4, 8})
+    for k, T in tors.items():
+        assert o.on_curve(S, T) and point_order_2k(S, T) == k
+    sub = [o.pt_mul(S, S.G, rnd.randrange(1, S.r)) for _ in range(4)]
+    mixed = [o.pt_add(S, sub[i % 4], T) for i, T in enumerate(tors.values())]
+    pool = sub + [o.pt_neg(S, sub[0]), o.IDENTITY, S.G] + list(tors.values()) + mixed
+    edge = [0, 1, 2, S.r - 1, S.r, S.r + 1, int("8000" * 16, 16), int("7fff" * 16, 16), (1 << 256) - 1,
+            int("8000" * 15 + "7fff", 16), 1 << 255]
+    cases = [([], []), ([sub[0]], [edge[3]]), ([tors[2]], [edge[8]]), ([o.IDENTITY], [edge[6]]),
+             ([sub[1], sub[1]], [edge[6], edge[7]]), ([sub[2], o.pt_neg(S, sub[2])], [edge[8], edge[8]]),
+             ([mixed[-1], tors[max(tors)]], [S.r, edge[9]])]
+    for P in pool:                                      # every base alone under every edge scalar
+        cases += [([P] * len(edge), edge)]
+    for _ in range(4):                                  # n = 37: everything at once
+        bases = [rnd.choice(pool) for _ in range(37)]
+        scalars = [rnd.choice(edge) if rnd.random() < 0.5 else rnd.getrandbits(256) for _ in range(37)]
+        cases.append((bases, scalars))
+    for j, (bases, scalars) in enumerate(cases):
+        want = msm_py(S, bases, scalars)
+        b = np.frombuffer(b"".join(pt_bytes(P) for P in bases), np.uint8)
+        k = np.frombuffer(b"".join(sc_bytes(x) for x in scalars), np.uint8)
+        for threads in (1, 4):
+            got, ident = corc.msm(sid, b, k, nthreads=threads)
+            assert pt_from_bytes(got) == want, (j, threads)
+            assert ident == (want == o.IDENTITY)
+    # the small-order component follows the integer scalar, not its residue mod r
+    T = tors[max(tors)]
+    assert corc.msm(sid, np.frombuffer(pt_bytes(T), np.uint8), np.frombuffer(sc_bytes(S.r), np.uint8))[1] is False
+    assert corc.msm(sid, np.frombuffer(pt_bytes(T), np.uint8), np.frombuffer(sc_bytes(S.r * max(tors)), np.uint8))[1]
 
 
 def test_c_ragged_batch():
