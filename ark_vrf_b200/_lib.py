@@ -118,6 +118,10 @@ SIGNATURES = {
     "avrf_server_free": (None, [C.c_void_p]),
     "avrf_server_submit": (C.c_int64, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 7),
     "avrf_server_wait": (C.c_int, [C.c_void_p, C.c_int64, i32p]),
+    "avrf_pedersen_server_new": (C.c_void_p, [C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
+    "avrf_pedersen_server_submit": (C.c_int64, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
+    "avrf_server_submit_compressed": (C.c_int64, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
+    "avrf_pedersen_server_submit_compressed": (C.c_int64, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 7),
     "avrf_mb_sha512": (C.c_int, [C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, i32p]),
     "avrf_microbench": (C.c_int, [C.c_uint32, C.c_uint32, C.POINTER(C.c_double), C.POINTER(C.c_float)]),
 }

@@ -64,6 +64,9 @@ struct avrf_batch {
   // inputs on the device
   DevBuf pk, r, s, ios, io_off, ad_off, ad;
   DevBuf ok, sb;                        // Pedersen only (pk holds the key commitments)
+  // decode buffers of the wire-format pushes (feed_api.inl, WireChunk): allocated by the first such push, so that
+  // pushes on different handles hold no lock shared with other handles or the handle-less entry points
+  DevBuf w_in, w_y, w_den, w_scr, w_fl, w_out, w_ok, w_sc, w_po, w_off, w_rec;
   // single-push staging on the host: pinned double buffer (eager handles), plain vectors otherwise
   PushStage stage[2];
   int cur = 0;
@@ -444,7 +447,8 @@ void avrf_thin_batch_free(avrf_batch* b) {
   DevBuf* bufs[] = {&b->ios, &b->io_off, &b->ad_off, &b->ad, &b->pts, &b->cs, &b->z, &b->renc,
                     &b->dig_w, &b->rank_w, &b->digits, &b->hist, &b->cursor, &b->offs, &b->toff, &b->btot, &b->totals, &b->entries, &b->tasks,
                     &b->task_out, &b->chunk_out, &b->wsum, &b->partial, &b->gpart, &b->flags, &b->w_tap, &b->scalars_tap,
-                    &b->segs_dev};
+                    &b->segs_dev, &b->w_in, &b->w_y, &b->w_den, &b->w_scr, &b->w_fl, &b->w_out, &b->w_ok, &b->w_sc,
+                    &b->w_po, &b->w_off, &b->w_rec};
   for (DevBuf* d : bufs) d->release();
   for (auto& e : b->ev) if (e) cudaEventDestroy(e);
   for (auto& e : b->prep_ev) cudaEventDestroy(e);

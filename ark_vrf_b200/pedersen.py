@@ -6,6 +6,7 @@ Mirror of `ark_vrf::pedersen` (reference src/pedersen.rs):
     BatchVerifier::{new, push, push_prepared, verify}   BatchVerifier  (pedersen.rs:322-427; the MSM has 5N+2 points)
     (wire-format proofs)             BatchVerifier.push_compressed(), serialize_proofs()  (Proof::{de,}serialize_compressed)
     (per-proof verdicts)             BatchVerifier.verify_each() / find_invalid()
+    (throughput mode)                BatchServer: whole batches on a native worker pool, decoded or in wire format
 A proof is `(pk_com, r, ok, s, sb)` (pedersen.rs:43-50)."""
 from __future__ import annotations
 
@@ -19,7 +20,7 @@ from . import _lib
 from .ops import pedersen_prove_many as prove_many          # noqa: F401  (re-exported: pedersen.prove_many)
 from .ops import point_compress
 from .synth import ORDER
-from .thin import Format, Suite, Tap, _bytes_of, _ios_bytes, _raise_for_status, ptr
+from .thin import Format, Suite, Tap, _ServerBase, _bytes_of, _ios_bytes, _raise_for_status, ptr
 
 
 @dataclass
@@ -129,6 +130,31 @@ class BatchVerifier:
             self.close()
         except Exception:
             pass
+
+
+class BatchServer(_ServerBase):
+    """Throughput mode for the Pedersen VRF: a native pool of worker threads, one Pedersen `BatchVerifier` handle each
+    (include/avrf.h, "Batch server").  `submit` / `submit_compressed` enqueue a whole batch (new + push + verify) and
+    return a ticket; `wait` returns its status code, `wait_compressed` the status and the decode flags of a wire-format
+    job.  Pool shapes as `thin.BatchServer`.  The arrays of a submitted batch are kept alive (and must not be modified)
+    until its `wait` returns."""
+
+    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL, workers: int = 4,
+                 hashers: int = 0, own_hash_workers: int = 0):
+        self._start(_lib.load().avrf_pedersen_server_new, suite, fmt, workers, hashers, own_hash_workers)
+
+    def submit(self, ios, io_offsets, ad_blob, ad_offsets, pk_com, r, ok, s, sb) -> int:
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        return self._submit(self._lib.avrf_pedersen_server_submit, (ios, io_offsets, ad_blob, ad_offsets, pk_com, r, ok, s, sb),
+                            n, False)
+
+    def submit_compressed(self, ios32, io_offsets, ad_blob, ad_offsets, proofs) -> int:
+        """A job of proofs in wire format, arguments as `BatchVerifier.push_compressed`."""
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        return self._submit(self._lib.avrf_pedersen_server_submit_compressed, (ios32, io_offsets, ad_blob, ad_offsets, proofs),
+                            n, True)
 
 
 def verify(suite: Union[Suite, int], ios, ad, proof: Proof, fmt: Union[Format, int] = Format.CANONICAL) -> None:

@@ -51,6 +51,19 @@ extern "C" {
         ad_blob: *const u8, ad_offsets: *const u32, r: *const u8, s: *const u8,
     ) -> i64;
     fn avrf_server_wait(sv: *mut AvrfServer, ticket: i64, status: *mut i32) -> i32;
+    fn avrf_server_submit_compressed(
+        sv: *mut AvrfServer, n: u64, pk32: *const u8, ios32: *const u8, io_offsets: *const u32,
+        ad_blob: *const u8, ad_offsets: *const u32, r32: *const u8, s: *const u8, ok: *mut u8, n_bad: *mut u64,
+    ) -> i64;
+    fn avrf_pedersen_server_new(suite: u32, fmt: u32, n_workers: u32, n_hashers: u32, n_own: u32) -> *mut AvrfServer;
+    fn avrf_pedersen_server_submit(
+        sv: *mut AvrfServer, n: u64, ios: *const u8, io_offsets: *const u32, ad_blob: *const u8,
+        ad_offsets: *const u32, pk_com: *const u8, r: *const u8, ok: *const u8, s: *const u8, sb: *const u8,
+    ) -> i64;
+    fn avrf_pedersen_server_submit_compressed(
+        sv: *mut AvrfServer, n: u64, ios32: *const u8, io_offsets: *const u32, ad_blob: *const u8,
+        ad_offsets: *const u32, proofs: *const u8, ok: *mut u8, n_bad: *mut u64,
+    ) -> i64;
     fn avrf_thin_verify_one(
         suite: u32, fmt: u32, pk: *const u8, ios: *const u8, n_ios: u32, ad: *const u8, ad_len: u32,
         r: *const u8, s: *const u8, status: *mut i32,
@@ -355,6 +368,65 @@ impl<S: GpuSuite> BatchServer<S> {
         assert!(id >= 0, "libavrf_gpu system error {id}");
         Ticket { id, server: self, _batch: PhantomData }
     }
+
+    /// A batch of proofs in wire format, the arrays of `BatchVerifier::push_compressed`: decoded and validated on the
+    /// GPU by the worker.
+    pub fn submit_compressed<'a>(
+        &'a self, pk32: &'a [[u8; 32]], ios32: &'a [[u8; 64]], io_offsets: &'a [u32], ad_blob: &'a [u8],
+        ad_offsets: &'a [u32], r32: &'a [[u8; 32]], s: &'a [[u8; 32]],
+    ) -> WireTicket<'a> {
+        let n = pk32.len();
+        assert!(r32.len() == n && s.len() == n && io_offsets.len() == n + 1 && ad_offsets.len() == n + 1);
+        let mut t = WireTicket::new(self.h, n);
+        t.id = unsafe {
+            avrf_server_submit_compressed(
+                self.h, n as u64, pk32.as_ptr() as *const u8, ios32.as_ptr() as *const u8, io_offsets.as_ptr(),
+                ad_blob.as_ptr(), ad_offsets.as_ptr(), r32.as_ptr() as *const u8, s.as_ptr() as *const u8,
+                t.ok.as_mut_ptr(), &mut *t.n_bad,
+            )
+        };
+        assert!(t.id >= 0, "libavrf_gpu system error {}", t.id);
+        t
+    }
+}
+
+/// A submitted wire-format batch of either scheme: keeps its arrays borrowed and owns the per-proof decode flags the
+/// worker fills in.  Dropping it without `wait` still waits, so the worker never writes into freed memory.
+pub struct WireTicket<'a> {
+    id: i64,
+    server: *mut AvrfServer,
+    ok: Box<[u8]>,
+    n_bad: Box<u64>,
+    _borrow: PhantomData<&'a [u8]>,
+}
+
+impl<'a> WireTicket<'a> {
+    fn new(server: *mut AvrfServer, n: usize) -> Self {
+        Self { id: -1, server, ok: vec![0u8; n.max(1)].into_boxed_slice(), n_bad: Box::new(0), _borrow: PhantomData }
+    }
+
+    /// Blocks for the verdict and the indices of the proofs that did not deserialize.  When that list is not empty
+    /// nothing was verified and the verdict is `Err(Error::InvalidData)`.
+    pub fn wait(mut self) -> (Result<(), Error>, Vec<usize>) {
+        let mut status = -1i32;
+        let rc = unsafe { avrf_server_wait(self.server, self.id, &mut status) };
+        self.id = -1;
+        let bad = if *self.n_bad > 0 {
+            self.ok.iter().enumerate().filter(|(_, &f)| f == 0).map(|(j, _)| j).collect()
+        } else {
+            Vec::new()
+        };
+        (status_to_result(rc, status), bad)
+    }
+}
+
+impl<'a> Drop for WireTicket<'a> {
+    fn drop(&mut self) {
+        if self.id >= 0 {
+            let mut status = -1i32;
+            unsafe { avrf_server_wait(self.server, self.id, &mut status) };
+        }
+    }
 }
 
 impl<'a, S: GpuSuite> Ticket<'a, S> {
@@ -527,4 +599,119 @@ pub mod pedersen {
         }
     }
     unsafe impl<S: GpuSuite + PedersenSuite> Send for BatchVerifier<S> {}
+
+    /// The flattened argument list of a whole Pedersen verification, for `BatchServer::submit`.  The proof fields are
+    /// kept as their arkworks memory images (`layout_self_check`).
+    pub struct Batch<S: GpuSuite + PedersenSuite> {
+        pk_com: Vec<[u8; 64]>,
+        r: Vec<[u8; 64]>,
+        ok: Vec<[u8; 64]>,
+        s: Vec<[u8; 32]>,
+        sb: Vec<[u8; 32]>,
+        ios: Vec<VrfIo<S>>,
+        io_offsets: Vec<u32>,
+        ad: Vec<u8>,
+        ad_offsets: Vec<u32>,
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Default for Batch<S> {
+        fn default() -> Self {
+            Self {
+                pk_com: vec![], r: vec![], ok: vec![], s: vec![], sb: vec![], ios: vec![], io_offsets: vec![0], ad: vec![],
+                ad_offsets: vec![0],
+            }
+        }
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Batch<S> {
+        pub fn push(&mut self, ios: impl AsRef<[VrfIo<S>]>, ad: impl AsRef<[u8]>, proof: &Proof<S>) {
+            let pt = |p: &AffinePoint<S>| unsafe { *(point_bytes::<S>(p) as *const [u8; 64]) };
+            let sc = |x: &ScalarField<S>| unsafe { *(scalar_bytes::<S>(x) as *const [u8; 32]) };
+            self.pk_com.push(pt(&proof.pk_com));
+            self.r.push(pt(&proof.r));
+            self.ok.push(pt(&proof.ok));
+            self.s.push(sc(&proof.s));
+            self.sb.push(sc(&proof.sb));
+            self.ios.extend_from_slice(ios.as_ref());
+            self.ad.extend_from_slice(ad.as_ref());
+            self.io_offsets.push(self.ios.len() as u32);
+            self.ad_offsets.push(self.ad.len() as u32);
+        }
+    }
+
+    /// Throughput mode for the Pedersen VRF: the worker pool of `gpu::BatchServer`, one Pedersen batch verifier per
+    /// worker (`avrf_pedersen_server_new`).  Every submitted batch gets the verdict `pedersen::BatchVerifier::verify`
+    /// would return for it.
+    pub struct BatchServer<S: GpuSuite + PedersenSuite> {
+        h: *mut AvrfServer,
+        _s: PhantomData<S>,
+    }
+
+    /// A submitted batch; keeps the batch borrowed until the verdict has been read.
+    pub struct Ticket<'a, S: GpuSuite + PedersenSuite> {
+        id: i64,
+        server: &'a BatchServer<S>,
+        _batch: PhantomData<&'a Batch<S>>,
+    }
+
+    impl<S: GpuSuite + PedersenSuite> BatchServer<S> {
+        /// `hashers` > 0: shared multi-buffer SHA-512 threads; `own_hash_workers` of the workers keep a core each.
+        pub fn new(workers: u32, hashers: u32, own_hash_workers: u32) -> Self {
+            let h = unsafe {
+                avrf_init(0);
+                avrf_pedersen_server_new(S::AVRF_SUITE, AVRF_FMT_MONTGOMERY, workers, hashers, own_hash_workers)
+            };
+            assert!(!h.is_null(), "avrf_pedersen_server_new failed (no CUDA device?)");
+            static CHECKED: std::sync::Once = std::sync::Once::new();
+            CHECKED.call_once(layout_self_check::<S>);
+            Self { h, _s: PhantomData }
+        }
+
+        pub fn submit<'a>(&'a self, b: &'a Batch<S>) -> Ticket<'a, S> {
+            let id = unsafe {
+                avrf_pedersen_server_submit(
+                    self.h, b.pk_com.len() as u64, b.ios.as_ptr() as *const u8, b.io_offsets.as_ptr(), b.ad.as_ptr(),
+                    b.ad_offsets.as_ptr(), b.pk_com.as_ptr() as *const u8, b.r.as_ptr() as *const u8,
+                    b.ok.as_ptr() as *const u8, b.s.as_ptr() as *const u8, b.sb.as_ptr() as *const u8,
+                )
+            };
+            assert!(id >= 0, "libavrf_gpu system error {id}");
+            Ticket { id, server: self, _batch: PhantomData }
+        }
+
+        /// A batch in wire format, the arrays of `BatchVerifier::push_compressed`.
+        pub fn submit_compressed<'a>(
+            &'a self, ios32: &'a [[u8; 64]], io_offsets: &'a [u32], ad_blob: &'a [u8], ad_offsets: &'a [u32],
+            proofs: &'a [[u8; 160]],
+        ) -> WireTicket<'a> {
+            let n = proofs.len();
+            assert!(io_offsets.len() == n + 1 && ad_offsets.len() == n + 1);
+            let mut t = WireTicket::new(self.h, n);
+            t.id = unsafe {
+                avrf_pedersen_server_submit_compressed(
+                    self.h, n as u64, ios32.as_ptr() as *const u8, io_offsets.as_ptr(), ad_blob.as_ptr(),
+                    ad_offsets.as_ptr(), proofs.as_ptr() as *const u8, t.ok.as_mut_ptr(), &mut *t.n_bad,
+                )
+            };
+            assert!(t.id >= 0, "libavrf_gpu system error {}", t.id);
+            t
+        }
+    }
+
+    impl<'a, S: GpuSuite + PedersenSuite> Ticket<'a, S> {
+        /// Blocks for the verdict.
+        pub fn wait(self) -> Result<(), Error> {
+            let mut status = -1i32;
+            let rc = unsafe { avrf_server_wait(self.server.h, self.id, &mut status) };
+            status_to_result(rc, status)
+        }
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Drop for BatchServer<S> {
+        fn drop(&mut self) {
+            unsafe { avrf_server_free(self.h) } // finishes queued batches, joins the workers
+        }
+    }
+    unsafe impl<S: GpuSuite + PedersenSuite> Send for BatchServer<S> {}
+    unsafe impl<S: GpuSuite + PedersenSuite> Sync for BatchServer<S> {}
 }

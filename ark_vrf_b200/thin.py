@@ -404,32 +404,29 @@ class ShardedBatchVerifier:
             pass
 
 
-class BatchServer:
-    """Throughput mode: a native pool of worker threads, one `BatchVerifier` handle each (include/avrf.h,
-    "Batch server").  `submit` enqueues a whole batch and returns a ticket; `wait` returns its status code.
-    The arrays of a submitted batch are kept alive (and must not be modified) until its `wait` returns."""
+class _ServerBase:
+    """What the batch servers of both schemes share (include/avrf.h, "Batch server"): tickets, waits and the lifetime
+    of borrowed arrays.  The arrays of a submitted batch (and the decode flags a wire-format submit allocates) are kept
+    alive, and must not be modified, until its `wait` returns."""
 
-    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL, workers: int = 4,
-                 hashers: int = 0, own_hash_workers: int = 0):
-        """`hashers` > 0: that many shared multi-buffer SHA-512 threads (eight batches' hash chains per thread)
-        instead of one hashing core per worker - for boxes with fewer free cores than batches in flight.
-        `own_hash_workers`: that many of the workers keep hashing on their own thread (mixed pool)."""
+    def _start(self, new, suite, fmt, workers: int, hashers: int, own_hash_workers: int) -> None:
         self._lib = _lib.load()
         self.suite, self.fmt, self.workers, self.hashers = Suite(suite), Format(fmt), int(workers), int(hashers)
-        self._h = self._lib.avrf_server_new_mixed(int(self.suite), int(self.fmt), self.workers, self.hashers, int(own_hash_workers))
+        self._h = new(int(self.suite), int(self.fmt), self.workers, self.hashers, int(own_hash_workers))
         if not self._h:
             msg = self._lib.avrf_last_error()
-            raise _lib.AvrfError(msg.decode() if msg else "avrf_server_new failed")
+            raise _lib.AvrfError(msg.decode() if msg else "batch server: creation failed")
         self._live = {}
+        self._dec_ok = {}                    # ticket -> decode flags of a wire-format job
 
-    def submit(self, pk, ios, io_offsets, ad_blob, ad_offsets, r, s) -> int:
-        n = len(io_offsets) - 1
-        assert len(ad_offsets) == n + 1
-        arrays = (pk, ios, io_offsets, ad_blob, ad_offsets, r, s)
-        t = int(self._lib.avrf_server_submit(self._h, n, *[ptr(a) for a in arrays]))
+    def _submit(self, fn, arrays, n: int, wire: bool) -> int:
+        ok = np.zeros(max(n, 1), dtype=np.uint8) if wire else None
+        t = int(fn(self._h, n, *[ptr(a) for a in arrays], *((ptr(ok), None) if wire else ())))
         if t < 0:
             _lib.check(t)
-        self._live[t] = arrays
+        self._live[t] = (arrays, ok)
+        if wire:
+            self._dec_ok[t] = ok[:n]
         return t
 
     def wait(self, ticket: int) -> int:
@@ -440,6 +437,15 @@ class BatchServer:
             self._live.pop(ticket, None)
         return st.value
 
+    def wait_compressed(self, ticket: int) -> Tuple[int, np.ndarray]:
+        """`wait` for a wire-format job: (status, per-proof decode flags).  When a flag is False the job's proofs did
+        not all decode, nothing was verified and the status is InvalidData."""
+        if ticket in self._live and ticket not in self._dec_ok:
+            raise ValueError(f"ticket {ticket} is not a wire-format job")
+        ok = self._dec_ok.pop(ticket, None)
+        status = self.wait(ticket)
+        return status, ok.astype(bool)
+
     def verify(self, ticket: int) -> None:
         """`wait`, mapped onto the reference's `Result<(), Error>`."""
         _raise_for_status(self.wait(ticket))
@@ -449,12 +455,39 @@ class BatchServer:
             self._lib.avrf_server_free(self._h)       # finishes queued batches first
             self._h = None
             self._live.clear()
+            self._dec_ok.clear()
 
     def __del__(self):
         try:
             self.close()
         except Exception:
             pass
+
+
+class BatchServer(_ServerBase):
+    """Throughput mode: a native pool of worker threads, one `BatchVerifier` handle each (include/avrf.h,
+    "Batch server").  `submit` enqueues a whole batch and returns a ticket; `wait` returns its status code.
+    The arrays of a submitted batch are kept alive (and must not be modified) until its `wait` returns."""
+
+    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL, workers: int = 4,
+                 hashers: int = 0, own_hash_workers: int = 0):
+        """`hashers` > 0: that many shared multi-buffer SHA-512 threads (eight batches' hash chains per thread)
+        instead of one hashing core per worker - for boxes with fewer free cores than batches in flight.
+        `own_hash_workers`: that many of the workers keep hashing on their own thread (mixed pool)."""
+        self._start(_lib.load().avrf_server_new_mixed, suite, fmt, workers, hashers, own_hash_workers)
+
+    def submit(self, pk, ios, io_offsets, ad_blob, ad_offsets, r, s) -> int:
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        return self._submit(self._lib.avrf_server_submit, (pk, ios, io_offsets, ad_blob, ad_offsets, r, s), n, False)
+
+    def submit_compressed(self, pk32, ios32, io_offsets, ad_blob, ad_offsets, r32, s) -> int:
+        """A job of proofs in wire format, arguments as `BatchVerifier.push_compressed`; `wait_compressed` returns its
+        status and decode flags."""
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        return self._submit(self._lib.avrf_server_submit_compressed, (pk32, ios32, io_offsets, ad_blob, ad_offsets, r32, s),
+                            n, True)
 
 
 def seed_of_stream(suite: Union[Suite, int], cs_stream) -> bytes:

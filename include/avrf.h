@@ -152,7 +152,11 @@ int avrf_thin_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* pk, cons
  * rejected for pk / I / O, allowed for R) and enter the push pipeline without a round trip: 160 instead of 296 bytes
  * per proof cross PCIe at M = 1.  All or nothing, as in the reference where a proof that fails to deserialize never
  * reaches push: when any proof does not decode, *n_bad is their number, ok[j] (optional, n bytes) is 0 for them, and
- * NOTHING is pushed.  Works with handles of either format. */
+ * NOTHING is pushed.  Works with handles of either format.
+ * The decode buffers belong to the handle (no lock shared with other handles or the handle-less entry points, so wire
+ * pushes on different handles overlap): the first wire push allocates about 226 bytes per compressed point of one
+ * 75776-proof chunk - about 70 MB for a Thin handle and 100 MB for a Pedersen handle at one I/O pair per proof (device
+ * allocations round up to at most twice that) - kept until the handle is freed. */
 int avrf_thin_batch_push_compressed(avrf_batch* b, uint64_t n, const uint8_t* pk32, const uint8_t* ios32,
                                     const uint32_t* io_offsets, const uint8_t* ad_blob, const uint32_t* ad_offsets,
                                     const uint8_t* r32, const uint8_t* s, uint8_t* ok, uint64_t* n_bad);
@@ -381,6 +385,29 @@ int64_t avrf_server_submit(avrf_server* sv, uint64_t n, const uint8_t* pk, const
                            const uint32_t* io_offsets, const uint8_t* ad_blob, const uint32_t* ad_offsets,
                            const uint8_t* r, const uint8_t* s);
 int avrf_server_wait(avrf_server* sv, int64_t ticket, int32_t* status);
+
+/* A Pedersen batch server: the same pool, hashers and own-thread split as avrf_server_new_mixed; every worker owns a
+ * Pedersen handle (avrf_pedersen_batch_new).  avrf_server_wait / avrf_server_free serve both kinds of server.  A job
+ * must match the server's scheme: a Thin submit (avrf_server_submit, avrf_server_submit_compressed) on a Pedersen
+ * server, or a Pedersen submit on a Thin server, is AVRF_ERR_ARG and issues no ticket. */
+avrf_server* avrf_pedersen_server_new(uint32_t suite, uint32_t fmt, uint32_t n_workers, uint32_t n_hashers, uint32_t n_own);
+/* pedersen::BatchVerifier new + push of n proofs + verify as one job; arguments as avrf_pedersen_batch_push_many.  The
+ * verdict is the one a fresh handle gives for the same arrays (AVRF_INVALID_DATA for an identity pk_com or I/O point). */
+int64_t avrf_pedersen_server_submit(avrf_server* sv, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
+                                    const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,
+                                    const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);
+/* Jobs of proofs in WIRE format: arguments exactly as avrf_thin_batch_push_compressed /
+ * avrf_pedersen_batch_push_compressed.  ok (n bytes) and n_bad are optional and, like the inputs, BORROWED until
+ * avrf_server_wait returns for the ticket; the worker fills them as the push would.  When any proof does not decode,
+ * nothing is verified: avrf_server_wait returns 0 with *status = AVRF_INVALID_DATA, *n_bad > 0 and ok[j] = 0 for the
+ * offending proofs (n_bad tells "did not deserialise" apart from "identity point"). */
+int64_t avrf_server_submit_compressed(avrf_server* sv, uint64_t n, const uint8_t* pk32, const uint8_t* ios32,
+                                      const uint32_t* io_offsets, const uint8_t* ad_blob, const uint32_t* ad_offsets,
+                                      const uint8_t* r32, const uint8_t* s, uint8_t* ok, uint64_t* n_bad);
+int64_t avrf_pedersen_server_submit_compressed(avrf_server* sv, uint64_t n, const uint8_t* ios32,
+                                               const uint32_t* io_offsets, const uint8_t* ad_blob,
+                                               const uint32_t* ad_offsets, const uint8_t* proofs, uint8_t* ok,
+                                               uint64_t* n_bad);
 
 /* Host-only utility: SHA-512 of n_streams independent byte streams through the batch server's multi-buffer hasher,
  * fed in interleaved chunk-byte updates; digests = 64 bytes per stream.  *simd (optional) = 1 if the AVX-512 path ran.

@@ -5,12 +5,13 @@
 //   thin::BatchItem<S>                            src/thin.rs:172-179
 //   thin::BatchVerifier<S>::{new_, prepare, push_prepared, push, verify}   src/thin.rs:198-326
 //   Public<S>::verify  (thin::Verifier)           src/thin.rs:95-109,131-165
-//   thin::BatchServer<S>::{submit, wait}          (new: worker pool over avrf_server_*, throughput mode)
+//   thin::BatchServer<S>::{submit, submit_compressed, wait}   (new: worker pool over avrf_server_*, throughput mode)
 //   thin::ShardedBatchVerifier<S>                 (new: one batch over several GPUs of this process, avrf_thin_sharded_*)
 //   pedersen::Proof{pk_com, r, ok, s, sb}         src/pedersen.rs:43-50
 //   pedersen::verify (pedersen::Verifier)         src/pedersen.rs:188-253
 //   pedersen::BatchVerifier<S>::{push, push_compressed, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
 //   pedersen::prove_many (Prover::prove, n proofs) src/pedersen.rs:136-186
+//   pedersen::BatchServer<S>::{submit, submit_compressed, wait}   (new: the same worker pool for Pedersen batches)
 //   Error::{VerificationFailure, InvalidData}     src/lib.rs:136-147
 //
 // The host toolchain of the reference (Rust) is absent from the build image, so this header is the
@@ -174,6 +175,16 @@ class BatchServer {
     if (t < 0) check((int)t);
     return t;
   }
+  // A batch of proofs in wire format, arguments as BatchVerifier::push_compressed.  The arrays, `ok` (n bytes) and
+  // `n_bad` (both optional) are borrowed until wait() returns for the ticket; a proof that does not decode makes the
+  // verdict InvalidData with *n_bad > 0 and ok[j] == 0 naming it.
+  int64_t submit_compressed(uint64_t n, const uint8_t* pk32, const uint8_t* ios32, const uint32_t* io_offsets,
+                            const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* r32, const uint8_t* s,
+                            uint8_t* ok = nullptr, uint64_t* n_bad = nullptr) {
+    int64_t t = avrf_server_submit_compressed(h_, n, pk32, ios32, io_offsets, ad_blob, ad_offsets, r32, s, ok, n_bad);
+    if (t < 0) check((int)t);
+    return t;
+  }
   Result wait(int64_t ticket) {
     int32_t st = -1;
     check(avrf_server_wait(h_, ticket, &st));
@@ -250,6 +261,65 @@ class BatchVerifier {
 
  private:
   avrf_batch* h_;
+};
+
+// The flattened argument list of a whole Pedersen verification, for BatchServer::submit (borrowed until wait).
+struct Batch {
+  std::vector<AffinePoint> pk_com, r, ok;
+  std::vector<ScalarField> s, sb;
+  std::vector<VrfIo> ios;
+  std::vector<uint32_t> io_offsets{0}, ad_offsets{0};
+  std::vector<uint8_t> ad;
+  void push(const std::vector<VrfIo>& ios_, const std::vector<uint8_t>& ad_, const Proof& proof) {
+    pk_com.push_back(proof.pk_com); r.push_back(proof.r); ok.push_back(proof.ok);
+    s.push_back(proof.s); sb.push_back(proof.sb);
+    ios.insert(ios.end(), ios_.begin(), ios_.end());
+    ad.insert(ad.end(), ad_.begin(), ad_.end());
+    io_offsets.push_back((uint32_t)ios.size());
+    ad_offsets.push_back((uint32_t)ad.size());
+  }
+  size_t len() const { return pk_com.size(); }
+};
+
+// Throughput mode for Pedersen batches: the worker pool of thin::BatchServer, one pedersen::BatchVerifier handle per
+// worker (avrf_pedersen_server_new).
+template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
+class BatchServer {
+ public:
+  // hashers > 0: shared multi-buffer SHA-512 threads; own_hash_workers of the workers keep a core each (mixed pool)
+  explicit BatchServer(uint32_t workers, uint32_t hashers = 0, uint32_t own_hash_workers = 0)
+      : h_(avrf_pedersen_server_new(S::ID, FMT, workers, hashers, own_hash_workers)) {
+    if (!h_) throw std::runtime_error(avrf_last_error());
+  }
+  ~BatchServer() { avrf_server_free(h_); }
+  BatchServer(const BatchServer&) = delete;
+  BatchServer& operator=(const BatchServer&) = delete;
+  int64_t submit(const Batch& b) {
+    const bool any = b.len() != 0;
+    int64_t t = avrf_pedersen_server_submit(h_, b.len(), b.ios.empty() ? nullptr : b.ios[0].input.data(), b.io_offsets.data(),
+                                            b.ad.empty() ? nullptr : b.ad.data(), b.ad_offsets.data(),
+                                            any ? b.pk_com[0].data() : nullptr, any ? b.r[0].data() : nullptr,
+                                            any ? b.ok[0].data() : nullptr, any ? b.s[0].data() : nullptr,
+                                            any ? b.sb[0].data() : nullptr);
+    if (t < 0) check((int)t);
+    return t;
+  }
+  // A batch in wire format, arguments as BatchVerifier::push_compressed; `ok` / `n_bad` as thin::BatchServer's.
+  int64_t submit_compressed(uint64_t n, const uint8_t* ios32, const uint32_t* io_offsets, const uint8_t* ad_blob,
+                            const uint32_t* ad_offsets, const uint8_t* proofs, uint8_t* ok = nullptr,
+                            uint64_t* n_bad = nullptr) {
+    int64_t t = avrf_pedersen_server_submit_compressed(h_, n, ios32, io_offsets, ad_blob, ad_offsets, proofs, ok, n_bad);
+    if (t < 0) check((int)t);
+    return t;
+  }
+  Result wait(int64_t ticket) {
+    int32_t st = -1;
+    check(avrf_server_wait(h_, ticket, &st));
+    return Result{st};
+  }
+
+ private:
+  avrf_server* h_;
 };
 
 struct Proven { std::vector<Proof> proofs; std::vector<ScalarField> blinding; };
