@@ -40,10 +40,11 @@ constexpr size_t PREP_CHUNK = 148 * 4 * 128;
 // SHA-512) remains to be hashed when the caller's push loop ends and verify is called
 constexpr size_t STAGE_CHUNK = PREP_CHUNK / 2;
 
-// Pinned SoA staging of single pushes (avrf_thin_batch_push): filled by the caller's thread, shipped to the
-// device one PREP_CHUNK at a time while the other buffer fills.
+// Pinned SoA staging of single pushes (avrf_thin_batch_push, avrf_pedersen_batch_push): one buffer per input column of
+// the handle's scheme (Scheme::col), filled by the caller's thread, shipped to the device one chunk at a time while the
+// other buffer fills.
 struct PushStage {
-  PinBuf pk, r, s, ios, ad, io_off, ad_off;
+  PinBuf col[5], ios, ad, io_off, ad_off;
   size_t n = 0, nio = 0, nad = 0, cap_io = 0, cap_ad = 0;
   cudaEvent_t free_ev = nullptr;        // recorded once the device has consumed the buffer
   bool inflight = false;
@@ -70,7 +71,7 @@ struct avrf_batch {
   // single-push staging on the host: pinned double buffer (eager handles), plain vectors otherwise
   PushStage stage[2];
   int cur = 0;
-  std::vector<uint8_t> h_pk, h_r, h_s, h_ios, h_ad;
+  std::vector<uint8_t> h_col[5], h_ios, h_ad;   // h_col: one vector per input column of the scheme (Scheme::col)
   std::vector<uint32_t> h_io_off{0}, h_ad_off{0};
   // derived
   DevBuf dig_w, rank_w;                 // window-major copies of the digits / ranks (k_sort_transpose)
@@ -473,7 +474,8 @@ int avrf_thin_batch_clear(avrf_batch* b) {
   b->prep_ev_chunks = 0;
   b->segs.clear();
   b->segs_dirty = true;
-  b->h_pk.clear(); b->h_r.clear(); b->h_s.clear(); b->h_ios.clear(); b->h_ad.clear();
+  for (auto& v : b->h_col) v.clear();
+  b->h_ios.clear(); b->h_ad.clear();
   b->h_io_off.assign(1, 0);
   b->h_ad_off.assign(1, 0);
   return 0;
@@ -733,11 +735,11 @@ static int push_many_impl(avrf_batch* b, uint64_t n, const Columns& cols, const 
   return 0;
 }
 
-static int stage_reserve(PushStage& sg, size_t cap_io, size_t cap_ad) {
+static int stage_reserve(const Scheme& sc, PushStage& sg, size_t cap_io, size_t cap_ad) {
   int rc;
-  if ((rc = sg.pk.reserve(64 * PREP_CHUNK)) || (rc = sg.r.reserve(64 * PREP_CHUNK)) || (rc = sg.s.reserve(32 * PREP_CHUNK)) ||
-      (rc = sg.io_off.reserve(4 * (PREP_CHUNK + 1))) || (rc = sg.ad_off.reserve(4 * (PREP_CHUNK + 1))))
-    return rc;
+  for (uint32_t k = 0; k < sc.ncol; k++)
+    if ((rc = sg.col[k].reserve(sc.col[k].bytes * PREP_CHUNK))) return rc;
+  if ((rc = sg.io_off.reserve(4 * (PREP_CHUNK + 1))) || (rc = sg.ad_off.reserve(4 * (PREP_CHUNK + 1)))) return rc;
   if (cap_io > sg.cap_io) { if ((rc = sg.ios.reserve(128 * cap_io, 128 * sg.nio))) return rc; sg.cap_io = cap_io; }
   if (cap_ad > sg.cap_ad) { if ((rc = sg.ad.reserve(cap_ad, sg.nad))) return rc; sg.cap_ad = cap_ad; }
   if (!sg.free_ev) CK(cudaEventCreateWithFlags(&sg.free_ev, cudaEventDisableTiming));
@@ -751,7 +753,10 @@ static int flush_stage(avrf_batch* b) {
   if (sg.n == 0) return 0;
   { int rc0 = bind_device(b->device); if (rc0) return rc0; }
   stage_fence();
-  int rc = push_many_impl(b, sg.n, {sg.pk.as<uint8_t>(), sg.r.as<uint8_t>(), sg.s.as<uint8_t>()}, sg.ios.as<uint8_t>(), sg.io_off.as<uint32_t>(), sg.ad.as<uint8_t>(),
+  const Scheme& sc = scheme_of(b);
+  Columns cols{};
+  for (uint32_t k = 0; k < sc.ncol; k++) cols[k] = sg.col[k].as<uint8_t>();
+  int rc = push_many_impl(b, sg.n, cols, sg.ios.as<uint8_t>(), sg.io_off.as<uint32_t>(), sg.ad.as<uint8_t>(),
                           sg.ad_off.as<uint32_t>(), sg.free_ev, sg.n == STAGE_CHUNK ? 4 : 0);
   if (rc) return rc;
   sg.n = sg.nio = sg.nad = 0;
@@ -767,25 +772,29 @@ static int flush_pending(avrf_batch* b) {
   if (rc) return rc;
   uint64_t pend = b->h_io_off.size() - 1;
   if (!pend) return 0;
-  rc = push_many_impl(b, pend, {b->h_pk.data(), b->h_r.data(), b->h_s.data()}, b->h_ios.data(), b->h_io_off.data(), b->h_ad.data(), b->h_ad_off.data());
+  const Scheme& sc = scheme_of(b);
+  Columns cols{};
+  for (uint32_t k = 0; k < sc.ncol; k++) cols[k] = b->h_col[k].data();
+  rc = push_many_impl(b, pend, cols, b->h_ios.data(), b->h_io_off.data(), b->h_ad.data(), b->h_ad_off.data());
   if (rc) return rc;
   if ((rc = quiesce(b))) return rc;        // host vectors are about to be cleared
-  b->h_pk.clear(); b->h_r.clear(); b->h_s.clear(); b->h_ios.clear(); b->h_ad.clear();
+  for (auto& v : b->h_col) v.clear();
+  b->h_ios.clear(); b->h_ad.clear();
   b->h_io_off.assign(1, 0);
   b->h_ad_off.assign(1, 0);
   return 0;
 }
 
-int avrf_thin_batch_push(avrf_batch* b, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
-                         uint32_t ad_len, const uint8_t r[64], const uint8_t s[32]) {
-  if (!b || !pk || !r || !s || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
-  if (b->scheme != 0) return fail(AVRF_ERR_ARG, "not a Thin-VRF batch");
+// One proof of a single push (avrf_thin_batch_push, avrf_pedersen_batch_push): `cols` holds one field per input column
+// of the handle's scheme, in table order.  Eager handles stage it in the pinned double buffer, shipped when it holds
+// STAGE_CHUNK proofs, when its I/O or ad room runs out, or when a later call reads or extends the handle (flush_pending).
+static int push_one(avrf_batch* b, const Columns& cols, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
+                    uint32_t ad_len) {
   if (b->inflight) ENTER(b);             // (the device is bound where CUDA is called: flush_stage)
+  const Scheme& sc = scheme_of(b);
   if (!b->eager) {
     // shards of a multi-process batch: plain host vectors, shipped at prepare
-    b->h_pk.insert(b->h_pk.end(), pk, pk + 64);
-    b->h_r.insert(b->h_r.end(), r, r + 64);
-    b->h_s.insert(b->h_s.end(), s, s + 32);
+    for (uint32_t k = 0; k < sc.ncol; k++) b->h_col[k].insert(b->h_col[k].end(), cols[k], cols[k] + sc.col[k].bytes);
     if (n_ios) b->h_ios.insert(b->h_ios.end(), ios, ios + 128 * (size_t)n_ios);
     if (ad_len) b->h_ad.insert(b->h_ad.end(), ad, ad + ad_len);
     b->h_io_off.push_back(b->h_io_off.back() + n_ios);
@@ -803,11 +812,12 @@ int avrf_thin_batch_push(avrf_batch* b, const uint8_t pk[64], const uint8_t* ios
     size_t want_io = std::max<size_t>(sg->cap_io, 2 * PREP_CHUNK), want_ad = std::max<size_t>(sg->cap_ad, 16 * PREP_CHUNK);
     while (want_io < sg->nio + n_ios) want_io *= 2;
     while (want_ad < sg->nad + ad_len) want_ad *= 2;
-    if ((rc = bind_device(b->device)) || (rc = stage_reserve(*sg, want_io, want_ad))) return rc;
+    if ((rc = bind_device(b->device)) || (rc = stage_reserve(sc, *sg, want_io, want_ad))) return rc;
   }
   size_t j = sg->n;
-  stage_proof(sg->pk.as<uint8_t>() + 64 * j, sg->r.as<uint8_t>() + 64 * j, sg->s.as<uint8_t>() + 32 * j,
-              sg->ios.as<uint8_t>() + 128 * sg->nio, pk, r, s, ios, 128 * (size_t)n_ios);
+  StageField f[5];
+  for (uint32_t k = 0; k < sc.ncol; k++) f[k] = {sg->col[k].as<uint8_t>() + sc.col[k].bytes * j, cols[k], sc.col[k].bytes};
+  stage_proof(f, sc.ncol, sg->ios.as<uint8_t>() + 128 * sg->nio, ios, 128 * (size_t)n_ios);
   if (ad_len) memcpy(sg->ad.as<uint8_t>() + sg->nad, ad, ad_len);
   if (j == 0) { sg->io_off.as<uint32_t>()[0] = 0; sg->ad_off.as<uint32_t>()[0] = 0; }
   sg->nio += n_ios;
@@ -818,6 +828,13 @@ int avrf_thin_batch_push(avrf_batch* b, const uint8_t pk[64], const uint8_t* ios
   return 0;
 }
 
+int avrf_thin_batch_push(avrf_batch* b, const uint8_t pk[64], const uint8_t* ios, uint32_t n_ios, const uint8_t* ad,
+                         uint32_t ad_len, const uint8_t r[64], const uint8_t s[32]) {
+  if (!b || !pk || !r || !s || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
+  if (b->scheme != 0) return fail(AVRF_ERR_ARG, "not a Thin-VRF batch");
+  return push_one(b, {pk, r, s}, ios, n_ios, ad, ad_len);
+}
+
 // push_many of arrays that the caller only lends for the duration of the call (thin.rs:218-225): returns once the
 // device has consumed them - not the hash, which proceeds on the hasher thread.
 static int push_borrowed(avrf_batch* b, uint64_t n, const Columns& cols, const uint8_t* ios, const uint32_t* io_offsets,
@@ -825,7 +842,7 @@ static int push_borrowed(avrf_batch* b, uint64_t n, const Columns& cols, const u
   int rc = check_offsets(n, io_offsets, ad_offsets, ios, ad_blob);
   if (rc) return rc;
   ENTER(b);
-  if ((rc = flush_pending(b))) return rc;          // (single pushes are Thin only: a no-op on a Pedersen handle)
+  if ((rc = flush_pending(b))) return rc;
   if ((rc = push_many_impl(b, n, cols, ios, io_offsets, ad_blob, ad_offsets))) return rc;
   CK(hsync(b, b->st_h2d));
   CK(hsync(b, b->prepared ? b->st_prep : b->st));
@@ -1286,6 +1303,15 @@ int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios,
   if (!io_offsets || !ad_offsets || !pk_com || !r || !ok || !s || !sb) return fail(AVRF_ERR_ARG, "null argument");
   // same pipeline as the thin verifier: chunked H2D -> k_prepare_ped -> D2H of (c, s, sb) -> incremental SHA-512
   return push_borrowed(b, n, {pk_com, r, s, ok, sb}, ios, io_offsets, ad_blob, ad_offsets);
+}
+
+// pedersen::BatchVerifier::push (src/pedersen.rs:322-427): one proof, staged exactly as avrf_thin_batch_push stages one.
+int avrf_pedersen_batch_push(avrf_batch* b, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad, uint32_t ad_len,
+                             const uint8_t pk_com[64], const uint8_t r[64], const uint8_t ok[64], const uint8_t s[32],
+                             const uint8_t sb[32]) {
+  if (!b || !pk_com || !r || !ok || !s || !sb || (n_ios && !ios) || (ad_len && !ad)) return fail(AVRF_ERR_ARG, "null argument");
+  if (b->scheme != 1) return fail(AVRF_ERR_ARG, "not a Pedersen batch");
+  return push_one(b, {pk_com, r, s, ok, sb}, ios, n_ios, ad, ad_len);
 }
 
 int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status) {

@@ -15,17 +15,13 @@ __attribute__((target("avx2"))) static void copy_nt_avx2(void* dst, const void* 
 
 static const bool g_avx2 = __builtin_cpu_supports("avx2");
 
-// One staged proof: pk (64 B), r (64 B), s (32 B) and n_ios pairs (128 B each), every destination 32-byte aligned.
-__attribute__((target("avx2"))) static void stage_proof_avx2(uint8_t* dpk, uint8_t* dr, uint8_t* ds, uint8_t* dio, const uint8_t* pk,
-                                                             const uint8_t* r, const uint8_t* s, const uint8_t* ios, size_t io_bytes) {
-  const __m256i a0 = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(pk)), a1 = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(pk + 32));
-  const __m256i b0 = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(r)), b1 = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(r + 32));
-  const __m256i c0 = _mm256_loadu_si256(reinterpret_cast<const __m256i*>(s));
-  _mm256_stream_si256(reinterpret_cast<__m256i*>(dpk), a0);
-  _mm256_stream_si256(reinterpret_cast<__m256i*>(dpk + 32), a1);
-  _mm256_stream_si256(reinterpret_cast<__m256i*>(dr), b0);
-  _mm256_stream_si256(reinterpret_cast<__m256i*>(dr + 32), b1);
-  _mm256_stream_si256(reinterpret_cast<__m256i*>(ds), c0);
+// One staged proof: its fixed-size fields (32-byte multiples each) and n_ios pairs (128 B each), every destination
+// 32-byte aligned.
+__attribute__((target("avx2"))) static void stage_proof_avx2(const avrf::StageField* f, size_t nf, uint8_t* dio, const uint8_t* ios,
+                                                             size_t io_bytes) {
+  for (size_t k = 0; k < nf; k++)
+    for (size_t i = 0; i < f[k].bytes; i += 32)
+      _mm256_stream_si256(reinterpret_cast<__m256i*>(f[k].dst + i), _mm256_loadu_si256(reinterpret_cast<const __m256i*>(f[k].src + i)));
   for (size_t i = 0; i < io_bytes; i += 32)
     _mm256_stream_si256(reinterpret_cast<__m256i*>(dio + i), _mm256_loadu_si256(reinterpret_cast<const __m256i*>(ios + i)));
 }
@@ -35,14 +31,11 @@ void stage_copy(void* dst, const void* src, size_t n) {
   if (g_avx2 && (n & 31) == 0 && (reinterpret_cast<uintptr_t>(dst) & 31) == 0) copy_nt_avx2(dst, src, n);
   else memcpy(dst, src, n);
 }
-void stage_proof(uint8_t* dpk, uint8_t* dr, uint8_t* ds, uint8_t* dio, const uint8_t* pk, const uint8_t* r, const uint8_t* s,
-                 const uint8_t* ios, size_t io_bytes) {
+void stage_proof(const StageField* f, size_t nf, uint8_t* dio, const uint8_t* ios, size_t io_bytes) {
   if (g_avx2) {
-    stage_proof_avx2(dpk, dr, ds, dio, pk, r, s, ios, io_bytes);
+    stage_proof_avx2(f, nf, dio, ios, io_bytes);
   } else {
-    memcpy(dpk, pk, 64);
-    memcpy(dr, r, 64);
-    memcpy(ds, s, 32);
+    for (size_t k = 0; k < nf; k++) memcpy(f[k].dst, f[k].src, f[k].bytes);
     if (io_bytes) memcpy(dio, ios, io_bytes);
   }
 }
@@ -51,11 +44,8 @@ void stage_fence() { _mm_sfence(); }
 #else
 namespace avrf {
 void stage_copy(void* dst, const void* src, size_t n) { memcpy(dst, src, n); }
-void stage_proof(uint8_t* dpk, uint8_t* dr, uint8_t* ds, uint8_t* dio, const uint8_t* pk, const uint8_t* r, const uint8_t* s,
-                 const uint8_t* ios, size_t io_bytes) {
-  memcpy(dpk, pk, 64);
-  memcpy(dr, r, 64);
-  memcpy(ds, s, 32);
+void stage_proof(const StageField* f, size_t nf, uint8_t* dio, const uint8_t* ios, size_t io_bytes) {
+  for (size_t k = 0; k < nf; k++) memcpy(f[k].dst, f[k].src, f[k].bytes);
   if (io_bytes) memcpy(dio, ios, io_bytes);
 }
 void stage_fence() {}

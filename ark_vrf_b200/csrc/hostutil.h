@@ -8,9 +8,15 @@ namespace avrf {
 // aligned destinations; plain memcpy otherwise): the staged bytes are read next by the GPU's DMA engine, not by
 // this core, so they need not displace the caller's working set or cost a read-for-ownership.
 void stage_copy(void* dst, const void* src, size_t n);
-// One proof of a single push into the staging arrays (all destinations 32-byte aligned), one call.
-void stage_proof(uint8_t* dpk, uint8_t* dr, uint8_t* ds, uint8_t* dio, const uint8_t* pk, const uint8_t* r, const uint8_t* s,
-                 const uint8_t* ios, size_t io_bytes);
+// One fixed-size field of a staged proof: `bytes` (a multiple of 32) from `src` to the 32-byte aligned `dst`.
+struct StageField {
+  uint8_t* dst;
+  const uint8_t* src;
+  size_t bytes;
+};
+// One proof of a single push into the staging arrays, one call: its `nf` fields, then `io_bytes` of I/O pairs into the
+// 32-byte aligned `dio`.
+void stage_proof(const StageField* f, size_t nf, uint8_t* dio, const uint8_t* ios, size_t io_bytes);
 // Orders the non-temporal stores before the DMA is queued.
 void stage_fence();
 }  // namespace avrf

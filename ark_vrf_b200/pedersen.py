@@ -3,7 +3,10 @@
 Mirror of `ark_vrf::pedersen` (reference src/pedersen.rs):
     Prover::prove                    prove_many(...)             (pedersen.rs:136-186, n proofs per call)
     Verifier::verify                 verify(suite, ios, ad, proof)  (pedersen.rs:188-253, exact)
-    BatchVerifier::{new, push, push_prepared, verify}   BatchVerifier  (pedersen.rs:322-427; the MSM has 5N+2 points)
+    BatchVerifier::{new, push, push_prepared, verify}   BatchVerifier  (pedersen.rs:322-427; the MSM has 5N+2 points;
+                                                    push stages each proof in pinned memory, shipped in chunks)
+    (handle controls, as thin.BatchVerifier)        BatchVerifier.{verify_async, verify_wait, reserve, set_blocking,
+                                                    set_hash_pool, invalidate, timings, stream, clear}
     (wire-format proofs)             BatchVerifier.push_compressed(), serialize_proofs()  (Proof::{de,}serialize_compressed)
     (per-proof verdicts)             BatchVerifier.verify_each() / find_invalid()
     (throughput mode)                BatchServer: whole batches on a native worker pool, decoded or in wire format
@@ -20,7 +23,7 @@ from . import _lib
 from .ops import pedersen_prove_many as prove_many          # noqa: F401  (re-exported: pedersen.prove_many)
 from .ops import point_compress
 from .synth import ORDER
-from .thin import Format, Suite, Tap, _ServerBase, _bytes_of, _ios_bytes, _raise_for_status, ptr
+from .thin import Format, Suite, Tap, _BatchBase, _ServerBase, _bytes_of, _ios_bytes, _raise_for_status, ptr
 
 
 @dataclass
@@ -40,15 +43,13 @@ class BatchItem:                          # pedersen::BatchItem; hashing deferre
     proof: Proof
 
 
-class BatchVerifier:
+class BatchVerifier(_BatchBase):
+    """pedersen::BatchVerifier<S> (src/pedersen.rs:322-427) on one B200; the handle controls are `thin.BatchVerifier`'s."""
+
     def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL):
         self._lib = _lib.load()
         self.suite, self.fmt = Suite(suite), Format(fmt)
-        self._h = self._lib.avrf_pedersen_batch_new(int(self.suite), int(self.fmt))
-        if not self._h:
-            msg = self._lib.avrf_last_error()
-            raise _lib.AvrfError(msg.decode() if msg else "avrf_pedersen_batch_new failed")
-        self._n = 0
+        self._open(self._lib.avrf_pedersen_batch_new(int(self.suite), int(self.fmt)), "avrf_pedersen_batch_new")
 
     @staticmethod
     def prepare(ios, ad, proof: Proof) -> BatchItem:
@@ -56,12 +57,10 @@ class BatchVerifier:
         return BatchItem(iob, k, bytes(ad), proof)
 
     def push_prepared(self, e: BatchItem) -> None:
-        io_off = np.array([0, e.n_ios], dtype=np.uint32)
-        ad_off = np.array([0, len(e.ad)], dtype=np.uint32)
-        f = lambda b, n: np.frombuffer(_bytes_of(b, n), dtype=np.uint8).copy()
-        self.push_many(np.frombuffer(e.ios + bytes(128), dtype=np.uint8).copy(), io_off,
-                       np.frombuffer(e.ad + bytes(16), dtype=np.uint8).copy(), ad_off,
-                       f(e.proof.pk_com, 64), f(e.proof.r, 64), f(e.proof.ok, 64), f(e.proof.s, 32), f(e.proof.sb, 32))
+        p = e.proof
+        _lib.check(self._lib.avrf_pedersen_batch_push(self._h, e.ios if e.n_ios else None, e.n_ios, e.ad if e.ad else None,
+                                                      len(e.ad), _bytes_of(p.pk_com, 64), _bytes_of(p.r, 64),
+                                                      _bytes_of(p.ok, 64), _bytes_of(p.s, 32), _bytes_of(p.sb, 32)))
 
     def push(self, ios, ad, proof: Proof) -> None:
         self.push_prepared(self.prepare(ios, ad, proof))
@@ -70,7 +69,6 @@ class BatchVerifier:
         n = len(io_offsets) - 1
         _lib.check(self._lib.avrf_pedersen_batch_push_many(self._h, n, ptr(ios), ptr(io_offsets), ptr(ad_blob),
                                                            ptr(ad_offsets), ptr(pk_com), ptr(r), ptr(ok), ptr(s), ptr(sb)))
-        self._n += n
 
     def push_compressed(self, ios32, io_offsets, ad_blob, ad_offsets, proofs) -> np.ndarray:
         """`avrf_pedersen_batch_push_compressed`: proofs in wire format, (n, 160) records of
@@ -83,53 +81,30 @@ class BatchVerifier:
         bad = C.c_uint64(0)
         _lib.check(self._lib.avrf_pedersen_batch_push_compressed(self._h, n, ptr(ios32), ptr(io_offsets), ptr(ad_blob),
                                                                  ptr(ad_offsets), ptr(proofs), ptr(ok), C.byref(bad)))
-        if bad.value == 0:
-            self._n += n
         return ok[:n]
-
-    def clear(self) -> None:
-        """Forget all pushed proofs, keep allocations."""
-        _lib.check(self._lib.avrf_thin_batch_clear(self._h))
-        self._n = 0
 
     def verify_status(self) -> int:
         st = C.c_int32(-1)
         _lib.check(self._lib.avrf_pedersen_batch_verify(self._h, C.byref(st)))
         return st.value
 
-    def verify(self) -> None:
-        _raise_for_status(self.verify_status())
-
     def verify_each(self) -> np.ndarray:
         """Per-proof status codes (0 Ok, 1 VerificationFailure, 2 InvalidData) under `pedersen::Verifier::verify`."""
-        out = np.full(max(self._n, 1), -1, dtype=np.int32)
+        n = len(self)
+        out = np.full(max(n, 1), -1, dtype=np.int32)
         _lib.check(self._lib.avrf_pedersen_batch_verify_each(self._h, ptr(out)))
-        return out[:self._n]
+        return out[:n]
 
     def find_invalid(self) -> np.ndarray:
         """Indices of the proofs a failed batch owes its verdict to; empty when every proof verifies."""
         return np.nonzero(self.verify_each() != 0)[0]
 
     def tap(self, what: Tap) -> np.ndarray:
-        n = self._n
+        n = len(self)
         size = {Tap.C: 16 * n, Tap.W: 32 * n, Tap.SEED: 64, Tap.SCALARS: 32 * (5 * n + 2), Tap.PARTIAL: 128}[Tap(what)]
         buf = np.zeros(max(size, 1), dtype=np.uint8)
         _lib.check(self._lib.avrf_thin_batch_tap(self._h, int(what), ptr(buf), buf.nbytes))
         return buf
-
-    def __len__(self) -> int:
-        return self._n
-
-    def close(self) -> None:
-        if getattr(self, "_h", None):
-            self._lib.avrf_thin_batch_free(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 class BatchServer(_ServerBase):

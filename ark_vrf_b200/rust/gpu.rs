@@ -85,6 +85,10 @@ extern "C" {
         b: *mut AvrfBatch, n: u64, ios: *const u8, io_offsets: *const u32, ad_blob: *const u8,
         ad_offsets: *const u32, pk_com: *const u8, r: *const u8, ok: *const u8, s: *const u8, sb: *const u8,
     ) -> i32;
+    fn avrf_pedersen_batch_push(
+        b: *mut AvrfBatch, ios: *const u8, n_ios: u32, ad: *const u8, ad_len: u32, pk_com: *const u8, r: *const u8,
+        ok: *const u8, s: *const u8, sb: *const u8,
+    ) -> i32;
     fn avrf_pedersen_batch_push_compressed(
         b: *mut AvrfBatch, n: u64, ios32: *const u8, io_offsets: *const u32, ad_blob: *const u8,
         ad_offsets: *const u32, proofs: *const u8, ok: *mut u8, n_bad: *mut u64,
@@ -541,13 +545,20 @@ pub mod pedersen {
             Self { h, _s: PhantomData }
         }
 
+        /// Like `Vec::with_capacity`: device memory for `n` proofs up front, so that a loop of `push` never reallocates.
+        pub fn with_capacity(n: usize, n_ios: usize, ad_bytes: usize) -> Self {
+            let v = Self::new();
+            let rc = unsafe { avrf_thin_batch_reserve(v.h, n as u64, n_ios as u64, ad_bytes as u64) };
+            assert!(rc == 0, "libavrf_gpu system error {rc}");
+            v
+        }
+
         pub fn push(&mut self, ios: impl AsRef<[VrfIo<S>]>, ad: impl AsRef<[u8]>, proof: &Proof<S>) {
             let (ios, ad) = (ios.as_ref(), ad.as_ref());
-            let io_off = [0u32, ios.len() as u32];
-            let ad_off = [0u32, ad.len() as u32];
+            // VrfIo<S> is { input: Input(Affine), output: Output(Affine) }: 128 contiguous bytes per pair
             let rc = unsafe {
-                avrf_pedersen_batch_push_many(
-                    self.h, 1, ios.as_ptr() as *const u8, io_off.as_ptr(), ad.as_ptr(), ad_off.as_ptr(),
+                avrf_pedersen_batch_push(
+                    self.h, ios.as_ptr() as *const u8, ios.len() as u32, ad.as_ptr(), ad.len() as u32,
                     point_bytes::<S>(&proof.pk_com), point_bytes::<S>(&proof.r), point_bytes::<S>(&proof.ok),
                     scalar_bytes::<S>(&proof.s), scalar_bytes::<S>(&proof.sb),
                 )

@@ -135,7 +135,77 @@ class BatchItem:                          # thin::BatchItem (src/thin.rs:172-179
     s: bytes
 
 
-class BatchVerifier:
+class _BatchBase:
+    """The controls of a batch handle that serve both schemes (include/avrf.h): `thin.BatchVerifier` and
+    `pedersen.BatchVerifier` share them.  Pushes, taps and per-proof verdicts are scheme-specific and stay in those
+    classes."""
+
+    def _open(self, handle, what: str) -> None:
+        self._h = handle
+        if not self._h:
+            msg = self._lib.avrf_last_error()
+            raise _lib.AvrfError(msg.decode() if msg else f"{what} failed")
+
+    def verify(self) -> None:
+        """Ok -> returns None; otherwise raises VerificationFailure or InvalidData."""
+        _raise_for_status(self.verify_status())
+
+    def verify_async(self) -> None:
+        """Enqueue the verification on the GPU and return (pair with `verify_wait`)."""
+        _lib.check(self._lib.avrf_thin_batch_verify_async(self._h))
+
+    def verify_wait(self) -> int:
+        st = C.c_int32(-1)
+        _lib.check(self._lib.avrf_thin_batch_verify_wait(self._h, C.byref(st)))
+        return st.value
+
+    def set_blocking(self, blocking: bool = True) -> None:
+        """Host waits sleep instead of spinning (use when several handles are driven from as many threads)."""
+        _lib.check(self._lib.avrf_thin_batch_set_blocking(self._h, 1 if blocking else 0))
+
+    def set_hash_pool(self, pool: Optional["HashPool"]) -> None:
+        """Hash this handle's batch seeds in a lane of a shared multi-buffer pool (None: on its own thread)."""
+        _lib.check(self._lib.avrf_thin_batch_set_hash_pool(self._h, pool._h if pool is not None else None))
+        self._pool = pool                 # keep it alive
+
+    def reserve(self, n: int, n_ios: int, ad_bytes: int) -> None:
+        """Room for `n` proofs (like `Vec::with_capacity`): pushes up to that size never reallocate device memory."""
+        _lib.check(self._lib.avrf_thin_batch_reserve(self._h, n, n_ios, ad_bytes))
+
+    def clear(self) -> None:
+        """Forget all pushed proofs, keep allocations."""
+        _lib.check(self._lib.avrf_thin_batch_clear(self._h))
+
+    def invalidate(self) -> None:
+        """Forget c_j / z_ij / prepared bases; inputs stay resident (next verify redoes prepare)."""
+        _lib.check(self._lib.avrf_thin_batch_invalidate(self._h))
+
+    def __len__(self) -> int:
+        return int(self._lib.avrf_thin_batch_len(self._h))
+
+    @property
+    def stream(self) -> int:
+        """The handle's CUDA stream (a ``cudaStream_t`` as an integer) - record timing events on it."""
+        return int(self._lib.avrf_thin_batch_stream(self._h))
+
+    def timings(self) -> dict:
+        t = _lib.Timings()
+        _lib.check(self._lib.avrf_thin_batch_timings(self._h, C.byref(t)))
+        return t.as_dict()
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.avrf_thin_batch_free(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class BatchVerifier(_BatchBase):
     """thin::BatchVerifier<S> (src/thin.rs:188-326) on one B200."""
 
     def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL, eager_seed: bool = True,
@@ -143,10 +213,7 @@ class BatchVerifier:
         self._lib = _lib.load()
         self.suite = Suite(suite)
         self.fmt = Format(fmt)
-        self._h = self._lib.avrf_thin_batch_new_on(int(device), int(self.suite), int(self.fmt))
-        if not self._h:
-            msg = self._lib.avrf_last_error()
-            raise _lib.AvrfError(msg.decode() if msg else "avrf_thin_batch_new failed")
+        self._open(self._lib.avrf_thin_batch_new_on(int(device), int(self.suite), int(self.fmt)), "avrf_thin_batch_new")
         self._n_ios = 0
         if not eager_seed:
             _lib.check(self._lib.avrf_thin_batch_set_eager(self._h, 0))
@@ -164,10 +231,6 @@ class BatchVerifier:
 
     def push(self, public, ios, ad, proof: Proof) -> None:
         self.push_prepared(self.prepare(public, ios, ad, proof))
-
-    def verify(self) -> None:
-        """Ok -> returns None; otherwise raises VerificationFailure or InvalidData."""
-        _raise_for_status(self.verify_status())
 
     # -- bulk / measurement API ---------------------------------------------------------------
     def push_many(self, pk, ios, io_offsets, ad_blob, ad_offsets, r, s) -> None:
@@ -191,19 +254,6 @@ class BatchVerifier:
             self._n_ios += int(io_offsets[n])
         return ok[:n]
 
-    def set_blocking(self, blocking: bool = True) -> None:
-        """Host waits sleep instead of spinning (use when several handles are driven from as many threads)."""
-        _lib.check(self._lib.avrf_thin_batch_set_blocking(self._h, 1 if blocking else 0))
-
-    def set_hash_pool(self, pool: Optional["HashPool"]) -> None:
-        """Hash this handle's batch seeds in a lane of a shared multi-buffer pool (None: on its own thread)."""
-        _lib.check(self._lib.avrf_thin_batch_set_hash_pool(self._h, pool._h if pool is not None else None))
-        self._pool = pool                 # keep it alive
-
-    def reserve(self, n: int, n_ios: int, ad_bytes: int) -> None:
-        """Room for `n` proofs (like `Vec::with_capacity`): pushes up to that size never reallocate device memory."""
-        _lib.check(self._lib.avrf_thin_batch_reserve(self._h, n, n_ios, ad_bytes))
-
     def verify_status(self) -> int:
         st = C.c_int32(-1)
         _lib.check(self._lib.avrf_thin_batch_verify(self._h, C.byref(st)))
@@ -220,30 +270,9 @@ class BatchVerifier:
         src/thin.rs:131-165); empty when every proof verifies.  The reference only reports that some proof is bad."""
         return np.nonzero(self.verify_each() != 0)[0]
 
-    def verify_async(self) -> None:
-        """Enqueue the verification on the GPU and return (pair with `verify_wait`)."""
-        _lib.check(self._lib.avrf_thin_batch_verify_async(self._h))
-
-    def verify_wait(self) -> int:
-        st = C.c_int32(-1)
-        _lib.check(self._lib.avrf_thin_batch_verify_wait(self._h, C.byref(st)))
-        return st.value
-
     def clear(self) -> None:
-        _lib.check(self._lib.avrf_thin_batch_clear(self._h))
+        super().clear()
         self._n_ios = 0
-
-    def invalidate(self) -> None:
-        """Forget c_j / z_ij / prepared bases; inputs stay resident (next verify redoes prepare)."""
-        _lib.check(self._lib.avrf_thin_batch_invalidate(self._h))
-
-    def __len__(self) -> int:
-        return int(self._lib.avrf_thin_batch_len(self._h))
-
-    @property
-    def stream(self) -> int:
-        """The handle's CUDA stream (a ``cudaStream_t`` as an integer) - record timing events on it."""
-        return int(self._lib.avrf_thin_batch_stream(self._h))
 
     def set_weights_mode(self, mode: int) -> None:
         _lib.check(self._lib.avrf_thin_batch_set_weights_mode(self._h, mode))
@@ -287,22 +316,6 @@ class BatchVerifier:
         buf = np.zeros(max(size, 1), dtype=np.uint8)
         _lib.check(self._lib.avrf_thin_batch_tap(self._h, int(what), ptr(buf), buf.nbytes))
         return buf
-
-    def timings(self) -> dict:
-        t = _lib.Timings()
-        _lib.check(self._lib.avrf_thin_batch_timings(self._h, C.byref(t)))
-        return t.as_dict()
-
-    def close(self) -> None:
-        if getattr(self, "_h", None):
-            self._lib.avrf_thin_batch_free(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 class HashPool:

@@ -246,14 +246,29 @@ int avrf_thin_sharded_timings(const avrf_sharded* sh, avrf_sharded_timings* out)
 avrf_batch* avrf_thin_sharded_shard(avrf_sharded* sh, int index);
 
 /* ---- Pedersen VRF batch verifier (SURVEY 8f-3; reference src/pedersen.rs:255-427) on the same MSM engine ---
- * pedersen::BatchVerifier::new / push (x n) / verify.  The handle is an avrf_batch: _free, _clear, _len,
+ * pedersen::BatchVerifier::new / push (x n) / verify.  The handle is an avrf_batch: _free, _clear, _len, _reserve,
+ * _invalidate, _set_eager, _set_blocking, _set_hash_pool, _verify_async / _verify_wait, _timings, _stream and
  * _tap (C, SEED, W = t_i||u_i, SCALARS, PARTIAL = the 5N+2-point MSM sum) apply; proofs are (pk_com 64, r 64,
- * ok 64, s 32, sb 32). */
+ * ok 64, s 32, sb 32).  AVRF_WEIGHTS_TREE, _tree_leaves and the sharded path are Thin only. */
 avrf_batch* avrf_pedersen_batch_new(uint32_t suite, uint32_t fmt);
 int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
                                   const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,
                                   const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);
 int avrf_pedersen_batch_verify(avrf_batch* b, int32_t* status);
+
+/* pedersen::BatchVerifier::push (src/pedersen.rs:322-427): one proof, `ios` = n_ios pairs (128 B each).  Behaves as
+ * avrf_thin_batch_push does for Thin handles: a verify still in flight completes first; on an eager handle the proof
+ * is staged in pinned host memory and shipped half a 75776-proof chunk at a time (or earlier, when the staging room for
+ * I/O pairs or ad runs out, or when any later call reads or extends the handle), so the batch order is the call order;
+ * on a non-eager handle it waits in host memory until prepare.  _len counts staged proofs, _clear drops them.  A null
+ * argument or a Thin handle is AVRF_ERR_ARG (and avrf_thin_batch_push refuses Pedersen handles).
+ * The first single push on a handle allocates two pinned staging buffers, each of 75776 x 256 bytes of proof columns
+ * (19.4 MB; a Thin handle stages 160 bytes per proof, 12.1 MB) plus room for 151552 I/O pairs (19.4 MB) and 1.2 MB of
+ * ad, which grows for larger proofs: about 81 MB for a Pedersen handle against 67 MB for a Thin one, kept until the
+ * handle is freed. */
+int avrf_pedersen_batch_push(avrf_batch* b, const uint8_t* ios, uint32_t n_ios, const uint8_t* ad, uint32_t ad_len,
+                             const uint8_t pk_com[64], const uint8_t r[64], const uint8_t ok[64], const uint8_t s[32],
+                             const uint8_t sb[32]);
 
 /* The same push for proofs in WIRE format: `proofs` is n records of 160 bytes, each exactly
  * pedersen::Proof::serialize_compressed (pk_com 32 | r 32 | ok 32 | s 32 | sb 32, src/pedersen.rs:43-50: compressed

@@ -9,7 +9,7 @@
 //   thin::ShardedBatchVerifier<S>                 (new: one batch over several GPUs of this process, avrf_thin_sharded_*)
 //   pedersen::Proof{pk_com, r, ok, s, sb}         src/pedersen.rs:43-50
 //   pedersen::verify (pedersen::Verifier)         src/pedersen.rs:188-253
-//   pedersen::BatchVerifier<S>::{push, push_compressed, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
+//   pedersen::BatchVerifier<S>::{reserve, push, push_compressed, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
 //   pedersen::prove_many (Prover::prove, n proofs) src/pedersen.rs:136-186
 //   pedersen::BatchServer<S>::{submit, submit_compressed, wait}   (new: the same worker pool for Pedersen batches)
 //   Error::{VerificationFailure, InvalidData}     src/lib.rs:136-147
@@ -220,13 +220,15 @@ class BatchVerifier {
   ~BatchVerifier() { avrf_thin_batch_free(h_); }
   BatchVerifier(const BatchVerifier&) = delete;
   BatchVerifier& operator=(const BatchVerifier&) = delete;
+  // like Vec::with_capacity: device memory for n proofs up front, so that a loop of push() never reallocates
+  void reserve(uint64_t n, uint64_t n_ios, uint64_t ad_bytes) { check(avrf_thin_batch_reserve(h_, n, n_ios, ad_bytes)); }
   int64_t len() const { return avrf_thin_batch_len(h_); }
   void clear() { check(avrf_thin_batch_clear(h_)); }
+  // one proof, staged in pinned memory and shipped to the device in chunks (avrf_pedersen_batch_push)
   void push(const std::vector<VrfIo>& ios, const std::vector<uint8_t>& ad, const Proof& proof) {
-    uint32_t io_off[2] = {0, (uint32_t)ios.size()}, ad_off[2] = {0, (uint32_t)ad.size()};
-    check(avrf_pedersen_batch_push_many(h_, 1, ios.empty() ? nullptr : ios[0].input.data(), io_off,
-                                        ad.empty() ? nullptr : ad.data(), ad_off, proof.pk_com.data(), proof.r.data(),
-                                        proof.ok.data(), proof.s.data(), proof.sb.data()));
+    check(avrf_pedersen_batch_push(h_, ios.empty() ? nullptr : ios[0].input.data(), (uint32_t)ios.size(),
+                                   ad.empty() ? nullptr : ad.data(), (uint32_t)ad.size(), proof.pk_com.data(),
+                                   proof.r.data(), proof.ok.data(), proof.s.data(), proof.sb.data()));
   }
   // Proofs in wire format: n records of Proof::serialize_compressed (pk_com | r | ok | s | sb, 160 bytes) and 64 bytes
   // of compressed (input, output) per pair, decoded and validated on the device.  Returns the number of proofs that

@@ -3,6 +3,11 @@ each, 4096 signers; every proof distinct).  Prints one JSON line with the device
 run.  Legs (best of --reps after a warm-up, except the latency leg):
   prove_many        avrf_pedersen_prove_many, proofs/s
   batch             push of the 2^20 proofs from pinned memory + verify, wall time, with avrf_thin_batch_timings
+  drop_in           the reference's call sequence: pedersen::BatchVerifier::push once per proof through the C++ mirror
+                    (tools/push_loop.cpp, heap items, Montgomery format) + verify, wall time of the push loop and of
+                    verify; beside it, at 2^14 proofs (a 2^20 loop of it takes too long to repeat), the same loop with
+                    each proof pushed as a one-proof push_many - what BatchVerifier::push did before single pushes were
+                    staged - reported per proof
   wire              the same batch serialised once (pedersen.serialize_proofs: 160-byte records, compressed I/O pairs),
                     pushed from pinned memory through push_compressed (decoded and validated on the GPU) + verify, wall
                     time; then one more push + verify under torch.profiler for the device time of the decode kernels
@@ -63,6 +68,41 @@ def decode_kernel_ms(fn):
     return out
 
 
+def drop_in(b, n, reps):
+    """The `drop_in` leg: best of `reps` push loops + verify after a warm-up, and the one-proof push_many loop."""
+    import numpy as np
+    from ark_vrf_b200 import Format, synth
+    pl = ctypes.CDLL(os.path.join(ROOT, "tools", "libavrf_pushloop.so"))
+    pl.avrf_pushloop_ped_new.restype = ctypes.c_void_p
+    pl.avrf_pushloop_ped_new.argtypes = [ctypes.c_uint64] + [ctypes.c_void_p] * 9
+    pl.avrf_pushloop_ped_step.argtypes = [ctypes.c_void_p, ctypes.c_uint64, ctypes.c_int,
+                                          ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]
+    pl.avrf_pushloop_ped_free.argtypes = [ctypes.c_void_p]
+    # the batch leg's statements, proven again with the points and scalars as arkworks values lie in memory
+    mb = synth.make_pedersen_batch(b.suite, n, 1, 4096, Format.MONTGOMERY)
+    arrs = [np.ascontiguousarray(x) for x in (mb.ios, mb.io_offsets, mb.ad_blob, mb.ad_offsets, mb.pk_com, mb.r, mb.ok,
+                                              mb.s, mb.sb)]
+    h = pl.avrf_pushloop_ped_new(n, *[x.ctypes.data for x in arrs])
+    assert h
+    pm, vm = ctypes.c_double(0), ctypes.c_double(0)
+
+    def step(n_items, one_by_one_many):
+        assert pl.avrf_pushloop_ped_step(h, n_items, one_by_one_many, ctypes.byref(pm), ctypes.byref(vm)) == 0
+        return pm.value, vm.value
+    try:
+        runs = [step(0, 0) for _ in range(reps + 1)][1:]
+        push_ms, verify_ms = min(runs, key=sum)
+        n_old = min(n, 1 << 14)
+        old = [step(n_old, 1) for _ in range(3)][1:]
+        new = [step(n_old, 0) for _ in range(3)][1:]
+    finally:
+        pl.avrf_pushloop_ped_free(h)
+    return {"n": n, "push_loop_ms": round(push_ms, 2), "verify_ms": round(verify_ms, 2),
+            "total_ms": round(push_ms + verify_ms, 2), "proofs_per_s": round(n / ((push_ms + verify_ms) * 1e-3)),
+            "one_proof_push_many": {"n": n_old, "push_us_per_proof": round(1e3 * min(p for p, _ in old) / n_old, 2),
+                                    "staged_push_us_per_proof": round(1e3 * min(p for p, _ in new) / n_old, 3)}}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--log2n", type=int, default=20)
@@ -104,6 +144,7 @@ def main():
     res["batch_push_verify_ms"] = round(1e3 * t, 2)
     res["batch_proofs_per_s"] = round(n / t)
     res["batch_timings"] = {k: (round(v, 3) if isinstance(v, float) else v) for k, v in tm.as_dict().items()}
+    res["drop_in"] = drop_in(b, n, a.reps)
 
     # wire format: what callers hold before Proof::deserialize_compressed
     nio = int(b.io_offsets[n])
