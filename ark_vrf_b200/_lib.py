@@ -92,6 +92,11 @@ SIGNATURES = {
     "avrf_thin_sharded_timings": (C.c_int, [C.c_void_p, C.POINTER(ShardedTimings)]),
     "avrf_thin_sharded_shard": (C.c_void_p, [C.c_void_p, C.c_int]),
     "avrf_pedersen_batch_new": (C.c_void_p, [C.c_uint32, C.c_uint32]),
+    "avrf_pedersen_batch_new_on": (C.c_void_p, [C.c_int, C.c_uint32, C.c_uint32]),
+    "avrf_pedersen_sharded_new": (C.c_void_p, [C.c_uint32, C.c_uint32]),
+    "avrf_pedersen_sharded_push_many": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
+    "avrf_pedersen_seed": (C.c_int, [C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "avrf_pedersen_seed_dev": (C.c_int, [C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p]),
     "avrf_pedersen_batch_push_many": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 9),
     "avrf_pedersen_batch_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32] + [C.c_void_p] * 5),
     "avrf_pedersen_batch_push_compressed": (C.c_int, [C.c_void_p, C.c_uint64] + [C.c_void_p] * 7),

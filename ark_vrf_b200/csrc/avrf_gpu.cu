@@ -166,6 +166,14 @@ static size_t batch_prefix(uint32_t suite, unsigned char buf[40]) {
   return sl + 1;
 }
 
+// SHA512(SUITE_ID || 0x50 || stream) of a host-resident batch-seed stream of n_items records of `stride` bytes (the
+// Scheme::cs_stride of the proofs' scheme): avrf_thin_seed, avrf_pedersen_seed.
+static int seed_of_stream(uint32_t suite, const uint8_t* stream, uint64_t n_items, size_t stride, uint8_t seed[64]) {
+  if (suite > 2 || !seed || (n_items && !stream)) return fail(AVRF_ERR_ARG, "bad argument");
+  unsigned char prefix[40];
+  return sha512({{prefix, batch_prefix(suite, prefix)}, {stream, stride * n_items}}, seed);
+}
+
 // Orders `waiter` after the work enqueued so far on `st`.
 static int stream_after(cudaStream_t waiter, cudaStream_t st) {
   cudaEvent_t e;
@@ -926,9 +934,11 @@ void* avrf_thin_batch_cs_dev(avrf_batch* b) {
 }
 
 int avrf_thin_seed(uint32_t suite, const uint8_t* cs_stream, uint64_t n_items, uint8_t seed[64]) {
-  if (suite > 2 || !seed || (n_items && !cs_stream)) return fail(AVRF_ERR_ARG, "bad argument");
-  unsigned char prefix[40];
-  return sha512({{prefix, batch_prefix(suite, prefix)}, {cs_stream, 64 * n_items}}, seed);
+  return seed_of_stream(suite, cs_stream, n_items, SCHEMES[0].cs_stride, seed);
+}
+
+int avrf_pedersen_seed(uint32_t suite, const uint8_t* stream, uint64_t n_items, uint8_t seed[64]) {
+  return seed_of_stream(suite, stream, n_items, SCHEMES[1].cs_stride, seed);
 }
 
 }  // extern "C"
@@ -1001,7 +1011,16 @@ static int seed_from_device(avrf_batch* b) {
 }
 
 static PinBuf g_pin_stream[AVRF_MAX_DEV];
-static std::mutex g_pin_mu;               // guards g_pin_stream (avrf_thin_seed_dev)
+static std::mutex g_pin_mu;               // guards g_pin_stream (avrf_thin_seed_dev, avrf_pedersen_seed_dev)
+
+// The same seed of a device-resident stream (avrf_thin_seed_dev, avrf_pedersen_seed_dev), on the default device.
+static int seed_of_dev_stream(uint32_t suite, const void* stream_dev, uint64_t n_items, size_t stride, uint8_t seed[64]) {
+  if (suite > 2 || !seed || (n_items && !stream_dev)) return fail(AVRF_ERR_ARG, "bad argument");
+  NEED_DEVICE();
+  std::lock_guard<std::mutex> lock(g_pin_mu);
+  return seed_of_device_stream(gs(), gc(), suite, (const uint8_t*)stream_dev, stride * n_items, g_pin_stream[g_device.load()],
+                               seed);
+}
 
 static void seed_to_words(Seed64& sd, const uint8_t seed[64]) {
   for (int i = 0; i < 8; i++) {
@@ -1170,10 +1189,11 @@ static void collect_timings(avrf_batch* b, bool with_prepare) {
 extern "C" {
 
 int avrf_thin_seed_dev(uint32_t suite, const void* cs_stream_dev, uint64_t n_items, uint8_t seed[64]) {
-  if (suite > 2 || !seed || (n_items && !cs_stream_dev)) return fail(AVRF_ERR_ARG, "bad argument");
-  NEED_DEVICE();
-  std::lock_guard<std::mutex> lock(g_pin_mu);
-  return seed_of_device_stream(gs(), gc(), suite, (const uint8_t*)cs_stream_dev, 64 * n_items, g_pin_stream[g_device.load()], seed);
+  return seed_of_dev_stream(suite, cs_stream_dev, n_items, SCHEMES[0].cs_stride, seed);
+}
+
+int avrf_pedersen_seed_dev(uint32_t suite, const void* stream_dev, uint64_t n_items, uint8_t seed[64]) {
+  return seed_of_dev_stream(suite, stream_dev, n_items, SCHEMES[1].cs_stride, seed);
 }
 
 int avrf_thin_batch_partial(avrf_batch* b, const uint8_t seed[64], uint64_t first_index, uint8_t partial[128]) {
@@ -1289,11 +1309,13 @@ int avrf_thin_batch_verify(avrf_batch* b, int32_t* status) {
 }
 
 // ---- Pedersen VRF batch verifier on the same engine (reference src/pedersen.rs:255-427) -------
-avrf_batch* avrf_pedersen_batch_new(uint32_t suite, uint32_t fmt) {
-  avrf_batch* b = avrf_thin_batch_new(suite, fmt);
+avrf_batch* avrf_pedersen_batch_new_on(int device, uint32_t suite, uint32_t fmt) {
+  avrf_batch* b = avrf_thin_batch_new_on(device, suite, fmt);
   if (b) b->scheme = 1;      // eager seeding like the thin verifier: push pipelines H2D, k_prepare_ped, D2H and the host SHA-512
   return b;
 }
+
+avrf_batch* avrf_pedersen_batch_new(uint32_t suite, uint32_t fmt) { return avrf_pedersen_batch_new_on(-1, suite, fmt); }
 
 int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
                                   const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,

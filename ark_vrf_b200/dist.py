@@ -15,7 +15,9 @@ The reference has no distributed code; this is the multi-GPU form of
      identity (thin.rs:320-324).
 
 The verdict is identical on every rank.  Shard boundaries need no alignment (weights are
-addressed by global index).
+addressed by global index).  A `pedersen.BatchVerifier` shard runs the same steps for
+`pedersen::BatchVerifier::verify` (src/pedersen.rs:341-426): 96-byte (c_j, s_j, sb_j) records in
+step 2, five MSM terms per proof and the shard's share of G and B in step 3.
 """
 from __future__ import annotations
 
@@ -63,10 +65,18 @@ class _DevView:
 _gather_buf = {}
 
 
-def _device_seed(shard, suite: int, group, device):
-    """NCCL fast path: all-gather the (c,s) streams device-to-device (equal shard sizes), then hash the
-    gathered stream with the chunked D2H overlapped with the host SHA-512.  Returns (seed, n_total)
-    or None when shard sizes differ (caller falls back to the generic path)."""
+def _seed_fns(stride: int):
+    """(host, device) seed functions of the scheme whose batch-seed records are `stride` bytes."""
+    from . import pedersen, thin
+    if stride == pedersen.BatchVerifier.cs_stride:
+        return pedersen.seed_of_stream, pedersen.seed_of_device_stream
+    return thin.seed_of_stream, thin.seed_of_device_stream
+
+
+def _device_seed(shard, suite: int, group, device, stride: int = 64):
+    """NCCL fast path: all-gather the batch-seed streams (`stride` bytes per proof) device-to-device (equal
+    shard sizes), then hash the gathered stream with the chunked D2H overlapped with the host SHA-512.
+    Returns (seed, n_total) or None when shard sizes differ (caller falls back to the generic path)."""
     import torch
     import torch.distributed as dist
     world = dist.get_world_size(group)
@@ -87,23 +97,28 @@ def _device_seed(shard, suite: int, group, device):
         _gather_buf[key] = out
     dist.all_gather_into_tensor(out, local, group=group)
     torch.cuda.current_stream(device).synchronize()
-    from . import thin
-    return thin.seed_of_device_stream(suite, out.data_ptr(), world * nl), world * nl
+    return _seed_fns(stride)[1](suite, out.data_ptr(), world * nl), world * nl
 
 
 def sharded_verify(shard, suite: int, first_index: int, group=None, device=None,
                    seed_fn: Optional[Callable] = None, combine_fn: Optional[Callable] = None,
                    timings: Optional[dict] = None, weights: str = "reference") -> int:
     """Verify one batch whose proofs [first_index, first_index + len(shard)) live in `shard`
-    (a `BatchVerifier` holding this rank's proofs).  Returns the status code (same on all ranks).
+    (a `thin.BatchVerifier` or `pedersen.BatchVerifier` holding this rank's proofs).  Returns the status
+    code (same on all ranks).
 
     `seed_fn(suite, stream_bytes)` / `combine_fn(suite, partials_bytes)` default to the library's
-    (avrf_thin_seed / avrf_thin_combine_partials); tests inject oracle-backed ones to exercise
-    the rank plumbing on CPU."""
+    (avrf_thin_seed or avrf_pedersen_seed, by the shard's `cs_stride`; avrf_thin_combine_partials);
+    tests inject oracle-backed ones to exercise the rank plumbing on CPU.  `weights="tree"` is
+    defined for Thin shards only: a Pedersen shard raises ValueError, on every rank, before any
+    collective."""
     import time
-    import torch.distributed as dist
     from . import thin
-    seed_fn = seed_fn or thin.seed_of_stream
+    stride = int(getattr(shard, "cs_stride", 64))
+    default_seed, _ = _seed_fns(stride)
+    if weights == "tree" and default_seed is not thin.seed_of_stream:
+        raise ValueError("weights='tree' is defined for Thin-VRF batches only")
+    seed_fn = seed_fn or default_seed
     combine_fn = combine_fn or thin.combine_partials
     dev = device if device is not None else "cpu"
     t0 = time.perf_counter()
@@ -119,9 +134,9 @@ def sharded_verify(shard, suite: int, first_index: int, group=None, device=None,
         n_total = sum(int.from_bytes(bytes(g[:8]), "little") for g in got)
         all_leaves = np.concatenate([g[8:] for g in got])
         fast = (thin.seed_of_tree(suite, n_total, all_leaves), n_total)
-    elif dev != "cpu" and hasattr(shard, "cs_stream_dev") and seed_fn is thin.seed_of_stream:
+    elif dev != "cpu" and hasattr(shard, "cs_stream_dev") and seed_fn is default_seed:
         t1 = time.perf_counter()
-        fast = _device_seed(shard, suite, group, dev)
+        fast = _device_seed(shard, suite, group, dev, stride)
     if fast is not None:
         seed, total = fast
         t2 = t3 = time.perf_counter()
@@ -133,7 +148,7 @@ def sharded_verify(shard, suite: int, first_index: int, group=None, device=None,
         t2 = time.perf_counter()
         seed = seed_fn(suite, np.ascontiguousarray(stream))
         t3 = time.perf_counter()
-        total = stream.size // 64
+        total = stream.size // stride
     if total == 0:
         return STATUS_OK                                       # thin.rs:262-264
     partial = shard.partial(seed, first_index) if len(shard) else None

@@ -10,6 +10,9 @@ Mirror of `ark_vrf::pedersen` (reference src/pedersen.rs):
     (wire-format proofs)             BatchVerifier.push_compressed(), serialize_proofs()  (Proof::{de,}serialize_compressed)
     (per-proof verdicts)             BatchVerifier.verify_each() / find_invalid()
     (throughput mode)                BatchServer: whole batches on a native worker pool, decoded or in wire format
+    (one batch over several GPUs)    ShardedBatchVerifier: every GPU of this process (init_multi);
+                                     BatchVerifier.{prepare_device, cs_stream, cs_stream_dev, partial}, seed_of_stream,
+                                     seed_of_device_stream: one process per GPU (dist.sharded_verify)
 A proof is `(pk_com, r, ok, s, sb)` (pedersen.rs:43-50)."""
 from __future__ import annotations
 
@@ -23,7 +26,8 @@ from . import _lib
 from .ops import pedersen_prove_many as prove_many          # noqa: F401  (re-exported: pedersen.prove_many)
 from .ops import point_compress
 from .synth import ORDER
-from .thin import Format, Suite, Tap, _BatchBase, _ServerBase, _bytes_of, _ios_bytes, _raise_for_status, ptr
+from .thin import (Format, Suite, Tap, _BatchBase, _ServerBase, _ShardedBase, _bytes_of, _ios_bytes, _raise_for_status,
+                   ptr)
 
 
 @dataclass
@@ -44,12 +48,20 @@ class BatchItem:                          # pedersen::BatchItem; hashing deferre
 
 
 class BatchVerifier(_BatchBase):
-    """pedersen::BatchVerifier<S> (src/pedersen.rs:322-427) on one B200; the handle controls are `thin.BatchVerifier`'s."""
+    """pedersen::BatchVerifier<S> (src/pedersen.rs:322-427) on one B200; the handle controls are `thin.BatchVerifier`'s.
+    `eager_seed=False` (a shard of a batch spread over processes: its seed comes from the gathered stream) and `device`
+    as in `thin.BatchVerifier`."""
 
-    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL):
+    cs_stride = 96                        # c || s || sb per proof (src/pedersen.rs:361-367)
+
+    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL, eager_seed: bool = True,
+                 device: int = -1):
         self._lib = _lib.load()
         self.suite, self.fmt = Suite(suite), Format(fmt)
-        self._open(self._lib.avrf_pedersen_batch_new(int(self.suite), int(self.fmt)), "avrf_pedersen_batch_new")
+        self._open(self._lib.avrf_pedersen_batch_new_on(int(device), int(self.suite), int(self.fmt)),
+                   "avrf_pedersen_batch_new")
+        if not eager_seed:
+            _lib.check(self._lib.avrf_thin_batch_set_eager(self._h, 0))
 
     @staticmethod
     def prepare(ios, ad, proof: Proof) -> BatchItem:
@@ -105,6 +117,55 @@ class BatchVerifier(_BatchBase):
         buf = np.zeros(max(size, 1), dtype=np.uint8)
         _lib.check(self._lib.avrf_thin_batch_tap(self._h, int(what), ptr(buf), buf.nbytes))
         return buf
+
+
+class _ShardView(BatchVerifier):
+    """One device's Pedersen handle inside a `ShardedBatchVerifier` (taps, timings, verify_each; owned by the parent)."""
+
+    def __init__(self, parent, handle):
+        self._lib, self.suite, self.fmt, self._h, self._parent = parent._lib, parent.suite, parent.fmt, handle, parent
+
+    def close(self) -> None:
+        self._h = None
+
+
+class ShardedBatchVerifier(_ShardedBase):
+    """pedersen::BatchVerifier<S> (src/pedersen.rs:322-427) over every GPU initialised with `thin.init_multi`, inside
+    ONE process: include/avrf.h, "Multi-GPU batches".  Seed, weights and verdict are those of one `BatchVerifier`
+    holding the same proofs in the same order; the serial batch-seed hash still runs once, on one core."""
+
+    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL):
+        self.suite, self.fmt = Suite(suite), Format(fmt)
+        self._open(_lib.load().avrf_pedersen_sharded_new, "avrf_pedersen_sharded_new")
+
+    def push_many(self, ios, io_offsets, ad_blob, ad_offsets, pk_com, r, ok, s, sb) -> None:
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        _lib.check(self._lib.avrf_pedersen_sharded_push_many(self._h, n, ptr(ios), ptr(io_offsets), ptr(ad_blob),
+                                                             ptr(ad_offsets), ptr(pk_com), ptr(r), ptr(ok), ptr(s),
+                                                             ptr(sb)))
+
+    def shard(self, index: int) -> _ShardView:
+        """Device `index`'s handle: `tap` (W: t_j || u_j, 32 bytes per proof; SCALARS: 5n + 2 terms), `timings` and
+        `verify_each`, indexed by the proof's position on that device."""
+        return _ShardView(self, self._shard_handle(index))
+
+
+def seed_of_stream(suite: Union[Suite, int], stream) -> bytes:
+    """SHA512(SUITE_ID || 0x50 || stream) of 96-byte records c || s || sb (src/pedersen.rs:361-367)."""
+    lib = _lib.load()
+    out = (C.c_uint8 * 64)()
+    n = (stream.nbytes if isinstance(stream, np.ndarray) else len(stream)) // BatchVerifier.cs_stride
+    _lib.check(lib.avrf_pedersen_seed(int(suite), ptr(stream), n, out))
+    return bytes(out)
+
+
+def seed_of_device_stream(suite: Union[Suite, int], dev_ptr: int, n_items: int) -> bytes:
+    """The same seed of `n_items` records resident on the default device (`avrf_pedersen_seed_dev`)."""
+    lib = _lib.load()
+    out = (C.c_uint8 * 64)()
+    _lib.check(lib.avrf_pedersen_seed_dev(int(suite), dev_ptr, n_items, out))
+    return bytes(out)
 
 
 class BatchServer(_ServerBase):

@@ -94,6 +94,11 @@ extern "C" {
         ad_offsets: *const u32, proofs: *const u8, ok: *mut u8, n_bad: *mut u64,
     ) -> i32;
     fn avrf_pedersen_batch_verify(b: *mut AvrfBatch, status: *mut i32) -> i32;
+    fn avrf_pedersen_sharded_new(suite: u32, fmt: u32) -> *mut AvrfSharded;
+    fn avrf_pedersen_sharded_push_many(
+        sh: *mut AvrfSharded, n: u64, ios: *const u8, io_offsets: *const u32, ad_blob: *const u8,
+        ad_offsets: *const u32, pk_com: *const u8, r: *const u8, ok: *const u8, s: *const u8, sb: *const u8,
+    ) -> i32;
     fn avrf_pedersen_batch_verify_each(b: *mut AvrfBatch, statuses: *mut i32) -> i32;
     fn avrf_pedersen_verify_one(
         suite: u32, fmt: u32, ios: *const u8, n_ios: u32, ad: *const u8, ad_len: u32, pk_com: *const u8,
@@ -649,6 +654,56 @@ pub mod pedersen {
             self.ad_offsets.push(self.ad.len() as u32);
         }
     }
+
+    /// One Pedersen batch over every GPU of the box, inside this process (`avrf_init_multi` +
+    /// `avrf_pedersen_sharded_*`, the other `avrf_thin_sharded_*` calls serve both schemes): same seed, weights and
+    /// verdict as a single-device `BatchVerifier` holding the same proofs in the same order.
+    pub struct ShardedBatchVerifier<S: GpuSuite + PedersenSuite> {
+        h: *mut AvrfSharded,
+        _s: PhantomData<S>,
+    }
+
+    impl<S: GpuSuite + PedersenSuite> ShardedBatchVerifier<S> {
+        /// `n_dev` <= 0: every CUDA device of the box.
+        pub fn new(n_dev: i32) -> Self {
+            let h = unsafe {
+                let rc = avrf_init_multi(n_dev, core::ptr::null());
+                assert!(rc == 0, "libavrf_gpu system error {rc}");
+                avrf_pedersen_sharded_new(S::AVRF_SUITE, AVRF_FMT_MONTGOMERY)
+            };
+            assert!(!h.is_null(), "avrf_pedersen_sharded_new failed");
+            static CHECKED: std::sync::Once = std::sync::Once::new();
+            CHECKED.call_once(layout_self_check::<S>);
+            Self { h, _s: PhantomData }
+        }
+        pub fn push_many(&mut self, b: &Batch<S>) {
+            let rc = unsafe {
+                avrf_pedersen_sharded_push_many(
+                    self.h, b.pk_com.len() as u64, b.ios.as_ptr() as *const u8, b.io_offsets.as_ptr(), b.ad.as_ptr(),
+                    b.ad_offsets.as_ptr(), b.pk_com.as_ptr() as *const u8, b.r.as_ptr() as *const u8,
+                    b.ok.as_ptr() as *const u8, b.s.as_ptr() as *const u8, b.sb.as_ptr() as *const u8,
+                )
+            };
+            assert!(rc == 0, "libavrf_gpu system error {rc}");
+        }
+        pub fn clear(&mut self) {
+            let rc = unsafe { avrf_thin_sharded_clear(self.h) };
+            assert!(rc == 0, "libavrf_gpu system error {rc}");
+        }
+        /// Same contract as `pedersen::BatchVerifier::verify` (src/pedersen.rs:341-426).
+        pub fn verify(&self) -> Result<(), Error> {
+            let mut status = -1i32;
+            let rc = unsafe { avrf_thin_sharded_verify(self.h, &mut status) };
+            status_to_result(rc, status)
+        }
+    }
+
+    impl<S: GpuSuite + PedersenSuite> Drop for ShardedBatchVerifier<S> {
+        fn drop(&mut self) {
+            unsafe { avrf_thin_sharded_free(self.h) }
+        }
+    }
+    unsafe impl<S: GpuSuite + PedersenSuite> Send for ShardedBatchVerifier<S> {}
 
     /// Throughput mode for the Pedersen VRF: the worker pool of `gpu::BatchServer`, one Pedersen batch verifier per
     /// worker (`avrf_pedersen_server_new`).  Every submitted batch gets the verdict `pedersen::BatchVerifier::verify`

@@ -137,8 +137,10 @@ class BatchItem:                          # thin::BatchItem (src/thin.rs:172-179
 
 class _BatchBase:
     """The controls of a batch handle that serve both schemes (include/avrf.h): `thin.BatchVerifier` and
-    `pedersen.BatchVerifier` share them.  Pushes, taps and per-proof verdicts are scheme-specific and stay in those
-    classes."""
+    `pedersen.BatchVerifier` share them, and so do the building blocks of a batch sharded over processes
+    (`dist.sharded_verify`).  Pushes, taps and per-proof verdicts are scheme-specific and stay in those classes."""
+
+    cs_stride = 64                        # bytes per proof of the batch-seed stream (Thin: c || s; Pedersen: c || s || sb)
 
     def _open(self, handle, what: str) -> None:
         self._h = handle
@@ -192,6 +194,33 @@ class _BatchBase:
         t = _lib.Timings()
         _lib.check(self._lib.avrf_thin_batch_timings(self._h, C.byref(t)))
         return t.as_dict()
+
+    # -- sharded path ------------------------------------------------------------------------
+    def prepare_device(self) -> bool:
+        """Runs the per-proof transcripts on the GPU; returns True if an identity pk (pk_com) / I / O was seen."""
+        inv = C.c_int32(0)
+        _lib.check(self._lib.avrf_thin_batch_prepare(self._h, C.byref(inv)))
+        return bool(inv.value)
+
+    def cs_stream(self) -> np.ndarray:
+        """The batch-seed stream of this handle's proofs, one `cs_stride`-byte record per proof."""
+        out = np.empty((len(self), self.cs_stride), dtype=np.uint8)
+        _lib.check(self._lib.avrf_thin_batch_cs_stream(self._h, ptr(out)))
+        return out
+
+    def cs_stream_dev(self):
+        """(device pointer, n_bytes) of the batch-seed stream after prepare (for a device-side all-gather)."""
+        p = self._lib.avrf_thin_batch_cs_dev(self._h)
+        if not p and len(self):
+            _lib.check(-1)
+        return p, self.cs_stride * len(self)
+
+    def partial(self, seed: bytes, first_index: int) -> bytes:
+        """This handle's share of the batch MSM under `seed`, its proofs at global indices first_index, ... (128 bytes,
+        extended coordinates in Montgomery form)."""
+        out = (C.c_uint8 * 128)()
+        _lib.check(self._lib.avrf_thin_batch_partial(self._h, _bytes_of(seed, 64), first_index, out))
+        return bytes(out)
 
     def close(self) -> None:
         if getattr(self, "_h", None):
@@ -277,36 +306,13 @@ class BatchVerifier(_BatchBase):
     def set_weights_mode(self, mode: int) -> None:
         _lib.check(self._lib.avrf_thin_batch_set_weights_mode(self._h, mode))
 
-    # -- sharded path ------------------------------------------------------------------------
-    def prepare_device(self) -> bool:
-        """Runs the per-proof transcripts on the GPU; returns True if an identity pk/I/O was seen."""
-        inv = C.c_int32(0)
-        _lib.check(self._lib.avrf_thin_batch_prepare(self._h, C.byref(inv)))
-        return bool(inv.value)
-
-    def cs_stream(self) -> np.ndarray:
-        out = np.empty((len(self), 64), dtype=np.uint8)
-        _lib.check(self._lib.avrf_thin_batch_cs_stream(self._h, ptr(out)))
-        return out
-
-    def cs_stream_dev(self):
-        """(device pointer, n_bytes) of the (c,s) stream after prepare (for a device-side all-gather)."""
-        p = self._lib.avrf_thin_batch_cs_dev(self._h)
-        if not p and len(self):
-            _lib.check(-1)
-        return p, 64 * len(self)
-
+    # -- sharded path (prepare_device, cs_stream, cs_stream_dev, partial: _BatchBase) --------------
     def tree_leaves(self, first_index: int = 0) -> np.ndarray:
         """Leaf digests of this handle's stream for AVRF_WEIGHTS_TREE (64 bytes per 32 proofs)."""
         out = np.zeros(((len(self) + 31) // 32 + 1, 64), dtype=np.uint8)
         n = C.c_uint64(0)
         _lib.check(self._lib.avrf_thin_batch_tree_leaves(self._h, first_index, ptr(out), C.byref(n)))
         return out[:n.value]
-
-    def partial(self, seed: bytes, first_index: int) -> bytes:
-        out = (C.c_uint8 * 128)()
-        _lib.check(self._lib.avrf_thin_batch_partial(self._h, _bytes_of(seed, 64), first_index, out))
-        return bytes(out)
 
     def tap(self, what: Tap) -> np.ndarray:
         n = len(self)
@@ -352,17 +358,22 @@ class _ShardView(BatchVerifier):
         self._h = None
 
 
-class ShardedBatchVerifier:
-    """thin::BatchVerifier<S> (src/thin.rs:188-326) over every GPU initialised with `init_multi`, inside ONE
-    process and without torch.distributed: include/avrf.h, "Multi-GPU batches"."""
+class _ShardedBase:
+    """What the multi-GPU batches of both schemes share (include/avrf.h, "Multi-GPU batches"): every
+    `avrf_thin_sharded_*` call but the constructor and the push serves either kind of handle."""
 
-    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL):
+    def _open(self, new, what: str) -> None:
         self._lib = _lib.load()
-        self.suite, self.fmt = Suite(suite), Format(fmt)
-        self._h = self._lib.avrf_thin_sharded_new(int(self.suite), int(self.fmt))
+        self._h = new(int(self.suite), int(self.fmt))
         if not self._h:
             msg = self._lib.avrf_last_error()
-            raise _lib.AvrfError(msg.decode() if msg else "avrf_thin_sharded_new failed")
+            raise _lib.AvrfError(msg.decode() if msg else f"{what} failed")
+
+    def _shard_handle(self, index: int):
+        h = self._lib.avrf_thin_sharded_shard(self._h, index)
+        if not h:
+            _lib.check(-2)
+        return h
 
     @property
     def devices(self) -> int:
@@ -370,12 +381,6 @@ class ShardedBatchVerifier:
 
     def __len__(self) -> int:
         return int(self._lib.avrf_thin_sharded_len(self._h))
-
-    def push_many(self, pk, ios, io_offsets, ad_blob, ad_offsets, r, s) -> None:
-        n = len(io_offsets) - 1
-        assert len(ad_offsets) == n + 1
-        _lib.check(self._lib.avrf_thin_sharded_push_many(self._h, n, ptr(pk), ptr(ios), ptr(io_offsets), ptr(ad_blob),
-                                                         ptr(ad_offsets), ptr(r), ptr(s)))
 
     def verify_status(self) -> int:
         st = C.c_int32(-1)
@@ -398,13 +403,6 @@ class ShardedBatchVerifier:
         _lib.check(self._lib.avrf_thin_sharded_timings(self._h, C.byref(t)))
         return t.as_dict()
 
-    def shard(self, index: int, n_ios: int) -> "_ShardView":
-        """Device `index`'s handle (taps / timings); `n_ios` = I/O pairs it holds (sizes the Z / SCALARS taps)."""
-        h = self._lib.avrf_thin_sharded_shard(self._h, index)
-        if not h:
-            _lib.check(-2)
-        return _ShardView(self, h, n_ios)
-
     def close(self) -> None:
         if getattr(self, "_h", None):
             self._lib.avrf_thin_sharded_free(self._h)
@@ -415,6 +413,25 @@ class ShardedBatchVerifier:
             self.close()
         except Exception:
             pass
+
+
+class ShardedBatchVerifier(_ShardedBase):
+    """thin::BatchVerifier<S> (src/thin.rs:188-326) over every GPU initialised with `init_multi`, inside ONE
+    process and without torch.distributed: include/avrf.h, "Multi-GPU batches"."""
+
+    def __init__(self, suite: Union[Suite, int], fmt: Union[Format, int] = Format.CANONICAL):
+        self.suite, self.fmt = Suite(suite), Format(fmt)
+        self._open(_lib.load().avrf_thin_sharded_new, "avrf_thin_sharded_new")
+
+    def push_many(self, pk, ios, io_offsets, ad_blob, ad_offsets, r, s) -> None:
+        n = len(io_offsets) - 1
+        assert len(ad_offsets) == n + 1
+        _lib.check(self._lib.avrf_thin_sharded_push_many(self._h, n, ptr(pk), ptr(ios), ptr(io_offsets), ptr(ad_blob),
+                                                         ptr(ad_offsets), ptr(r), ptr(s)))
+
+    def shard(self, index: int, n_ios: int) -> "_ShardView":
+        """Device `index`'s handle (taps / timings); `n_ios` = I/O pairs it holds (sizes the Z / SCALARS taps)."""
+        return _ShardView(self, self._shard_handle(index), n_ios)
 
 
 class _ServerBase:

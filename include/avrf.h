@@ -189,12 +189,17 @@ int avrf_thin_batch_verify_each(avrf_batch* b, int32_t* statuses);
  * rank-local:  avrf_thin_batch_prepare -> avrf_thin_batch_cs_stream  (gather streams, in
  * global proof order, on every rank) -> avrf_thin_seed -> avrf_thin_batch_partial
  * (first_index = global index of this shard's first proof) -> gather the 128-byte partials
- * -> avrf_thin_combine_partials on any rank. */
+ * -> avrf_thin_combine_partials on any rank.
+ * The same building blocks take Pedersen handles (avrf_pedersen_batch_new / _new_on): prepare, cs_stream, cs_dev,
+ * partial and combine_partials below serve both schemes; the seed of a Pedersen stream is avrf_pedersen_seed /
+ * avrf_pedersen_seed_dev (96-byte records instead of 64). */
 
 /* BatchVerifier::prepare for every pushed proof (src/thin.rs:209-226) on the GPU.
- * `invalid` (may be NULL) receives 1 if any pk / I / O is the identity (src/thin.rs:266-271). */
+ * `invalid` (may be NULL) receives 1 if any pk / I / O is the identity (src/thin.rs:266-271); on a Pedersen handle,
+ * if any pk_com or I/O point is (the InvalidData gate of pedersen::BatchVerifier::verify). */
 int avrf_thin_batch_prepare(avrf_batch* b, int32_t* invalid);
-/* 64 bytes per proof: LE32(c_j) || LE32(s_j), the bytes src/thin.rs:276-279 absorbs. */
+/* 64 bytes per proof: LE32(c_j) || LE32(s_j), the bytes src/thin.rs:276-279 absorbs.  On a Pedersen handle 96 bytes
+ * per proof: c_j || s_j || sb_j, 32 bytes each, the bytes src/pedersen.rs:361-367 absorbs. */
 int avrf_thin_batch_cs_stream(avrf_batch* b, uint8_t* out);
 /* Device address of the same stream (valid until the next push / clear), for a device-side
  * all-gather; avrf_thin_seed_dev hashes a device-resident stream (chunked D2H overlapped with the
@@ -203,13 +208,23 @@ void* avrf_thin_batch_cs_dev(avrf_batch* b);
 int avrf_thin_seed_dev(uint32_t suite, const void* cs_stream_dev, uint64_t n_items, uint8_t seed[64]);
 /* seed = SHA512(SUITE_ID || 0x50 || stream)  (src/thin.rs:274-279; host, serial). */
 int avrf_thin_seed(uint32_t suite, const uint8_t* cs_stream, uint64_t n_items, uint8_t seed[64]);
+/* The Pedersen batch seed: SHA512(SUITE_ID || 0x50 || stream), stream = n_items 96-byte records c || s || sb
+ * (src/pedersen.rs:361-367), as avrf_thin_batch_cs_stream returns them for a Pedersen handle.  A host hash that needs
+ * no device (as avrf_thin_seed); a bad suite, a null seed or a null stream of n_items > 0 is AVRF_ERR_ARG. */
+int avrf_pedersen_seed(uint32_t suite, const uint8_t* stream, uint64_t n_items, uint8_t seed[64]);
+/* The same of a device-resident stream (avrf_thin_batch_cs_dev of a Pedersen handle, or a gathered copy), hashed as
+ * avrf_thin_seed_dev hashes one; AVRF_ERR_ARG as avrf_pedersen_seed, then AVRF_ERR_NO_DEVICE without a device. */
+int avrf_pedersen_seed_dev(uint32_t suite, const void* stream_dev, uint64_t n_items, uint8_t seed[64]);
 /* AVRF_WEIGHTS_TREE building blocks: leaf_i = SHA512(0x00 || LE64(i) || (c,s) stream of proofs 32i..32i+31),
  * seed = SHA512(SUITE_ID || 0x50 || 0x01 || LE64(n_total) || leaf_0 || leaf_1 || ...).  first_index % 32 == 0. */
 int avrf_thin_batch_tree_leaves(avrf_batch* b, uint64_t first_index, uint8_t* out, uint64_t* n_leaves);
 int avrf_thin_seed_tree(uint32_t suite, uint64_t n_total, const uint8_t* leaves, uint64_t n_leaves, uint8_t seed[64]);
-/* This shard's share of the MSM of src/thin.rs:282-319 (incl. its share of the G term). */
+/* This shard's share of the MSM of src/thin.rs:282-319 (incl. its share of the G term).  On a Pedersen handle its share
+ * of the 5N+2-point MSM of src/pedersen.rs:373-418: five terms per proof, (t_j, u_j) squeezed at the GLOBAL index
+ * first_index + j (two proofs per 64-byte block, so first_index may be odd), and its share of the G and B terms. */
 int avrf_thin_batch_partial(avrf_batch* b, const uint8_t seed[64], uint64_t first_index, uint8_t partial[128]);
-/* Sum n partials and test for the identity (src/thin.rs:320-324): *status = OK / VERIFICATION_FAILURE. */
+/* Sum n partials and test for the identity (src/thin.rs:320-324): *status = OK / VERIFICATION_FAILURE.  Partials of
+ * either scheme (they are points of the suite's curve). */
 int avrf_thin_combine_partials(uint32_t suite, const uint8_t* partials, uint32_t n, int32_t* status);
 
 int avrf_thin_batch_tap(avrf_batch* b, uint32_t what, void* out, size_t out_bytes);
@@ -222,7 +237,13 @@ int avrf_thin_batch_tap(avrf_batch* b, uint32_t what, void* out, size_t out_byte
  * src/thin.rs:289), the tail of its fold kernel stores the partial and the identity-gate flag into a peer-mapped
  * slot on the first device, which adds the slots and writes the verdict (src/thin.rs:320-324).  Seed, weights and
  * verdict are bit-identical to a single-device handle holding the same proofs in the same order.
- * avrf_thin_sharded_shard returns the ordinary handle of one device (taps, timings; do not push to it). */
+ * avrf_thin_sharded_shard returns the ordinary handle of one device (taps, timings; do not push to it).
+ * avrf_pedersen_sharded_new makes the same over pedersen::BatchVerifier (src/pedersen.rs:255-427): its shards are
+ * Pedersen handles, the one hashing thread absorbs the 96-byte (c_j, s_j, sb_j) records (src/pedersen.rs:361-367),
+ * each device reduces its 5 terms per proof and its share of G and B.  Every avrf_thin_sharded_* call below except
+ * _new and _push_many serves both kinds of handle; the handle records its scheme, and a push of the other scheme
+ * (avrf_thin_sharded_push_many on a Pedersen handle, avrf_pedersen_sharded_push_many on a Thin one) is AVRF_ERR_ARG
+ * and leaves its proofs and seed as they were.  AVRF_WEIGHTS_TREE has no sharded form (either scheme). */
 typedef struct avrf_sharded avrf_sharded;
 typedef struct avrf_sharded_timings {
   float hash_wait_ms;      /* verify waited this long for the hashing thread */
@@ -244,13 +265,25 @@ int avrf_thin_sharded_verify(avrf_sharded* sh, int32_t* status);
 int avrf_thin_sharded_seed(const avrf_sharded* sh, uint8_t seed[64]);
 int avrf_thin_sharded_timings(const avrf_sharded* sh, avrf_sharded_timings* out);
 avrf_batch* avrf_thin_sharded_shard(avrf_sharded* sh, int index);
+/* pedersen::BatchVerifier (src/pedersen.rs:255-427) over every initialised device; NULL on error (avrf_last_error:
+ * a bad suite / fmt, or no device). */
+avrf_sharded* avrf_pedersen_sharded_new(uint32_t suite, uint32_t fmt);
+/* Push n proofs, arguments as avrf_pedersen_batch_push_many; the parts are cut as avrf_thin_sharded_push_many cuts
+ * them.  A null handle or argument is AVRF_ERR_ARG. */
+int avrf_pedersen_sharded_push_many(avrf_sharded* sh, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
+                                    const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,
+                                    const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);
 
 /* ---- Pedersen VRF batch verifier (SURVEY 8f-3; reference src/pedersen.rs:255-427) on the same MSM engine ---
  * pedersen::BatchVerifier::new / push (x n) / verify.  The handle is an avrf_batch: _free, _clear, _len, _reserve,
  * _invalidate, _set_eager, _set_blocking, _set_hash_pool, _verify_async / _verify_wait, _timings, _stream and
  * _tap (C, SEED, W = t_i||u_i, SCALARS, PARTIAL = the 5N+2-point MSM sum) apply; proofs are (pk_com 64, r 64,
- * ok 64, s 32, sb 32).  AVRF_WEIGHTS_TREE, _tree_leaves and the sharded path are Thin only. */
+ * ok 64, s 32, sb 32).  The sharded building blocks (_prepare, _cs_stream, _cs_dev, _partial; avrf_pedersen_seed) and
+ * the multi-GPU path (avrf_pedersen_sharded_*) serve Pedersen batches too; AVRF_WEIGHTS_TREE and _tree_leaves are Thin
+ * only. */
 avrf_batch* avrf_pedersen_batch_new(uint32_t suite, uint32_t fmt);
+/* The same on a chosen device, as avrf_thin_batch_new_on (device < 0: the default device). */
+avrf_batch* avrf_pedersen_batch_new_on(int device, uint32_t suite, uint32_t fmt);
 int avrf_pedersen_batch_push_many(avrf_batch* b, uint64_t n, const uint8_t* ios, const uint32_t* io_offsets,
                                   const uint8_t* ad_blob, const uint32_t* ad_offsets, const uint8_t* pk_com,
                                   const uint8_t* r, const uint8_t* ok, const uint8_t* s, const uint8_t* sb);

@@ -12,6 +12,7 @@
 //   pedersen::BatchVerifier<S>::{reserve, push, push_compressed, verify, verify_each, find_invalid}   src/pedersen.rs:322-427
 //   pedersen::prove_many (Prover::prove, n proofs) src/pedersen.rs:136-186
 //   pedersen::BatchServer<S>::{submit, submit_compressed, wait}   (new: the same worker pool for Pedersen batches)
+//   pedersen::ShardedBatchVerifier<S>             (new: one Pedersen batch over several GPUs of this process)
 //   Error::{VerificationFailure, InvalidData}     src/lib.rs:136-147
 //
 // The host toolchain of the reference (Rust) is absent from the build image, so this header is the
@@ -281,6 +282,39 @@ struct Batch {
     ad_offsets.push_back((uint32_t)ad.size());
   }
   size_t len() const { return pk_com.size(); }
+};
+
+using thin::init_multi;
+
+// One Pedersen batch over every GPU initialised with init_multi(), inside this process (include/avrf.h, "Multi-GPU
+// batches": avrf_pedersen_sharded_new / _push_many and the avrf_thin_sharded_* calls that serve both schemes).
+template <class S, uint32_t FMT = AVRF_FMT_MONTGOMERY>
+class ShardedBatchVerifier {
+ public:
+  ShardedBatchVerifier() : h_(avrf_pedersen_sharded_new(S::ID, FMT)) { if (!h_) throw std::runtime_error(avrf_last_error()); }
+  ~ShardedBatchVerifier() { avrf_thin_sharded_free(h_); }
+  ShardedBatchVerifier(const ShardedBatchVerifier&) = delete;
+  ShardedBatchVerifier& operator=(const ShardedBatchVerifier&) = delete;
+  void push_many(const Batch& b) {
+    const bool any = b.len() != 0;
+    check(avrf_pedersen_sharded_push_many(h_, b.len(), b.ios.empty() ? nullptr : b.ios[0].input.data(), b.io_offsets.data(),
+                                          b.ad.empty() ? nullptr : b.ad.data(), b.ad_offsets.data(),
+                                          any ? b.pk_com[0].data() : nullptr, any ? b.r[0].data() : nullptr,
+                                          any ? b.ok[0].data() : nullptr, any ? b.s[0].data() : nullptr,
+                                          any ? b.sb[0].data() : nullptr));
+  }
+  Result verify() const {
+    int32_t st = -1;
+    check(avrf_thin_sharded_verify(h_, &st));
+    return Result{st};
+  }
+  void clear() { check(avrf_thin_sharded_clear(h_)); }
+  int devices() const { return avrf_thin_sharded_devices(h_); }
+  int64_t len() const { return avrf_thin_sharded_len(h_); }
+  avrf_sharded* handle() const { return h_; }
+
+ private:
+  avrf_sharded* h_;
 };
 
 // Throughput mode for Pedersen batches: the worker pool of thin::BatchServer, one pedersen::BatchVerifier handle per

@@ -3,6 +3,9 @@ each, 4096 signers; every proof distinct).  Prints one JSON line with the device
 run.  Legs (best of --reps after a warm-up, except the latency leg):
   prove_many        avrf_pedersen_prove_many, proofs/s
   batch             push of the 2^20 proofs from pinned memory + verify, wall time, with avrf_thin_batch_timings
+  sharded           the same push + verify through pedersen.ShardedBatchVerifier over every GPU of the run
+                    (avrf_init_multi), wall time, with avrf_thin_sharded_timings (hash_wait_ms, host_hash_ms,
+                    shard_msm_ms_max), the device count and every card's name and power limit; beside the batch leg
   drop_in           the reference's call sequence: pedersen::BatchVerifier::push once per proof through the C++ mirror
                     (tools/push_loop.cpp, heap items, Montgomery format) + verify, wall time of the push loop and of
                     verify; beside it, at 2^14 proofs (a 2^20 loop of it takes too long to repeat), the same loop with
@@ -34,6 +37,15 @@ def device_info():
                          capture_output=True, text=True)
     name, power = (x.strip() for x in out.stdout.strip().split(",")) if out.returncode == 0 else ("unknown", "unknown")
     return name, power
+
+
+def cards():
+    """(name, power limit) of every GPU of the run, read now."""
+    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                         text=True)
+    if out.returncode != 0:
+        return []
+    return [[x.strip() for x in line.split(",")] for line in out.stdout.strip().splitlines()]
 
 
 def best(fn, reps):
@@ -103,6 +115,34 @@ def drop_in(b, n, reps):
                                     "staged_push_us_per_proof": round(1e3 * min(p for p, _ in new) / n_old, 3)}}
 
 
+def sharded(arrs, n, reps, batch_ms):
+    """The `sharded` leg: best of `reps` clear + push_many + verify of the batch over every GPU after a warm-up, and the
+    sharded timings of that best run."""
+    import torch
+    import ark_vrf_b200 as av
+    from ark_vrf_b200 import pedersen as ped
+    nd = av.init_multi(torch.cuda.device_count())
+    sh = ped.ShardedBatchVerifier(0, av.Format.CANONICAL)
+    status, runs = [], []
+
+    def run():
+        t0 = time.perf_counter()
+        sh.clear()
+        sh.push_many(*arrs)
+        status.append(sh.verify_status())
+        runs.append((time.perf_counter() - t0, sh.timings()))
+    run()                                  # warm-up
+    runs.clear()
+    for _ in range(reps):
+        run()
+    assert set(status) == {0}, status
+    t, tm = min(runs, key=lambda x: x[0])
+    sh.close()
+    return {"devices": nd, "cards": cards(), "n": n, "push_verify_ms": round(1e3 * t, 2), "proofs_per_s": round(n / t),
+            "hash_wait_ms": round(tm["hash_wait_ms"], 2), "host_hash_ms": round(tm["host_hash_ms"], 2),
+            "shard_msm_ms_max": round(tm["shard_msm_ms_max"], 3), "batch_push_verify_ms": batch_ms}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--log2n", type=int, default=20)
@@ -144,6 +184,7 @@ def main():
     res["batch_push_verify_ms"] = round(1e3 * t, 2)
     res["batch_proofs_per_s"] = round(n / t)
     res["batch_timings"] = {k: (round(v, 3) if isinstance(v, float) else v) for k, v in tm.as_dict().items()}
+    res["sharded"] = sharded(arrs, n, a.reps, res["batch_push_verify_ms"])
     res["drop_in"] = drop_in(b, n, a.reps)
 
     # wire format: what callers hold before Proof::deserialize_compressed
